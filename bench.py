@@ -31,6 +31,12 @@ N > 1  = per-GPU batch fixed (weak scaling); time = max over ranks.
 --impl reference = the UNMODIFIED reference (baseline/_ref or /root/reference: models.py + torch CPU ops, all host
          threads, its own train-loop body train.py:748-779) on a bounded sample of the same workload; when the
          staged reference is absent, the oracle port (cpu_baseline.kind says which).
+--dump-outputs DIR = after the timed steps of the selected workload, write what its last timed step handed back to
+         the caller as DIR/<name>.npy (float32; integer outputs as float64), outputs larger than 16 MB as a fixed,
+         seeded sample: training -> per-utterance loss and the updated parameters; inference -> loss, log-probs,
+         their CTC gradient, greedy tokens and token counts; sweep -> loss and token counts of the whole pass.  With
+         --gpus N > 1 rank 0 writes: its batch, or for the sweep its shard.
+         Inputs and weights are seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -219,6 +225,27 @@ def measured_peaks():
 		return None
 
 
+DUMP_BYTES_PER_ARRAY = 16 << 20
+DUMP_BYTES_TOTAL = 64 << 20
+
+
+def host_outputs(outputs):
+	"""device tensors -> numpy arrays for --dump-outputs: float32, integer tensors as float64 (exact); a tensor above
+	DUMP_BYTES_PER_ARRAY becomes a sample of its flattened values at indices drawn from a fixed seed, the same in every run"""
+	import numpy as np
+	out = {}
+	for name, t in outputs.items():
+		t = t.detach()
+		dtype = torch.float32 if t.is_floating_point() else torch.float64
+		limit = DUMP_BYTES_PER_ARRAY // (4 if dtype == torch.float32 else 8)
+		if t.numel() > limit:
+			idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), limit))
+			t = t.flatten()[torch.from_numpy(idx).to(t.device)]
+		out[name] = t.to(dtype).cpu().numpy()
+	assert sum(a.nbytes for a in out.values()) <= DUMP_BYTES_TOTAL, {n: a.nbytes for n, a in out.items()}
+	return out
+
+
 # --------------------------------------------------------------------------------------------
 # reference arms: the UNMODIFIED reference (baseline/_ref staged by __graft_entry__.build(), or /root/reference) through
 # its own public API; the oracle port only when neither exists
@@ -384,7 +411,8 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 	replicas = None
 
 	def infer_once(s, xl, yy, yl, want_grad):
-		"""eval forward (loss included through the public API) + device part of GreedyCTCGenerator + optionally the CTC gradient"""
+		"""eval forward (loss included through the public API) + device part of GreedyCTCGenerator + optionally the CTC gradient
+		(left in the returned log-probs' .grad)"""
 		with torch.no_grad():
 			out = model(s, xl)
 		lp = out['log_probs'][0]
@@ -393,7 +421,7 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		nll = ops.ctc_loss(lp.permute(2, 0, 1), yy[:, 0], out['olen'][0], yl[:, 0], blank = C - 1)
 		if want_grad:
 			nll.sum().backward()  # grad w.r.t. the log-probs/logits only: CTC alpha || beta -> gradient scatter
-		return nll, tok, cnt
+		return nll, tok, cnt, lp
 
 	if kind == 'train':
 		from convasr_b200 import optimizers, training
@@ -418,7 +446,7 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		run = [run_eager]  # swapped for the CUDA-graph replay after the eager launch count
 
 		def step_device():
-			return run[0](sig_d, xlen_d, y_d, ylen_d)
+			return dict(loss = run[0](sig_d, xlen_d, y_d, ylen_d))
 
 		def step_e2e(batch):
 			_, _, s, xl, yy, yl = batch  # this step's H2D was issued on the copy stream during the previous step
@@ -433,7 +461,8 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		flops = flops_fwd
 
 		def step_device():
-			return infer_once(sig_d, xlen_d, y_d, ylen_d, True)[0]
+			nll, tok, cnt, lp = infer_once(sig_d, xlen_d, y_d, ylen_d, True)
+			return dict(loss = nll, log_probs = lp.detach(), log_probs_grad = lp.grad, tokens = tok, token_counts = cnt)
 
 		def step_e2e(batch):
 			_, _, s, xl, yy, yl = batch
@@ -458,11 +487,17 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		shard_ylen = torch.randint(max(1, L // 3), L + 1, (n_local, 1), generator = g, device = dev)
 		flops = flops_fwd * n_local / B
 
+		keep = args.dump_outputs and level == 'full' and rank == 0  # per-micro-batch results are kept only for the dump
+
 		def step_device():
-			nll = None
+			kept = []
 			for a in range(0, n_local, B):
-				nll = infer_once(shard[a:a + B], shard_xlen[a:a + B], shard_y[a:a + B], shard_ylen[a:a + B], False)[0]
-			return nll
+				res = infer_once(shard[a:a + B], shard_xlen[a:a + B], shard_y[a:a + B], shard_ylen[a:a + B], False)
+				if keep:
+					kept.append(res)
+			if keep:
+				return dict(loss = torch.cat([r[0] for r in kept]), token_counts = torch.cat([r[2] for r in kept]))
+			return dict(loss = res[0])
 
 		loss_host = torch.empty(n_local, dtype = torch.float32).pin_memory()
 		cnt_host = torch.empty(n_local, dtype = torch.int32).pin_memory()
@@ -484,7 +519,8 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		tensor_entries = ['cab_conv1d_fused']
 		kernel_label = 'conv1d_umma_kernel'
 		audio_per_step = n_local * seconds
-		steps, warmup = max(1, min(steps, 2)), 1
+		if level != 'full':  # one pass is ~0.4 s per GPU: as a secondary line two timed passes are enough
+			steps, warmup = min(steps, 2), 1
 
 	def barrier():
 		if world > 1:
@@ -492,16 +528,17 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		torch.cuda.synchronize()
 
 	def timed(fn, n):
+		"""(total ms of n calls of fn, what the last call returned)"""
 		evs = []
 		for _ in range(n):
 			flush.zero_()
 			e0, e1 = torch.cuda.Event(enable_timing = True), torch.cuda.Event(enable_timing = True)
 			e0.record()
-			fn()
+			last = fn()
 			e1.record()
 			evs.append((e0, e1))
 		torch.cuda.synchronize()
-		return sum(a.elapsed_time(b) for a, b in evs)  # ms
+		return sum(a.elapsed_time(b) for a, b in evs), last
 
 	# one eager step counts this repo's kernel launches per step (graph replays bypass the counter)
 	step_device()
@@ -560,7 +597,7 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 			print(f'[bench] rank {rank}: CUDA-graph capture of the data-parallel step failed ({e!r}); eager step instead', file = sys.stderr)
 			config['cuda_graphs'] = False
 	for _ in range(warmup):
-		nll = step_device()
+		nll = step_device()['loss']
 	torch.cuda.synchronize()
 	assert bool(torch.isfinite(nll).all()), 'synthetic targets must admit an alignment'
 	sampler = ClockSampler(local_rank)
@@ -568,11 +605,18 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 		sampler.start()
 	barrier()
 	t_wall0 = time.time()
-	ms = timed(step_device, steps)
+	ms, last = timed(step_device, steps)
 	barrier()
 	t_wall1 = time.time()
 	clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
 	result = dict(ms = ms, ms_e2e = None, steps = steps)
+	if args.dump_outputs and level == 'full' and rank == 0:
+		if kind == 'train':  # the step hands back the loss; its other result is the updated parameters
+			last['parameters'] = torch.cat([p.detach().flatten() for p in train_params])
+		if 'tokens' in last:  # the collapse leaves the entries past each row's count unwritten
+			tok = last['tokens']
+			last['tokens'] = torch.where(torch.arange(tok.shape[1], device = dev) < last['token_counts'][:, None], tok, 0)
+		result['outputs'] = host_outputs(last)
 	if roofline is not None:
 		roofline['share_of_step'] = roofline['kernel_ms_per_step'] / (ms / steps)
 	if kind == 'train' and world > 1:
@@ -597,14 +641,14 @@ def measure(name, args, rank, world, local_rank, dev, steps, warmup, level):
 				return feed_mod.DeviceFeeder(((None, None) + tuple(t[a:a + B] for t in host) for a in range(0, n_local, B)), dev)
 			step_e2e(batches())
 			barrier()
-			result['ms_e2e'] = timed(lambda: step_e2e(batches()), steps)
+			result['ms_e2e'] = timed(lambda: step_e2e(batches()), steps)[0]
 			h2d = sum(t.numel() * t.element_size() for t in host)
 		else:
 			feeder = iter(feed_mod.DeviceFeeder(((None, None, sig_pin, xlen_pin, y_pin, ylen_pin) for _ in range(steps + 8)), dev))
 			for _ in range(3):
 				step_e2e(next(feeder))
 			barrier()
-			result['ms_e2e'] = timed(lambda: step_e2e(next(feeder)), steps)
+			result['ms_e2e'] = timed(lambda: step_e2e(next(feeder)), steps)[0]
 			h2d = sum(t.numel() * t.element_size() for t in (sig, xlen, y, ylen))
 		barrier()
 		result['h2d'] = h2d
@@ -627,7 +671,12 @@ def main():
 	ap.add_argument('--no-gpu-baseline', action = 'store_true')
 	ap.add_argument('--cpu-sample-batch', type = int, default = 4)
 	ap.add_argument('--no-cuda-graphs', action = 'store_true')
+	ap.add_argument('--dump-outputs', metavar = 'DIR', help = 'write the outputs of the last timed step as DIR/<name>.npy')
 	args = ap.parse_args()
+	if args.steps < 1:
+		ap.error('--steps must be at least 1')
+	if args.dump_outputs and args.impl != 'native':
+		ap.error('--dump-outputs writes the outputs of the native timed path (--impl native)')
 	model_name, C, B, seconds, precision, kind, lengths = WORKLOADS[args.workload]
 	rank = int(os.environ.get('RANK', 0))
 	world = int(os.environ.get('WORLD_SIZE', 1))
@@ -668,6 +717,11 @@ def main():
 	if rank == 0 and world == 1 and not args.no_cpu_baseline:
 		_, _, cpu_baseline = run_cpu_reference(args.workload, args.cpu_sample_batch, 3, 1)
 	r = measure(args.workload, args, rank, world, local_rank, dev, steps, warmup, 'full')
+	if args.dump_outputs and rank == 0:
+		import numpy as np
+		os.makedirs(args.dump_outputs, exist_ok = True)
+		for name, a in r['outputs'].items():
+			np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
 	ms, ms_e2e = reduce_max([r['ms'], r['ms_e2e']])
 	also = None
 	if not args.no_secondary and args.workload == DEFAULT_WORKLOAD:
