@@ -7,7 +7,8 @@
 // models.entropy / weighted_mean_entropy models.py:645-673.
 //
 // The recursions are T sequential steps, so each utterance gets one CTA with the extended
-// target states across threads and the previous time step in shared memory.
+// target states across threads and the previous time step in shared memory -- or, for alignments
+// of targets too long for one CTA, one thread-block cluster (ctc_align_cluster_kernel).
 #include "common.cuh"
 #include "../../include/convasr_b200.h"
 #include <atomic>
@@ -347,6 +348,27 @@ __device__ __forceinline__ float half_fn(const uint16_t* __restrict__ table, flo
     if (table == nullptr) return rh(computed);
     return __half2float(__ushort_as_half(__ldg(table + __half_as_ushort(__float2half_rn(x_half_valued)))));
 }
+// One state of one frame: alpha from the three predecessors p0 (stay), p1 (step), p2 (skip, already ZERO where the skip is
+// not allowed) plus the emission e_t, and the back-pointer `arg` (first maximum wins: stay, then step, then skip, ctc.py:50).
+// Shared by both alignment kernels, so they agree bit for bit wherever both run.
+template <bool HALF>
+__device__ __forceinline__ float ctc_align_state(float p0, float p1, float p2, float e_t, const uint16_t* __restrict__ tab_exp,
+                                                 const uint16_t* __restrict__ tab_log, int& arg) {
+    const float m = fmaxf(p0, fmaxf(p1, p2));
+    arg = 0;
+    if (p1 > p0) arg = 1;
+    if (p2 > fmaxf(p0, p1)) arg = 2;
+    const float ms = (fabsf(m) == INFINITY) ? 0.f : m;
+    if (HALF) {
+        const float d0 = rh(p0 - ms), d1 = rh(p1 - ms), d2 = rh(p2 - ms);
+        const float e0 = half_fn(tab_exp, d0, expf(d0)), e1 = half_fn(tab_exp, d1, expf(d1)), e2 = half_fn(tab_exp, d2, expf(d2));
+        const float ssum = rh((e0 + e1) + e2);
+        const float lse = rh(half_fn(tab_log, ssum, logf(ssum)) + ms);
+        return rh(e_t + lse);
+    }
+    const float lse = logf(expf(p0 - ms) + expf(p1 - ms) + expf(p2 - ms)) + ms;
+    return e_t + lse;
+}
 template <bool HALF>
 __global__ void ctc_align_kernel(const float* __restrict__ lp, int64_t st, int64_t sb, int64_t sc,
                                  const int64_t* __restrict__ targets, const int64_t* __restrict__ in_len,
@@ -401,22 +423,9 @@ __global__ void ctc_align_kernel(const float* __restrict__ lp, int64_t st, int64
                 const float p0 = prev[s + 2];
                 const float p1 = prev[s + 1];
                 const float p2 = diff[i] ? prev[s] : ZERO;
-                float m = fmaxf(p0, fmaxf(p1, p2));
-                int arg = 0;  // first maximum wins: stay, then step, then skip (ctc.py:50)
-                if (p1 > p0) arg = 1;
-                if (p2 > fmaxf(p0, p1)) arg = 2;
-                const float ms = (fabsf(m) == INFINITY) ? 0.f : m;
                 const float e_t = lpb[(int64_t)t * st + (int64_t)ext[i] * sc];
-                if (HALF) {
-                    const float d0 = rh(p0 - ms), d1 = rh(p1 - ms), d2 = rh(p2 - ms);
-                    const float e0 = half_fn(tab_exp, d0, expf(d0)), e1 = half_fn(tab_exp, d1, expf(d1)), e2 = half_fn(tab_exp, d2, expf(d2));
-                    const float ssum = rh((e0 + e1) + e2);
-                    const float lse = rh(half_fn(tab_log, ssum, logf(ssum)) + ms);
-                    cur[s + 2] = rh(e_t + lse);
-                } else {
-                    const float lse = logf(expf(p0 - ms) + expf(p1 - ms) + expf(p2 - ms)) + ms;
-                    cur[s + 2] = e_t + lse;
-                }
+                int arg;
+                cur[s + 2] = ctc_align_state<HALF>(p0, p1, p2, e_t, tab_exp, tab_log, arg);
                 bp[(size_t)t * S_max + s] = (uint8_t)arg;
             }
         }
@@ -440,6 +449,210 @@ __global__ void ctc_align_kernel(const float* __restrict__ lp, int64_t st, int64
                 if (s < 0) s = 0;
             }
         }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// ctc.alignment for long targets: one thread-block cluster per utterance.
+// The extended states are cut into slices of W states (W % 4 == 0); slice k lives on CTA k % n of the cluster, in its
+// local slot k / n (n = cluster size; one slot per CTA unless a caller forces small slices).  A slot holds two guard
+// cells in front of its W states: the last two alpha values of slice k-1 at the previous frame, which the CTA owning
+// slice k-1 stores there through distributed shared memory.  One cluster barrier per frame orders those stores
+// (and the local double buffer) -- every CTA runs every frame, live states or not, so no barrier can be missed.
+// A thread owns groups of 4 consecutive states: their four 2-bit back-pointers make one byte of the packed
+// workspace [B, T, ceil(S_max / 4)] (code of state s in bits 2*(s%4)), so no two threads write the same byte.
+// The recursion leaves the start state of the back-trace in out[b, 0]; ctc_align_backtrace_kernel takes it from there.
+// ------------------------------------------------------------------------------------------
+constexpr int kAlignClusterMax = 16;   // CTAs per utterance (non-portable cluster size)
+constexpr int kAlignGroupsPer = 2;     // groups of 4 states per thread
+constexpr int kAlignCtaStates = 4 * kAlignGroupsPer * 1024;  // states one CTA holds
+constexpr int kAlignLongMaxL = (kAlignClusterMax * kAlignCtaStates - 1) / 2;  // 65535: S = 131071
+
+__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
+__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+__device__ __forceinline__ uint32_t cluster_nctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
+    return r;
+}
+// generic address of `p` (a shared-memory address of this CTA) in the shared memory of CTA `rank` of the cluster
+__device__ __forceinline__ float* cluster_map(float* p, uint32_t rank) {
+    uint64_t out;
+    asm volatile("mapa.u64 %0, %1, %2;" : "=l"(out) : "l"(reinterpret_cast<uint64_t>(p)), "r"(rank));
+    return reinterpret_cast<float*>(out);
+}
+
+template <bool HALF>
+__global__ void __launch_bounds__(1024, 1)
+ctc_align_cluster_kernel(const float* __restrict__ lp, int64_t st, int64_t sb, int64_t sc, const int64_t* __restrict__ targets,
+                         const int64_t* __restrict__ in_len, const int64_t* __restrict__ tgt_len, int T, int L_max, int blank,
+                         int W, int n_slots, int64_t pitch, uint8_t* __restrict__ bp_ws, int64_t* __restrict__ out,
+                         const uint16_t* __restrict__ tab_exp, const uint16_t* __restrict__ tab_log) {
+    extern __shared__ float sh[];
+    const float ZERO = HALF ? -65504.f : -FLT_MAX;  // torch.finfo(dtype).min, ctc.py:29
+    const int n = (int)cluster_nctarank(), c = (int)cluster_ctarank();
+    const int b = blockIdx.x / n;
+    int tl = (int)tgt_len[b];
+    tl = tl < 0 ? 0 : (tl > L_max ? L_max : tl);
+    const int S = 2 * tl + 1;
+    const int slot_len = W + 2;
+    const int buf_len = n_slots * slot_len;
+    float* s_term = sh + 2 * buf_len;  // [2] alpha of states 2tl-1, 2tl at frame T-1 (on CTA 0)
+    const int gps = W >> 2;            // groups per slice
+    const int n_groups = n_slots * gps;
+    const float* lpb = lp + (int64_t)b * sb;
+    uint8_t* bp = bp_ws + (int64_t)b * T * pitch;
+
+    for (int i = threadIdx.x; i < 2 * buf_len + 2; i += blockDim.x) sh[i] = ZERO;
+
+    int loc[kAlignGroupsPer], s0[kAlignGroupsPer], lab1[kAlignGroupsPer], lab3[kAlignGroupsPer];
+    bool live[kAlignGroupsPer], skip1[kAlignGroupsPer], skip3[kAlignGroupsPer];
+    float* next_guard[kAlignGroupsPer];  // guard cells of slice k+1 in buffer 0 (buffer 1: + buf_len), or nullptr
+#pragma unroll
+    for (int i = 0; i < kAlignGroupsPer; ++i) {
+        const int g = threadIdx.x + i * blockDim.x;
+        const int j = g / gps, o = (g - j * gps) * 4, k = j * n + c;
+        live[i] = g < n_groups && k * W + o < S;
+        s0[i] = k * W + o;
+        loc[i] = j * slot_len + 2 + o;
+        lab1[i] = lab3[i] = blank;
+        skip1[i] = skip3[i] = false;
+        next_guard[i] = nullptr;
+        if (!live[i]) continue;
+        const int64_t* tg = targets + (int64_t)b * L_max;
+        if (s0[i] + 1 < S) {  // odd states may skip from the label two behind when it differs (ctc.py:23-27)
+            lab1[i] = (int)tg[(s0[i] + 1) >> 1];
+            skip1[i] = s0[i] + 1 >= 3 && lab1[i] != (int)tg[((s0[i] + 1) >> 1) - 1];
+        }
+        if (s0[i] + 3 < S) {
+            lab3[i] = (int)tg[(s0[i] + 3) >> 1];
+            skip3[i] = lab3[i] != lab1[i];
+        }
+        const int k1 = k + 1;
+        if (o == W - 4 && k1 < n * n_slots) {
+            next_guard[i] = cluster_map(sh + (k1 / n) * slot_len, (uint32_t)(k1 % n));
+        }
+    }
+    __syncthreads();  // ZERO fill before the frame-0 values
+#pragma unroll
+    for (int i = 0; i < kAlignGroupsPer; ++i)
+        if (live[i] && s0[i] == 0) {  // ctc.py:32-33
+            sh[loc[i]] = lpb[(int64_t)blank * sc];
+            if (S > 1) sh[loc[i] + 1] = lpb[(int64_t)lab1[i] * sc];
+        }
+
+    // emissions of the next frame are loaded while the cluster barrier of this one is pending
+    float eb[kAlignGroupsPer], e1[kAlignGroupsPer], e3[kAlignGroupsPer];
+    auto load_e = [&](int t) {
+#pragma unroll
+        for (int i = 0; i < kAlignGroupsPer; ++i)
+            if (live[i]) {
+                const float* r = lpb + (int64_t)t * st;
+                eb[i] = r[(int64_t)blank * sc];
+                e1[i] = r[(int64_t)lab1[i] * sc];
+                e3[i] = r[(int64_t)lab3[i] * sc];
+            }
+    };
+    cluster_arrive();  // every CTA of the cluster has started and initialised its buffers
+    if (T > 1) load_e(1);
+    cluster_wait();
+
+    // NB: the reference runs the recursion over ALL T frames of the padded batch (ctc.py:47)
+    for (int t = 1; t < T; ++t) {
+        const float* prev = sh + ((t - 1) & 1) * buf_len;
+        float* cur = sh + (t & 1) * buf_len;
+#pragma unroll
+        for (int i = 0; i < kAlignGroupsPer; ++i) {
+            if (!live[i]) continue;
+            const float* p = prev + loc[i];
+            const float am1 = p[-1], a0 = p[0], a1 = p[1], a2 = p[2], a3 = p[3];
+            // all four states unconditionally (independent chains, no branches): states >= S of the last live group are
+            // never read by a live state, the terminal read or the back-trace
+            int arg0, arg1, arg2, arg3;
+            const float v0 = ctc_align_state<HALF>(a0, am1, ZERO, eb[i], tab_exp, tab_log, arg0);  // even states: blanks, no skip
+            const float v1 = ctc_align_state<HALF>(a1, a0, skip1[i] ? am1 : ZERO, e1[i], tab_exp, tab_log, arg1);
+            const float v2 = ctc_align_state<HALF>(a2, a1, ZERO, eb[i], tab_exp, tab_log, arg2);
+            const float v3 = ctc_align_state<HALF>(a3, a2, skip3[i] ? a1 : ZERO, e3[i], tab_exp, tab_log, arg3);
+            cur[loc[i]] = v0;
+            cur[loc[i] + 1] = v1;
+            cur[loc[i] + 2] = v2;
+            cur[loc[i] + 3] = v3;
+            bp[(int64_t)t * pitch + (s0[i] >> 2)] = (uint8_t)(arg0 | (arg1 << 2) | (arg2 << 4) | (arg3 << 6));
+            if (next_guard[i]) {
+                float* gd = next_guard[i] + (t & 1) * buf_len;
+                gd[0] = v2;
+                gd[1] = v3;
+            }
+        }
+        cluster_arrive();
+        if (t + 1 < T) load_e(t + 1);
+        cluster_wait();
+    }
+
+    // terminal state from log_alpha after the FULL loop (global T-1), ctc.py:56-61: both values meet on CTA 0
+    if (threadIdx.x < 2) {
+        const int x = 2 * tl - 1 + (int)threadIdx.x;  // tl == 0: state -1 keeps ZERO
+        const int k = x / W;
+        if (x >= 0 && k % n == c) *cluster_map(s_term + threadIdx.x, 0) = sh[((T - 1) & 1) * buf_len + (k / n) * slot_len + 2 + (x - k * W)];
+    }
+    cluster_arrive();
+    cluster_wait();
+    if (c == 0 && threadIdx.x == 0) {
+        const int s = 2 * tl - 1 + (s_term[1] > s_term[0] ? 1 : 0);
+        out[(int64_t)b * L_max] = s < 0 ? 0 : s;
+    }
+}
+
+// Back-trace over the packed back-pointers, one warp per utterance.  s moves down by at most 2 per frame, so the codes of
+// the next 32 frames lie within 17 bytes of each row: every lane fetches one row's window (all loads of a strip in
+// flight at once), then lane 0 walks the strip from shared memory -- one memory round trip per 32 frames instead of one
+// per frame.  Output: the last frame spent in each label, zeros past target_length, zeros everywhere when il < 1.
+constexpr int kTraceWin = 17;
+__global__ void __launch_bounds__(32)
+ctc_align_backtrace_kernel(const uint8_t* __restrict__ bp_ws, int64_t pitch, const int64_t* __restrict__ in_len, int T, int L_max,
+                           int64_t* __restrict__ out) {
+    __shared__ uint8_t strip[32][kTraceWin + 3];
+    const int b = blockIdx.x, lane = threadIdx.x;
+    int64_t* ob = out + (int64_t)b * L_max;
+    int s = (int)ob[0];  // start state left by ctc_align_cluster_kernel
+    __syncwarp();
+    for (int l = lane; l < L_max; l += 32) ob[l] = 0;
+    int il = (int)in_len[b];
+    if (il > T) il = T;
+    if (il < 1) return;
+    __syncwarp();
+    const uint8_t* bpb = bp_ws + (int64_t)b * T * pitch;
+    int last_state = -1;
+    for (int t = il - 1; t >= 0; t -= 32) {
+        const int wb = max(0, (s >> 2) - (kTraceWin - 1));
+        const int r = t - lane;
+        if (r > 0) {
+            const uint8_t* row = bpb + (int64_t)r * pitch;
+#pragma unroll
+            for (int k = 0; k < kTraceWin; ++k)
+                if (wb + k < pitch) strip[lane][k] = row[wb + k];
+        }
+        __syncwarp();
+        if (lane == 0) {
+            for (int u = 0; u < 32 && t - u >= 0; ++u) {
+                const int tt = t - u;
+                if (s != last_state) {
+                    if (s & 1) ob[s >> 1] = tt;  // last frame spent in label s
+                    last_state = s;
+                }
+                if (tt > 0) {
+                    s -= (strip[u][(s >> 2) - wb] >> (2 * (s & 3))) & 3;
+                    if (s < 0) s = 0;
+                }
+            }
+        }
+        s = __shfl_sync(0xffffffffu, s, 0);
+        __syncwarp();
     }
 }
 
@@ -849,6 +1062,93 @@ extern "C" int cab_ctc_alignment(const float* log_probs, int64_t stride_t, int64
                                                               ws_backptr, out_alignment, nullptr, nullptr);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
+
+extern "C" int cab_ctc_alignment_long_workspace(int B, int T, int L_max, int64_t* bytes) {
+    CAB_CHECK_ARG(bytes != nullptr, "null output");
+    CAB_CHECK_ARG(B > 0 && T > 0 && L_max >= 0, "bad shape B=%d T=%d L=%d", B, T, L_max);
+    CAB_CHECK_ARG(L_max <= kAlignLongMaxL, "target too long: L_max=%d (the cluster alignment handles L_max <= %d)", L_max, kAlignLongMaxL);
+    *bytes = (int64_t)B * T * ((2 * (int64_t)L_max + 1 + 3) / 4);
+    return 0;
+}
+
+template <bool HALF>
+static int launch_align_cluster(int n, int threads, size_t smem, cudaStream_t stream, int B, const float* log_probs, int64_t st,
+                                int64_t sb, int64_t sc, const int64_t* targets, const int64_t* input_lengths,
+                                const int64_t* target_lengths, int T, int L_max, int blank, int W, int n_slots, int64_t pitch,
+                                uint8_t* ws, int64_t* out, const uint16_t* tab_exp, const uint16_t* tab_log) {
+    auto kernel = ctc_align_cluster_kernel<HALF>;
+    static size_t smem_set = 0;
+    if (smem_set == 0) CAB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    if (smem > smem_set) {
+        CAB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set = smem;
+    }
+    cudaLaunchConfig_t cfg = {};
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = n;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.gridDim = dim3(B * n);
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    int clusters = 0;
+    CAB_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg));
+    CAB_CHECK_ARG(clusters > 0, "a cluster of %d CTAs x %d threads with %zu B of shared memory does not fit this device", n, threads, smem);
+    CAB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, log_probs, st, sb, sc, targets, input_lengths, target_lengths, T, L_max, blank, W,
+                                      n_slots, pitch, ws, out, tab_exp, tab_log));
+    return 0;
+}
+
+extern "C" int cab_ctc_alignment_long(const float* log_probs, int64_t stride_t, int64_t stride_b, int64_t stride_c,
+                                      const int64_t* targets, const int64_t* input_lengths, const int64_t* target_lengths, int B,
+                                      int T, int C, int L_max, int blank, uint8_t* ws_backptr, int64_t* out_alignment,
+                                      int fp16_arithmetic, const uint16_t* fp16_exp_table, const uint16_t* fp16_log_table,
+                                      int states_per_cta, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CAB_CHECK_ARG(log_probs && targets && input_lengths && target_lengths, "null pointer argument");
+    CAB_CHECK_ARG(B > 0 && T > 0 && C > 0 && L_max >= 0, "bad shape B=%d T=%d C=%d L=%d", B, T, C, L_max);
+    CAB_CHECK_ARG(blank >= 0 && blank < C, "blank=%d out of range", blank);
+    CAB_CHECK_ARG(L_max <= kAlignLongMaxL, "target too long: L_max=%d (the cluster alignment handles L_max <= %d)", L_max, kAlignLongMaxL);
+    CAB_CHECK_ARG(ws_backptr && out_alignment, "null workspace/output");
+    CAB_CHECK_ARG((fp16_exp_table == nullptr) == (fp16_log_table == nullptr), "give both fp16 tables or neither");
+    CAB_CHECK_ARG(states_per_cta >= 0 && states_per_cta % 4 == 0, "states_per_cta=%d must be 0 or a positive multiple of 4", states_per_cta);
+    if (L_max == 0) return 0;  // out has no element
+    const int S_max = 2 * L_max + 1;
+    const int G4 = (S_max + 3) / 4;  // bytes per packed row
+    int n, W, n_slots;
+    if (states_per_cta > 0) {  // forced slice size: slices round-robin over up to kAlignClusterMax CTAs
+        W = states_per_cta;
+        const int n_slices = (S_max + W - 1) / W;
+        n = n_slices < kAlignClusterMax ? n_slices : kAlignClusterMax;
+        n_slots = (n_slices + n - 1) / n;
+    } else {  // one slice per CTA of at most ~2048 states
+        n = (S_max + 2047) / 2048;
+        if (n > kAlignClusterMax) n = kAlignClusterMax;
+        W = 4 * ((G4 + n - 1) / n);
+        n_slots = 1;
+    }
+    CAB_CHECK_ARG((int64_t)n_slots * W <= kAlignCtaStates, "states_per_cta=%d puts %lld states on one CTA (at most %d)", states_per_cta,
+                  (long long)n_slots * W, kAlignCtaStates);
+    const int groups = n_slots * W / 4;
+    const int per = groups > 1024 ? kAlignGroupsPer : 1;
+    const int threads = ((groups + per - 1) / per + 31) / 32 * 32;
+    const size_t smem = sizeof(float) * (2 * (size_t)n_slots * (W + 2) + 2);
+    int rc = fp16_arithmetic
+                 ? launch_align_cluster<true>(n, threads, smem, stream, B, log_probs, stride_t, stride_b, stride_c, targets, input_lengths,
+                                              target_lengths, T, L_max, blank, W, n_slots, G4, ws_backptr, out_alignment, fp16_exp_table,
+                                              fp16_log_table)
+                 : launch_align_cluster<false>(n, threads, smem, stream, B, log_probs, stride_t, stride_b, stride_c, targets, input_lengths,
+                                               target_lengths, T, L_max, blank, W, n_slots, G4, ws_backptr, out_alignment, nullptr, nullptr);
+    if (rc != 0) return rc;
+    ctc_align_backtrace_kernel<<<B, 32, 0, stream>>>(ws_backptr, G4, input_lengths, T, L_max, out_alignment);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(2, std::memory_order_relaxed);
     return 0;
 }
 

@@ -1,12 +1,15 @@
 """Drop-in replacement for the reference's `ctc` module (ctc.py:6-75): forced alignment on the
-GPU with one CTA per utterance (convasr_b200/csrc/ctc.cu: ctc_align_kernel).
+GPU (convasr_b200/csrc/ctc.cu).  Targets of up to 2047 labels run on one CTA per utterance
+(ctc_align_kernel); longer ones, up to 65535 labels (hour-long recordings), on a thread-block
+cluster per utterance (ctc_align_cluster_kernel + ctc_align_backtrace_kernel).
 
 All of the reference's behaviours are reproduced, including the batch-coupled ones (recursion
 over all T frames of the padded batch, terminal state read after the last global frame,
 back-trace from input_length-1, finite "zero", stay-preferred argmax ties) -- SURVEY.md A12 -- and
 its fp16 mode: on fp16 log_probs every operation of the recursion rounds to fp16 ("zero" = finfo(float16).min).
-`pack_backpointers` only changes the reference's memory format, never its result; the native
-kernel keeps one byte per back-pointer in a caller-owned workspace and ignores the flag.
+`pack_backpointers` only changes the reference's memory format, never its result, and is ignored
+here: the short-target kernel keeps one byte per back-pointer, the cluster kernel always packs
+four 2-bit back-pointers per byte (B * T * ceil((2L+1)/4) bytes).
 """
 import torch
 

@@ -440,22 +440,36 @@ def _fp16_tables(device):
 	return _FP16_TABLES[key]
 
 
-def ctc_alignment(log_probs, targets, input_lengths, target_lengths, blank = 0):
+CTC_ALIGN_CTA_STATES = 4096  # 2 * L_max + 1 up to which one CTA per utterance aligns (cab_ctc_alignment)
+
+
+def ctc_alignment(log_probs, targets, input_lengths, target_lengths, blank = 0, _states_per_cta = None):
 	"""fp16 log_probs: the recursion rounds to fp16 after every operation, as the reference does on an fp16 tensor (the
-	values are handed to the kernel as their exact fp32 images)"""
+	values are handed to the kernel as their exact fp32 images).  Targets up to 2047 labels run on one CTA per utterance
+	with a byte per back-pointer; longer ones (up to 65535 labels) on a thread-block cluster per utterance with 2-bit
+	back-pointers -- the same result wherever both run.  _states_per_cta (tests only) forces the cluster path with that
+	slice size (0: the library's choice)."""
 	half = log_probs.dtype == torch.float16
 	lp = log_probs if log_probs.dtype == torch.float32 else log_probs.float()
 	T, B, C, L, targets, input_lengths, target_lengths = _ctc_args(lp, targets, input_lengths, target_lengths)
 	S = 2 * L + 1
-	bp = torch.empty(B, T, S, dtype = torch.uint8, device = lp.device)
+	lib = _lib.load()
+	cluster = _states_per_cta is not None or S > CTC_ALIGN_CTA_STATES
 	out = torch.empty(B, L, dtype = torch.int64, device = lp.device)
 	if B == 0 or L == 0:
 		return out.zero_()
+	if cluster:
+		nbytes = ctypes.c_int64()
+		_lib.check(lib.cab_ctc_alignment_long_workspace(B, T, L, ctypes.byref(nbytes)), 'cab_ctc_alignment_long_workspace')
+		bp = torch.empty(nbytes.value, dtype = torch.uint8, device = lp.device)
+	else:
+		bp = torch.empty(B, T, S, dtype = torch.uint8, device = lp.device)
 	st, sb, sc = _tbc_strides(lp)
-	tabs = _fp16_tables(lp.device) if half else None
-	rc = _lib.load().cab_ctc_alignment(
-		_p(lp), st, sb, sc, _p(targets), _p(input_lengths), _p(target_lengths), B, T, C, L, blank, _p(bp), _p(out),
-		int(half), _p(tabs[0]) if half else None, _p(tabs[1]) if half else None, _stream()
-	)
-	_lib.check(rc, 'cab_ctc_alignment')
+	tabs = _fp16_tables(lp.device) if half else (None, None)
+	args = (_p(lp), st, sb, sc, _p(targets), _p(input_lengths), _p(target_lengths), B, T, C, L, blank, _p(bp), _p(out), int(half),
+			_p(tabs[0]), _p(tabs[1]))
+	if cluster:
+		_lib.check(lib.cab_ctc_alignment_long(*args, int(_states_per_cta or 0), _stream()), 'cab_ctc_alignment_long')
+	else:
+		_lib.check(lib.cab_ctc_alignment(*args, _stream()), 'cab_ctc_alignment')
 	return out

@@ -392,6 +392,26 @@ int cab_ctc_alignment(const float* log_probs, int64_t stride_t, int64_t stride_b
                       const uint16_t* fp16_exp_table, const uint16_t* fp16_log_table, cab_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * A12, long targets: the same alignment (same arguments, same result wherever both run) for
+ *   L_max <= 65535 (S_max = 2*L_max+1 <= 131071); cab_ctc_alignment stops at S_max <= 4096.
+ *   One thread-block cluster of up to 16 CTAs per utterance, the extended states split into
+ *   contiguous slices, neighbouring slices exchanging their boundary alpha through distributed
+ *   shared memory at every frame; then a back-trace launch (one warp per utterance).
+ *   ws_backptr: packed back-pointers, 2 bits per state, 4 states per byte (state s in bits 2*(s%4)),
+ *   uint8 [B, T, ceil((2*L_max+1)/4)]; cab_ctc_alignment_long_workspace gives its size in bytes
+ *   (host only, no device work) and fails, like cab_ctc_alignment_long, for L_max > 65535.
+ *   states_per_cta: 0 = the library picks the slice size; > 0 (a multiple of 4) forces it, and
+ *   slices beyond 16 CTAs go round-robin over the cluster (at most 8192 states per CTA).
+ * ------------------------------------------------------------------------------------- */
+int cab_ctc_alignment_long_workspace(int B, int T, int L_max, int64_t* bytes);
+int cab_ctc_alignment_long(const float* log_probs, int64_t stride_t, int64_t stride_b,
+                           int64_t stride_c, const int64_t* targets, const int64_t* input_lengths,
+                           const int64_t* target_lengths, int B, int T, int C, int L_max, int blank,
+                           uint8_t* ws_backptr, int64_t* out_alignment, int fp16_arithmetic,
+                           const uint16_t* fp16_exp_table, const uint16_t* fp16_log_table,
+                           int states_per_cta, cab_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * A13: GreedyDecoder.decode (decoders.py:5-16): per-frame top-K class ids of [B, C, T],
  *   out int32 [B, K, T], ordered by descending value, ties -> lowest id first.
  * ------------------------------------------------------------------------------------- */
