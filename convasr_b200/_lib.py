@@ -103,7 +103,13 @@ SIGNATURES = {
 						c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
 	'cab_ctc_loss_bwd': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
 						c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_i64, c_i64, c_i64, c_void_p],
-	'cab_ctc_alignment': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+	'cab_ctc_loss_one_cta_covers': [c_int],
+	'cab_ctc_loss_long_workspace': [c_int, c_int, c_int, ctypes.POINTER(c_i64)],
+	'cab_ctc_loss_long_fwd': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+								c_void_p, c_void_p, c_void_p, c_int, c_void_p],
+	'cab_ctc_loss_long_bwd': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
+								c_void_p, c_void_p, c_void_p, c_void_p, c_i64, c_i64, c_i64, c_int, c_void_p],
+	'cab_ctc_alignment':[c_void_p, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
 						c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
 	'cab_ctc_alignment_long': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
 								c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p],
@@ -114,7 +120,7 @@ SIGNATURES = {
 	'cab_top2_probs': [c_void_p, c_i64, c_i64, c_i64, c_int, c_int, c_int, c_void_p, c_void_p],
 	'cab_entropy': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
 }
-HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
+HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace', 'cab_ctc_loss_one_cta_covers', 'cab_ctc_loss_long_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
 INTROSPECTION = {'cab_abi_version': c_int, 'cab_last_error': ctypes.c_char_p, 'cab_launch_count': c_i64}
 
 

@@ -7,8 +7,9 @@
 // models.entropy / weighted_mean_entropy models.py:645-673.
 //
 // The recursions are T sequential steps, so each utterance gets one CTA with the extended
-// target states across threads and the previous time step in shared memory -- or, for alignments
-// of targets too long for one CTA, one thread-block cluster (ctc_align_cluster_kernel).
+// target states across threads and the previous time step in shared memory -- or, for losses and
+// alignments of targets too long for one CTA, one thread-block cluster (ctc_loss_cluster_kernel,
+// ctc_align_cluster_kernel).
 #include "common.cuh"
 #include "../../include/convasr_b200.h"
 #include <atomic>
@@ -657,6 +658,233 @@ ctc_align_backtrace_kernel(const uint8_t* __restrict__ bp_ws, int64_t pitch, con
 }
 
 // ------------------------------------------------------------------------------------------
+// CTC loss for long targets: one thread-block cluster per utterance and direction, on the geometry of
+// ctc_align_cluster_kernel (slices of W states, slice k in slot k / n of CTA k % n, two guard cells in front of each slot
+// written by the owner of the previous slice through distributed shared memory, one cluster barrier per frame with the
+// next frame's inputs loaded between arrive and wait).  Utterance b recurses over its own input_lengths[b] frames (all
+// CTAs of a cluster share it, so none misses a barrier); "zero" is -inf.  Beta is alpha on the time- and state-reversed
+// problem, as in ctc_recursion_kernel, whose arithmetic this is -- the same lse3_fast calls with the same argument order,
+// re-centring by the maximum of the live values at the end of every kCtcPrefetch-frame sub-block counted from frame 1
+// (and the final partial one), fp64 offsets in the same [B, 2, G_cap] table -- so the nll is bit-identical wherever both
+// kernels run.  The maximum is taken over the cluster: at the end of a sub-block every CTA stores its block maximum into
+// entry c of a 16-entry array on every CTA (two arrays, by sub-block parity) before it arrives; after the wait every CTA
+// reduces the same values.  The shift is applied as the values are read at the next frame (v - m: the rounding of the
+// one-CTA kernel's in-place subtraction), to the slice and its guard cells alike, so it needs no pass or barrier of its own.
+// MODE 0: alpha, nll and offsets only.  MODE 1: also stores the re-centred alpha into ws [B, T, S_max].
+// MODE 2: beta plus the gradient.  At every frame it reads that frame's stored alpha row (loaded a frame ahead, like the
+// emissions) and subtracts exp(alpha + beta + (O_alpha + O_beta - ll) - lp) * go -- ctc_grad_scatter_kernel's formula --
+// from grad (already exp(lp) * go from ctc_grad_init_kernel): atomics for label states; blank occupancies are summed per
+// CTA in shared memory and added with one atomic per CTA and frame after the barrier.
+// ------------------------------------------------------------------------------------------
+template <int MODE>
+__global__ void __launch_bounds__(1024, 1)
+ctc_loss_cluster_kernel(const float* __restrict__ lp, int64_t st, int64_t sb, int64_t sc, const int64_t* __restrict__ targets,
+                        const int64_t* __restrict__ in_len, const int64_t* __restrict__ tgt_len, int T, int L_max, int blank,
+                        int W, int n_slots, float* __restrict__ ws, double* __restrict__ off_ws, int G_cap,
+                        float* __restrict__ nll, const float* __restrict__ go, float* __restrict__ grad, int64_t gt, int64_t gb,
+                        int64_t gc) {
+    constexpr bool rev = MODE == 2;
+    extern __shared__ float sh[];
+    const int n = (int)cluster_nctarank(), c = (int)cluster_ctarank();
+    const int b = blockIdx.x / n;
+    const int S_max = 2 * L_max + 1;
+    const int tl = (int)tgt_len[b];
+    const int il = (int)in_len[b];
+    const int S = 2 * tl + 1;
+    double* off = off_ws + ((int64_t)b * 2 + (rev ? 1 : 0)) * G_cap;
+    if (il <= 0 || il > T || tl > L_max || tl < 0) {  // the same for every CTA of the cluster: all leave before any barrier
+        if (!rev && c == 0 && threadIdx.x == 0) {
+            nll[b] = INFINITY;
+            off[G_cap - 1] = -(double)INFINITY;
+        }
+        return;
+    }
+    const int slot_len = W + 2;
+    const int buf_len = n_slots * slot_len;
+    float* s_max = sh + 2 * buf_len;                // [2][kAlignClusterMax] block maxima of the cluster, by sub-block parity
+    float* s_red = s_max + 2 * kAlignClusterMax;    // [32] warp maxima
+    float* s_misc = s_red + 32;                     // [2] alpha of states S-1, S-2 at the last frame (CTA 0) / blank sums by frame parity
+    const int gps = W >> 2;                         // groups per slice
+    const int n_groups = n_slots * gps;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+    const int64_t* tg = targets + (int64_t)b * L_max;
+    const float* lp0 = lp + (int64_t)b * sb + (int64_t)(rev ? il - 1 : 0) * st;  // virtual frame 0
+    const int64_t st_v = rev ? -st : st;
+
+    for (int i = threadIdx.x; i < 2 * buf_len; i += blockDim.x) sh[i] = -INFINITY;
+    if (threadIdx.x < 2) s_misc[threadIdx.x] = rev ? 0.f : -INFINITY;
+    if (c == 0 && threadIdx.x == 0) off[0] = 0.0;
+
+    // virtual state s (recursion order) is real state rev ? S-1-s : s; S is odd, so even virtual states are blanks
+    auto label = [&](int s) { return (int)tg[(rev ? S - 1 - s : s) >> 1]; };
+    int loc[kAlignGroupsPer], s0[kAlignGroupsPer], lab1[kAlignGroupsPer], lab3[kAlignGroupsPer];
+    bool live[kAlignGroupsPer], skip1[kAlignGroupsPer], skip3[kAlignGroupsPer];
+    float* next_guard[kAlignGroupsPer];  // guard cells of slice k+1 in buffer 0 (buffer 1: + buf_len), or nullptr
+#pragma unroll
+    for (int i = 0; i < kAlignGroupsPer; ++i) {
+        const int g = threadIdx.x + i * blockDim.x;
+        const int j = g / gps, o = (g - j * gps) * 4, k = j * n + c;
+        s0[i] = k * W + o;
+        live[i] = g < n_groups && s0[i] < S;
+        loc[i] = j * slot_len + 2 + o;
+        lab1[i] = lab3[i] = blank;
+        skip1[i] = skip3[i] = false;
+        next_guard[i] = nullptr;
+        if (!live[i]) continue;
+        if (s0[i] + 1 < S) {  // a label state may skip from the one two behind when the labels differ
+            lab1[i] = label(s0[i] + 1);
+            skip1[i] = s0[i] >= 2 && lab1[i] != label(s0[i] - 1);
+        }
+        if (s0[i] + 3 < S) {
+            lab3[i] = label(s0[i] + 3);
+            skip3[i] = lab3[i] != lab1[i];
+        }
+        const int k1 = k + 1;
+        if (o == W - 4 && k1 < n * n_slots) next_guard[i] = cluster_map(sh + (k1 / n) * slot_len, (uint32_t)(k1 % n));
+    }
+
+    float eb[kAlignGroupsPer], e1[kAlignGroupsPer], e3[kAlignGroupsPer];
+    auto load_e = [&](int u) {
+        const float* r = lp0 + (int64_t)u * st_v;
+#pragma unroll
+        for (int i = 0; i < kAlignGroupsPer; ++i)
+            if (live[i]) {
+                eb[i] = r[(int64_t)blank * sc];
+                e1[i] = r[(int64_t)lab1[i] * sc];
+                e3[i] = r[(int64_t)lab3[i] * sc];
+            }
+    };
+    // MODE 2: the stored alpha of the frame (real states S-1-s0 .. S-4-s0) and its offset
+    float al[kAlignGroupsPer][4];
+    double oa = 0.0, ll = 0.0;
+    float g_out = 0.f;
+    const double* off_a = off_ws + (int64_t)b * 2 * G_cap;
+    auto load_a = [&](int u) {
+        const int t = il - 1 - u;
+        const float* row = ws + ((int64_t)b * T + t) * S_max + (S - 1);
+#pragma unroll
+        for (int i = 0; i < kAlignGroupsPer; ++i)
+            if (live[i]) {
+#pragma unroll
+                for (int q = 0; q < 4; ++q) al[i][q] = s0[i] + q < S ? row[-(s0[i] + q)] : 0.f;
+            }
+        oa = off_a[t == 0 ? 0 : (t - 1) / kCtcPrefetch];
+    };
+    if (rev) {
+        ll = off_a[G_cap - 1];
+        g_out = go[b];
+    }
+
+    cluster_arrive();  // every CTA of the cluster has started and initialised its buffers
+    load_e(0);
+    if (rev) load_a(0);
+    cluster_wait();
+
+    double O = 0.0;
+    float shift = 0.f;  // re-centring still to be applied to the values of the previous frame
+    for (int u = 0; u < il; ++u) {
+        const float* prev = sh + ((u + 1) & 1) * buf_len;
+        float* cur = sh + (u & 1) * buf_len;
+        const int t = rev ? il - 1 - u : u;  // real frame
+        const float nl = rev ? (float)(oa + O - ll) : 0.f;
+        float* gr = rev ? grad + (int64_t)t * gt + (int64_t)b * gb : nullptr;
+        float* wrow = MODE == 1 ? ws + ((int64_t)b * T + t) * S_max : nullptr;
+        float mloc = -INFINITY, bacc = 0.f;
+#pragma unroll
+        for (int i = 0; i < kAlignGroupsPer; ++i) {
+            if (!live[i]) continue;
+            float v[4];
+            if (u == 0) {
+                v[0] = s0[i] == 0 ? eb[i] : -INFINITY;
+                v[1] = s0[i] == 0 && S > 1 ? e1[i] : -INFINITY;
+                v[2] = v[3] = -INFINITY;
+            } else {
+                const float* p = prev + loc[i];
+                const float am1 = p[-1] - shift, a0 = p[0] - shift, a1 = p[1] - shift, a2 = p[2] - shift, a3 = p[3] - shift;
+                // all four states unconditionally; states >= S of the last live group are never read by a live state
+                v[0] = lse3_fast(a0, am1, -INFINITY) + eb[i];
+                v[1] = lse3_fast(a1, a0, skip1[i] ? am1 : -INFINITY) + e1[i];
+                v[2] = lse3_fast(a2, a1, -INFINITY) + eb[i];
+                v[3] = lse3_fast(a3, a2, skip3[i] ? a1 : -INFINITY) + e3[i];
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) cur[loc[i] + q] = v[q];
+            if (next_guard[i]) {
+                float* gd = next_guard[i] + (u & 1) * buf_len;
+                gd[0] = v[2];
+                gd[1] = v[3];
+            }
+            const int nv = S - s0[i];  // live states of the group (>= 1)
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+                if (q < nv) {
+                    mloc = fmaxf(mloc, v[q]);
+                    if (MODE == 1) wrow[s0[i] + q] = v[q];
+                    if (MODE == 2) {
+                        const float e = (q & 1) ? (q == 1 ? e1[i] : e3[i]) : eb[i];
+                        const float occ = expf((al[i][q] + v[q]) + nl - e);
+                        if (q & 1) atomicAdd(gr + (int64_t)(q == 1 ? lab1[i] : lab3[i]) * gc, -occ * g_out);
+                        else bacc += occ;
+                    }
+                }
+        }
+        if (rev) {
+            bacc = warp_sum(bacc);
+            if (lane == 0) atomicAdd(s_misc + (u & 1), bacc);
+        }
+        const bool block_end = u >= 1 && (u % kCtcPrefetch == 0 || u == il - 1);
+        const int par = ((u - 1) / kCtcPrefetch) & 1;
+        if (block_end) {
+            mloc = warp_max(mloc);
+            if (lane == 0) s_red[warp] = mloc;
+            __syncthreads();
+            if (warp == 0) {
+                float m = s_red[lane < n_warps ? lane : 0];
+                m = warp_max(m);
+                if (lane < n) *cluster_map(s_max + par * kAlignClusterMax + c, (uint32_t)lane) = m;
+            }
+        }
+        cluster_arrive();
+        if (u + 1 < il) {
+            load_e(u + 1);
+            if (rev) load_a(u + 1);
+        }
+        cluster_wait();
+        if (rev && threadIdx.x == 0) {
+            const float s = s_misc[u & 1];
+            s_misc[u & 1] = 0.f;
+            atomicAdd(gr + (int64_t)blank * gc, -s * g_out);
+        }
+        shift = 0.f;
+        if (block_end) {
+            float m = s_max[par * kAlignClusterMax];
+            for (int r = 1; r < n; ++r) m = fmaxf(m, s_max[par * kAlignClusterMax + r]);
+            if (m > -INFINITY && m < INFINITY) {
+                shift = m;
+                O += (double)m;
+            }
+            if (c == 0 && threadIdx.x == 0) off[(u - 1) / kCtcPrefetch + 1] = O;
+        }
+    }
+    if (rev) return;
+
+    // log-likelihood from states S-1 and S-2 of the last frame, re-centred: both values meet on CTA 0
+    if (threadIdx.x < 2) {
+        const int x = S - 1 - (int)threadIdx.x;  // S == 1: state -1 keeps -inf
+        const int k = x / W;
+        if (x >= 0 && k % n == c)
+            *cluster_map(s_misc + threadIdx.x, 0) = sh[((il - 1) & 1) * buf_len + (k / n) * slot_len + 2 + (x - k * W)] - shift;
+    }
+    cluster_arrive();
+    cluster_wait();
+    if (c == 0 && threadIdx.x == 0) {
+        const double l = (double)lse2(s_misc[0], s_misc[1]) + O;
+        nll[b] = (float)(-l);
+        off[G_cap - 1] = l;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // log_softmax + argmax over dim 1 of [B, C, T]; block = (32 t) x (8 class groups)
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
@@ -939,12 +1167,23 @@ static int ctc_threads(int S_max) {
     return th;
 }
 
-// shared memory of ctc_recursion_kernel for a staging depth of G steps; picks the deepest that fits
-static int ctc_rec_config(int S_max, int* G_out, size_t* smem_out) {
+// shared memory of ctc_recursion_kernel for a staging depth of G steps
+constexpr size_t kCtcRecSmemBudget = 200 * 1024;
+static size_t ctc_rec_bytes(int S_max, int G) {
     const int S_pad = S_max | 1;
+    return sizeof(float) * (2 * (size_t)(S_max + 2) + 32 + (size_t)S_max + 2 * (size_t)G * S_pad);
+}
+// does ctc_recursion_kernel take targets of L_max labels (at least kCtcPrefetch staged frames in shared memory)?
+static bool ctc_one_cta_covers(int L_max) {
+    const int S_max = 2 * L_max + 1;
+    return L_max >= 0 && S_max <= kCtcMaxPer * 1024 && ctc_rec_bytes(S_max, kCtcPrefetch) <= kCtcRecSmemBudget;
+}
+
+// picks the deepest staging that fits
+static int ctc_rec_config(int S_max, int* G_out, size_t* smem_out) {
     for (int G = 32; G >= kCtcPrefetch; G >>= 1) {
-        const size_t bytes = sizeof(float) * (2 * (size_t)(S_max + 2) + 32 + (size_t)S_max + 2 * (size_t)G * S_pad);
-        if (bytes <= 200 * 1024) {
+        const size_t bytes = ctc_rec_bytes(S_max, G);
+        if (bytes <= kCtcRecSmemBudget) {
             *G_out = G;
             *smem_out = bytes;
             static size_t attr_set = 0;
@@ -1073,6 +1312,33 @@ extern "C" int cab_ctc_alignment_long_workspace(int B, int T, int L_max, int64_t
     return 0;
 }
 
+// How the cluster kernels split S_max extended states: n CTAs, slices of W states (W % 4 == 0), n_slots slices per CTA.
+// states_per_cta > 0 forces W, with slices round-robin over up to kAlignClusterMax CTAs; 0 gives one slice per CTA of
+// at most ~2048 states.
+static int ctc_cluster_geometry(int S_max, int states_per_cta, int* n_out, int* W_out, int* n_slots_out, int* threads_out) {
+    int n, W, n_slots;
+    if (states_per_cta > 0) {
+        W = states_per_cta;
+        const int n_slices = (S_max + W - 1) / W;
+        n = n_slices < kAlignClusterMax ? n_slices : kAlignClusterMax;
+        n_slots = (n_slices + n - 1) / n;
+    } else {
+        n = (S_max + 2047) / 2048;
+        if (n > kAlignClusterMax) n = kAlignClusterMax;
+        W = 4 * (((S_max + 3) / 4 + n - 1) / n);
+        n_slots = 1;
+    }
+    CAB_CHECK_ARG((int64_t)n_slots * W <= kAlignCtaStates, "states_per_cta=%d puts %lld states on one CTA (at most %d)", states_per_cta,
+                  (long long)n_slots * W, kAlignCtaStates);
+    const int groups = n_slots * W / 4;
+    const int per = groups > 1024 ? kAlignGroupsPer : 1;
+    *n_out = n;
+    *W_out = W;
+    *n_slots_out = n_slots;
+    *threads_out = ((groups + per - 1) / per + 31) / 32 * 32;
+    return 0;
+}
+
 template <bool HALF>
 static int launch_align_cluster(int n, int threads, size_t smem, cudaStream_t stream, int B, const float* log_probs, int64_t st,
                                 int64_t sb, int64_t sc, const int64_t* targets, const int64_t* input_lengths,
@@ -1121,23 +1387,8 @@ extern "C" int cab_ctc_alignment_long(const float* log_probs, int64_t stride_t, 
     if (L_max == 0) return 0;  // out has no element
     const int S_max = 2 * L_max + 1;
     const int G4 = (S_max + 3) / 4;  // bytes per packed row
-    int n, W, n_slots;
-    if (states_per_cta > 0) {  // forced slice size: slices round-robin over up to kAlignClusterMax CTAs
-        W = states_per_cta;
-        const int n_slices = (S_max + W - 1) / W;
-        n = n_slices < kAlignClusterMax ? n_slices : kAlignClusterMax;
-        n_slots = (n_slices + n - 1) / n;
-    } else {  // one slice per CTA of at most ~2048 states
-        n = (S_max + 2047) / 2048;
-        if (n > kAlignClusterMax) n = kAlignClusterMax;
-        W = 4 * ((G4 + n - 1) / n);
-        n_slots = 1;
-    }
-    CAB_CHECK_ARG((int64_t)n_slots * W <= kAlignCtaStates, "states_per_cta=%d puts %lld states on one CTA (at most %d)", states_per_cta,
-                  (long long)n_slots * W, kAlignCtaStates);
-    const int groups = n_slots * W / 4;
-    const int per = groups > 1024 ? kAlignGroupsPer : 1;
-    const int threads = ((groups + per - 1) / per + 31) / 32 * 32;
+    int n, W, n_slots, threads;
+    if (ctc_cluster_geometry(S_max, states_per_cta, &n, &W, &n_slots, &threads) != 0) return -1;
     const size_t smem = sizeof(float) * (2 * (size_t)n_slots * (W + 2) + 2);
     int rc = fp16_arithmetic
                  ? launch_align_cluster<true>(n, threads, smem, stream, B, log_probs, stride_t, stride_b, stride_c, targets, input_lengths,
@@ -1148,6 +1399,105 @@ extern "C" int cab_ctc_alignment_long(const float* log_probs, int64_t stride_t, 
     if (rc != 0) return rc;
     ctc_align_backtrace_kernel<<<B, 32, 0, stream>>>(ws_backptr, G4, input_lengths, T, L_max, out_alignment);
     CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(2, std::memory_order_relaxed);
+    return 0;
+}
+
+extern "C" int cab_ctc_loss_one_cta_covers(int L_max) { return ctc_one_cta_covers(L_max) ? 1 : 0; }
+
+extern "C" int cab_ctc_loss_long_workspace(int B, int T, int L_max, int64_t* bytes) {
+    CAB_CHECK_ARG(bytes != nullptr, "null output");
+    CAB_CHECK_ARG(B > 0 && T > 0 && L_max >= 0, "bad shape B=%d T=%d L=%d", B, T, L_max);
+    CAB_CHECK_ARG(L_max <= kAlignLongMaxL, "target too long: L_max=%d (the cluster CTC loss handles L_max <= %d)", L_max, kAlignLongMaxL);
+    *bytes = (int64_t)sizeof(float) * B * T * (2 * (int64_t)L_max + 1);
+    return 0;
+}
+
+// one launch of ctc_loss_cluster_kernel<MODE>, B clusters of n CTAs
+template <int MODE>
+static int launch_loss_cluster(int states_per_cta, cudaStream_t stream, const float* log_probs, int64_t st, int64_t sb, int64_t sc,
+                               const int64_t* targets, const int64_t* input_lengths, const int64_t* target_lengths, int B, int T,
+                               int L_max, int blank, float* ws, double* ws_offsets, float* nll, const float* grad_out, float* grad,
+                               int64_t gt, int64_t gb, int64_t gc) {
+    int n, W, n_slots, threads;
+    if (ctc_cluster_geometry(2 * L_max + 1, states_per_cta, &n, &W, &n_slots, &threads) != 0) return -1;
+    // two frame buffers of n_slots * (W + 2) values, block maxima [2][16], warp maxima [32], two scalars
+    const size_t smem = sizeof(float) * (2 * (size_t)n_slots * (W + 2) + 2 * kAlignClusterMax + 32 + 2);
+    auto kernel = ctc_loss_cluster_kernel<MODE>;
+    static size_t smem_set = 0;
+    if (smem_set == 0) CAB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    if (smem > smem_set) {
+        CAB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        smem_set = smem;
+    }
+    cudaLaunchConfig_t cfg = {};
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = n;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.gridDim = dim3(B * n);
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    int clusters = 0;
+    CAB_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg));
+    CAB_CHECK_ARG(clusters > 0, "a cluster of %d CTAs x %d threads with %zu B of shared memory does not fit this device", n, threads, smem);
+    const int G_cap = (T + kCtcPrefetch - 1) / kCtcPrefetch + 2;
+    CAB_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, log_probs, st, sb, sc, targets, input_lengths, target_lengths, T, L_max, blank, W,
+                                      n_slots, ws, ws_offsets, G_cap, nll, grad_out, grad, gt, gb, gc));
+    return 0;
+}
+
+#define CTC_LONG_CHECKS()                                                                                                  \
+    CAB_CHECK_ARG(log_probs && targets && input_lengths && target_lengths, "null pointer argument");                      \
+    CAB_CHECK_ARG(B > 0 && T > 0 && C > 0 && L_max >= 0, "bad shape B=%d T=%d C=%d L=%d", B, T, C, L_max);                \
+    CAB_CHECK_ARG(blank >= 0 && blank < C, "blank=%d out of range", blank);                                                \
+    CAB_CHECK_ARG(L_max <= kAlignLongMaxL, "target too long: L_max=%d (the cluster CTC loss handles L_max <= %d)", L_max, \
+                  kAlignLongMaxL);                                                                                         \
+    CAB_CHECK_ARG(states_per_cta >= 0 && states_per_cta % 4 == 0, "states_per_cta=%d must be 0 or a positive multiple of 4", \
+                  states_per_cta);
+
+extern "C" int cab_ctc_loss_long_fwd(const float* log_probs, int64_t stride_t, int64_t stride_b, int64_t stride_c,
+                                     const int64_t* targets, const int64_t* input_lengths, const int64_t* target_lengths, int B,
+                                     int T, int C, int L_max, int blank, float* ws_alpha, double* ws_offsets, float* nll,
+                                     int states_per_cta, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CTC_LONG_CHECKS();
+    CAB_CHECK_ARG(ws_offsets && nll, "null workspace/output");
+    const int rc = ws_alpha ? launch_loss_cluster<1>(states_per_cta, stream, log_probs, stride_t, stride_b, stride_c, targets, input_lengths,
+                                                     target_lengths, B, T, L_max, blank, ws_alpha, ws_offsets, nll, nullptr, nullptr, 0, 0, 0)
+                            : launch_loss_cluster<0>(states_per_cta, stream, log_probs, stride_t, stride_b, stride_c, targets, input_lengths,
+                                                     target_lengths, B, T, L_max, blank, nullptr, ws_offsets, nll, nullptr, nullptr, 0, 0, 0);
+    if (rc != 0) return rc;
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
+
+extern "C" int cab_ctc_loss_long_bwd(const float* log_probs, int64_t stride_t, int64_t stride_b, int64_t stride_c,
+                                     const int64_t* targets, const int64_t* input_lengths, const int64_t* target_lengths, int B,
+                                     int T, int C, int L_max, int blank, const float* ws_alpha, double* ws_offsets,
+                                     const float* grad_out, float* grad, int64_t gstride_t, int64_t gstride_b, int64_t gstride_c,
+                                     int states_per_cta, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CTC_LONG_CHECKS();
+    CAB_CHECK_ARG(ws_alpha && ws_offsets && grad_out && grad, "null workspace/output");
+    int n_, W_, n_slots_, threads_;  // a refused split launches nothing
+    if (ctc_cluster_geometry(2 * L_max + 1, states_per_cta, &n_, &W_, &n_slots_, &threads_) != 0) return -1;
+    {
+        const int64_t n = (int64_t)B * T * C;
+        int blocks = (int)((n + 255) / 256);
+        if (blocks > 148 * 16) blocks = 148 * 16;
+        ctc_grad_init_kernel<<<blocks, 256, 0, stream>>>(log_probs, stride_t, stride_b, stride_c, input_lengths, grad_out, B, T, C, grad,
+                                                         gstride_t, gstride_b, gstride_c);
+        CAB_CHECK_LAUNCH();
+    }
+    const int rc = launch_loss_cluster<2>(states_per_cta, stream, log_probs, stride_t, stride_b, stride_c, targets, input_lengths,
+                                          target_lengths, B, T, L_max, blank, const_cast<float*>(ws_alpha), ws_offsets, nullptr, grad_out,
+                                          grad, gstride_t, gstride_b, gstride_c);
+    if (rc != 0) return rc;
     g_launch_count.fetch_add(2, std::memory_order_relaxed);
     return 0;
 }

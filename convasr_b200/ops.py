@@ -380,10 +380,33 @@ def _ctc_args(log_probs, targets, input_lengths, target_lengths):
 
 class _CtcLoss(torch.autograd.Function):
 	@staticmethod
-	def forward(ctx, log_probs, targets, input_lengths, target_lengths, blank):
+	def forward(ctx, log_probs, targets, input_lengths, target_lengths, blank, states_per_cta):
 		lp = log_probs if log_probs.dtype == torch.float32 else log_probs.float()
 		T, B, C, L, targets, input_lengths, target_lengths = _ctc_args(lp, targets, input_lengths, target_lengths)
 		S = 2 * L + 1
+		lib = _lib.load()
+		ctx.blank = blank
+		ctx.in_dtype = log_probs.dtype
+		ctx.states_per_cta = states_per_cta
+		if states_per_cta is not None or not lib.cab_ctc_loss_one_cta_covers(L):
+			# one thread-block cluster per utterance: alpha is stored only when a gradient will be wanted, beta is
+			# recomputed by the backward
+			alpha = None
+			if ctx.needs_input_grad[0]:
+				nbytes = ctypes.c_int64()
+				_lib.check(lib.cab_ctc_loss_long_workspace(B, T, L, ctypes.byref(nbytes)), 'cab_ctc_loss_long_workspace')
+				alpha = torch.empty(nbytes.value // 4, dtype = torch.float32, device = lp.device)
+			nll = torch.empty(B, dtype = torch.float32, device = lp.device)
+			offsets = torch.empty(B, 2, (T + 7) // 8 + 2, dtype = torch.float64, device = lp.device)
+			st, sb, sc = _tbc_strides(lp)
+			rc = lib.cab_ctc_loss_long_fwd(
+				_p(lp), st, sb, sc, _p(targets), _p(input_lengths), _p(target_lengths), B, T, C, L, blank, _p(alpha), _p(offsets),
+				_p(nll), int(states_per_cta or 0), _stream()
+			)
+			_lib.check(rc, 'cab_ctc_loss_long_fwd')
+			ctx.cluster = True
+			ctx.save_for_backward(lp, targets, input_lengths, target_lengths, alpha, offsets)
+			return nll
 		alpha = torch.empty(B, T, S, dtype = torch.float32, device = lp.device)
 		# when a gradient will be wanted, alpha and beta run concurrently in one launch
 		beta = torch.empty_like(alpha) if ctx.needs_input_grad[0] else None
@@ -397,8 +420,7 @@ class _CtcLoss(torch.autograd.Function):
 		_lib.check(rc, 'cab_ctc_loss_fwd')
 		ctx.beta = beta
 		ctx.save_for_backward(lp, targets, input_lengths, target_lengths, alpha, offsets)
-		ctx.blank = blank
-		ctx.in_dtype = log_probs.dtype
+		ctx.cluster = False
 		return nll
 
 	@staticmethod
@@ -406,6 +428,16 @@ class _CtcLoss(torch.autograd.Function):
 		lp, targets, input_lengths, target_lengths, alpha, offsets = ctx.saved_tensors
 		T, B, C = lp.shape
 		L = targets.shape[1]
+		if ctx.cluster:
+			grad = torch.empty_strided(lp.shape, lp.stride(), dtype = torch.float32, device = lp.device)
+			st, sb, sc = _tbc_strides(lp)
+			go = grad_out.to(torch.float32).contiguous()
+			rc = _lib.load().cab_ctc_loss_long_bwd(
+				_p(lp), st, sb, sc, _p(targets), _p(input_lengths), _p(target_lengths), B, T, C, L, ctx.blank, _p(alpha), _p(offsets),
+				_p(go), _p(grad), grad.stride(0), grad.stride(1), grad.stride(2), int(ctx.states_per_cta or 0), _stream()
+			)
+			_lib.check(rc, 'cab_ctc_loss_long_bwd')
+			return grad.to(ctx.in_dtype), None, None, None, None, None
 		beta_ready = ctx.beta is not None
 		beta = ctx.beta if beta_ready else torch.empty_like(alpha)
 		ctx.beta = None
@@ -418,12 +450,15 @@ class _CtcLoss(torch.autograd.Function):
 			_p(beta), int(beta_ready), _p(offsets), _p(go), _p(grad), grad.stride(0), grad.stride(1), grad.stride(2), _stream()
 		)
 		_lib.check(rc, 'cab_ctc_loss_bwd')
-		return grad.to(ctx.in_dtype), None, None, None, None
+		return grad.to(ctx.in_dtype), None, None, None, None, None
 
 
-def ctc_loss(log_probs, targets, input_lengths, target_lengths, blank = 0):
-	"""F.ctc_loss(log_probs[T,B,C], targets[B,L], ..., reduction='none', zero_infinity=False)."""
-	return _CtcLoss.apply(log_probs, targets, input_lengths, target_lengths, int(blank))
+def ctc_loss(log_probs, targets, input_lengths, target_lengths, blank = 0, _states_per_cta = None):
+	"""F.ctc_loss(log_probs[T,B,C], targets[B,L], ..., reduction='none', zero_infinity=False).  Targets up to 1345 labels
+	run on one CTA per utterance and direction; longer ones (up to 65535 labels) on a thread-block cluster per utterance,
+	with one fp32 [B, T, 2L+1] workspace when a gradient is wanted and none for the loss alone -- the same nll bit for bit
+	wherever both run.  _states_per_cta (tests only) forces the cluster path with that slice size (0: the library's choice)."""
+	return _CtcLoss.apply(log_probs, targets, input_lengths, target_lengths, int(blank), _states_per_cta)
 
 
 _FP16_TABLES = {}

@@ -374,6 +374,36 @@ int cab_ctc_loss_bwd(const float* log_probs, int64_t stride_t, int64_t stride_b,
                      int64_t gstride_c, cab_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * A11, long targets: the same loss and gradient for L_max <= 65535 (about an hour of speech).
+ *   cab_ctc_loss_fwd/bwd take a batch when cab_ctc_loss_one_cta_covers(L_max) returns 1 (host only:
+ *   L_max <= 1345, where one CTA stages 8 frames of emissions in shared memory); beyond, these run
+ *   one thread-block cluster of up to 16 CTAs per utterance and direction, the extended states in
+ *   contiguous slices, neighbouring slices exchanging boundary values through distributed shared
+ *   memory at every frame.  The nll is bit-identical to cab_ctc_loss_fwd wherever both run; the
+ *   gradient differs only in the order of its atomic additions.
+ *   ws_alpha: fp32 [B, T, 2*L_max+1], cab_ctc_loss_long_workspace gives its size in bytes (host only,
+ *   64-bit; fails for L_max > 65535).  cab_ctc_loss_long_fwd with ws_alpha NULL computes the loss
+ *   only and needs no [B, T, S] workspace; with ws_alpha it stores alpha for cab_ctc_loss_long_bwd,
+ *   which recomputes beta and writes the gradient without a second workspace.  ws_offsets, nll,
+ *   grad and the strides as for cab_ctc_loss_fwd/bwd; ws_offsets carries the forward's offsets and
+ *   log-likelihood to the backward.  states_per_cta as for cab_ctc_alignment_long.  No host
+ *   synchronisation and no allocation: both can be captured into a CUDA graph.
+ * ------------------------------------------------------------------------------------- */
+int cab_ctc_loss_one_cta_covers(int L_max);
+int cab_ctc_loss_long_workspace(int B, int T, int L_max, int64_t* bytes);
+int cab_ctc_loss_long_fwd(const float* log_probs, int64_t stride_t, int64_t stride_b, int64_t stride_c,
+                          const int64_t* targets, const int64_t* input_lengths,
+                          const int64_t* target_lengths, int B, int T, int C, int L_max, int blank,
+                          float* ws_alpha_or_null, double* ws_offsets, float* nll, int states_per_cta,
+                          cab_stream_t stream);
+int cab_ctc_loss_long_bwd(const float* log_probs, int64_t stride_t, int64_t stride_b, int64_t stride_c,
+                          const int64_t* targets, const int64_t* input_lengths,
+                          const int64_t* target_lengths, int B, int T, int C, int L_max, int blank,
+                          const float* ws_alpha, double* ws_offsets, const float* grad_out, float* grad,
+                          int64_t gstride_t, int64_t gstride_b, int64_t gstride_c, int states_per_cta,
+                          cab_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * A12: forced alignment, ctc.alignment (ctc.py:6-75) with all of its quirks: finite "zero"
  *   (finfo.min), logsumexp alpha with argmax back-pointers (stay preferred on ties), the
  *   recursion runs over all T frames of the padded batch, terminal state read at global T-1,
