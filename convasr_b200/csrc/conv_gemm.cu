@@ -21,7 +21,6 @@
 #include "../../include/convasr_b200.h"
 #include <mutex>
 #include <atomic>
-#include <cstdlib>
 
 namespace cab {
 
@@ -73,11 +72,6 @@ struct alignas(64) ConvParams {
     // per-row log-sum-exp and argmax from an online softmax across the N tiles of an M tile (M-tile-major schedule)
     float* lse;
     int mtile_major;
-    // dynamic tile scheduling: units (tiles, or M tiles when mtile_major) are claimed with atomicAdd on this zeroed counter
-    // instead of the static blockIdx.x + i * gridDim.x walk -- a CTA that starts late (its SM was busy with another kernel,
-    // e.g. an NCCL all-reduce of the data-parallel step) simply claims fewer units instead of delaying the whole launch.
-    // null = static schedule.
-    int* tile_counter;
     // rows t >= ceil(skip_frac[b] * skip_T) + skip_margin of utterance b are structural zeros (padding of a
     // ragged batch): M tiles that lie entirely there are not computed, the epilogue stores zeros
     const float* skip_frac;
@@ -88,7 +82,6 @@ struct alignas(64) ConvParams {
     // the BatchNorm backward will read), the epilogue accumulates sum(dz) and sum(dz * y) per channel, dz = g * act'(y*scale +
     // shift) * (t < len_b), into fp64 partials [CAB_BN_SUM_REPLICAS][2][bnr_C]: the separate reduce pass over (y, g) -- two of the
     // five activation-sized passes of the BatchNorm backward -- disappears.
-    int stats_columns;       // forward statistics: column-parallel pass over the staged tile (default) or the per-row shuffle butterfly
     CUtensorMap ymap;
     const float* bnr_ss;     // [4][bnr_C]: scale, shift, (mean, invstd)
     const float* bnr_xlen;   // temporal mask of the layer (or null)
@@ -107,51 +100,19 @@ __device__ __forceinline__ int live_mtiles(const ConvParams& p, int b) {
 }
 // Unit sequence of one CTA.  A unit is a tile (N tile fastest: neighbouring units share the A tile in L2), or -- mtile_major --
 // one compacted M tile whose N tiles the CTA then walks in order (the online softmax of the large-vocabulary head needs every
-// class of a row in one CTA).  Static schedule: unit j of this CTA = blockIdx.x + j * gridDim.x.  Dynamic schedule: the
-// producer thread claims units with atomicAdd and publishes them to the MMA / epilogue warps through a 4-deep shared-memory
-// ring (full / empty mbarriers); every role then derives (am, nt) and its TileCursor position from the same unit index.
-constexpr int kSched = 4;
-struct SchedRing {
-    int* unit;          // [kSched]
-    uint64_t* full;     // [kSched], 1 arrival (producer)
-    uint64_t* empty;    // [kSched], 1 (MMA thread) + 4 (epilogue warps) arrivals
-};
-// The producer claims one unit AHEAD: the atomicAdd for unit j + 1 is issued when unit j is published and its result is first
-// needed a whole tile later, so the ~1 us round trip of the global atomic never sits on the producer's critical path.
-__device__ __forceinline__ int sched_produce(const ConvParams& p, const SchedRing& r, int j, int& ahead) {
-    if (p.tile_counter == nullptr) return blockIdx.x + j * gridDim.x;
-    const int slot = j % kSched;
-    const int u = j == 0 ? atomicAdd(p.tile_counter, 1) : ahead;
-    mbar_wait(&r.empty[slot], ((j / kSched) & 1) ^ 1);
-    r.unit[slot] = u;
-    mbar_arrive(&r.full[slot]);  // release: the slot's value is visible to whoever acquires the barrier
-    ahead = atomicAdd(p.tile_counter, 1);
-    return u;
-}
-template <bool WARP>  // WARP: called by all 32 lanes of a warp (one arrival per warp), else by a single thread
-__device__ __forceinline__ int sched_consume(const ConvParams& p, const SchedRing& r, int j, int lane) {
-    if (p.tile_counter == nullptr) return blockIdx.x + j * gridDim.x;
-    const int slot = j % kSched;
-    mbar_wait(&r.full[slot], (j / kSched) & 1);
-    const int u = r.unit[slot];
-    if (WARP) {
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&r.empty[slot]);
-    } else {
-        mbar_arrive(&r.empty[slot]);
-    }
-    return u;
-}
-// next (am, nt) of a role's walk; `u`, `nt_next`, `j` are the role's private state
-#define CAB_NEXT_UNIT(FETCH)                                                   \
+// class of a row in one CTA).  Unit j of this CTA is blockIdx.x + j * gridDim.x; every role walks this sequence on its own
+// and derives (am, nt) and its TileCursor position from it.  An atomic-claim schedule, where late CTAs take fewer units, was
+// measured 1 % slower on the training step on one B200 and 3 % slower on eight (profiles/r02_tile_schedule_ab.md).
+// next (am, nt) of a role's walk; `u` (starts at blockIdx.x - gridDim.x) and `nt_next` (starts at 0) are the role's private state
+#define CAB_NEXT_UNIT()                                                        \
     int am, nt;                                                                \
     if (p.mtile_major) {                                                       \
-        if (nt_next == 0) u = (FETCH);                                         \
+        if (nt_next == 0) u += gridDim.x;                                      \
         am = u;                                                                \
         nt = nt_next;                                                          \
         nt_next = nt_next + 1 == p.n_ntiles ? 0 : nt_next + 1;                 \
     } else {                                                                   \
-        u = (FETCH);                                                           \
+        u += gridDim.x;                                                        \
         nt = u % p.n_ntiles;                                                   \
         am = u / p.n_ntiles;                                                   \
     }
@@ -202,24 +163,6 @@ __device__ __forceinline__ float act_t(float x, float a, float b) {
 
 // One 32-column chunk of the bf16 epilogue: bias + activation + mask, pack to bf16 (hi, lo),
 // write the thread's 64-byte row into the 64B-swizzled staging tile(s).
-// Per-column sums over the 32 rows a warp holds (one row per lane, 32 columns per lane): butterfly
-// reduce-scatter -- after the 5 exchange steps lane l holds the warp total of column l.
-__device__ __forceinline__ float warp_colsum32(float (&x)[32], int lane) {
-#pragma unroll
-    for (int step = 0; step < 5; ++step) {
-        const int half = 16 >> step;  // values kept per lane after this step
-        const bool upper = (lane & half) != 0;
-#pragma unroll
-        for (int j = 0; j < half; ++j) {
-            // keep columns [0, half) if lower lane-half, [half, 2*half) if upper; send the other half
-            const float mine = upper ? x[j + half] : x[j];
-            const float send = upper ? x[j] : x[j + half];
-            x[j] = mine + __shfl_xor_sync(0xffffffffu, send, half);
-        }
-    }
-    return x[0];
-}
-
 template <int ACT, bool LO>
 __device__ __forceinline__ void epi_chunk(const uint32_t (&v)[32], const float* __restrict__ sb, float a, float b,
                                           bool keep, int row, uint8_t* st_hi, uint8_t* st_lo) {
@@ -276,7 +219,7 @@ __device__ __forceinline__ void bnr_column_pass(const uint8_t* __restrict__ st_g
 }
 
 // Forward batch statistics over one staged chunk, same thread mapping as bnr_column_pass: per-channel sum / sum of squares of
-// the stored values (hi [+ lo]) over the tile's rows < nrows.  Replaces two 31-step shuffle butterflies per thread and chunk.
+// the stored values (hi [+ lo]) over the tile's rows < nrows.
 template <bool LO>
 __device__ __forceinline__ void stats_column_pass(const uint8_t* __restrict__ st_h, const uint8_t* __restrict__ st_l, int et, int nrows,
                                                   float& s_out, float& q_out) {
@@ -307,12 +250,8 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
     uint64_t* empty_bar = full_bar + kStages;
     uint64_t* tmem_full = empty_bar + kStages;
     uint64_t* tmem_empty = tmem_full + kAccStages;
-    SchedRing ring;
-    ring.full = tmem_empty + kAccStages;
-    ring.empty = ring.full + kSched;
-    ring.unit = reinterpret_cast<int*>(ring.empty + kSched);
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(ring.unit + kSched);
-    uint64_t* ybar = reinterpret_cast<uint64_t*>(ring.unit + kSched + 2);  // [2]: y tiles of the folded BatchNorm-backward reduction
+    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tmem_empty + kAccStages);  // 4 bytes in an 8-byte slot
+    uint64_t* ybar = tmem_empty + kAccStages + 1;  // [2]: y tiles of the folded BatchNorm-backward reduction
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -338,10 +277,6 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
             mbar_init(&tmem_full[i], 1);
             mbar_init(&tmem_empty[i], 4);  // one arrive per epilogue warp
         }
-        for (int i = 0; i < kSched; ++i) {
-            mbar_init(&ring.full[i], 1);
-            mbar_init(&ring.empty[i], 5);  // MMA thread + one per epilogue warp
-        }
         mbar_init(&ybar[0], 1);
         mbar_init(&ybar[1], 1);
         mbar_fence_init();
@@ -365,10 +300,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
             uint32_t phase = 0;
             TileCursor cur;
             cur.init(p);
-            int u = 0, nt_next = 0, j = 0, ahead = 0;
+            int u = (int)blockIdx.x - (int)gridDim.x, nt_next = 0;
             for (;;) {
-                CAB_NEXT_UNIT(sched_produce(p, ring, j, ahead))
-                if (!p.mtile_major || nt == 0) ++j;
+                CAB_NEXT_UNIT()
                 if (!cur.seek(p, am)) break;
                 const int b = cur.b;
                 const int t0 = (am - cur.base) * kBlockM;
@@ -402,9 +336,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
             uint32_t acc_phase = 0;
             TileCursor cur;
             cur.init(p);
-            int u = 0, nt_next = 0, j = 0;
+            int u = (int)blockIdx.x - (int)gridDim.x, nt_next = 0;
             for (;;) {
-                CAB_NEXT_UNIT(sched_consume<false>(p, ring, j++, 0))
+                CAB_NEXT_UNIT()
                 (void)nt;
                 if (!cur.seek(p, am)) break;
                 mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
@@ -447,9 +381,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
         int run_i = 0;
         uint32_t yphase = 0;  // bit i = parity ybar[i] completes next
         const bool fold = p.bnr_partials != nullptr;  // (host: ACT_BF16 epilogue, no lo output, no stats)
-        int u = 0, nt_next = 0, j = 0;
+        int u = (int)blockIdx.x - (int)gridDim.x, nt_next = 0;
         for (;;) {
-            CAB_NEXT_UNIT(sched_consume<true>(p, ring, j++, lane))
+            CAB_NEXT_UNIT()
             if (!cur.seek(p, am)) break;
             const int b = cur.b;
             const int t0 = (am - cur.base) * kBlockM;
@@ -534,39 +468,6 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                         default: CAB_EPI_CALL(CAB_ACT_NONE) break;
                     }
 #undef CAB_EPI_CALL
-                    if (p.stats != nullptr && !p.stats_columns) {
-                        // BatchNorm batch statistics of what was just stored (bf16-rounded; hi + lo in the split
-                        // tier), valid rows only
-                        float xs[32], xq[32];
-                        const uint4* mine = reinterpret_cast<const uint4*>(st_hi + row * 64);
-                        const uint4* mine_lo = reinterpret_cast<const uint4*>(st_lo + row * 64);
-                        const int sw = (row >> 1) & 3;
-#pragma unroll
-                        for (int qd = 0; qd < 4; ++qd) {
-                            const uint4 w4 = mine[qd ^ sw];
-                            const uint32_t w[4] = {w4.x, w4.y, w4.z, w4.w};
-                            uint4 l4 = make_uint4(0, 0, 0, 0);
-                            if (has_lo) l4 = mine_lo[qd ^ sw];
-                            const uint32_t wl[4] = {l4.x, l4.y, l4.z, l4.w};
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) {
-                                float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[j]));
-                                const float2 fl = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&wl[j]));
-                                f.x += fl.x; f.y += fl.y;
-                                const float f0 = row_ok ? f.x : 0.f, f1 = row_ok ? f.y : 0.f;
-                                xs[qd * 8 + 2 * j] = f0; xs[qd * 8 + 2 * j + 1] = f1;
-                                xq[qd * 8 + 2 * j] = f0 * f0; xq[qd * 8 + 2 * j + 1] = f1 * f1;
-                            }
-                        }
-                        const float cs = warp_colsum32(xs, lane);
-                        const float cq = warp_colsum32(xq, lane);
-                        // lane l now owns column bit-reversed?  no: the butterfly keeps column index == lane
-                        const int col = n0 + c0 + lane;
-                        if (col < p.C_out) {
-                            atomicAdd(p.stats + col, (double)cs);
-                            atomicAdd(p.stats + p.C_out + col, (double)cq);
-                        }
-                    }
                     fence_async_smem();  // generic-proxy smem writes -> visible to the TMA engine
                     epi_bar(3);
                     if (et == 0) {
@@ -574,8 +475,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                         if (has_lo) tma_store_3d(&p.omap_lo, st_lo, n0 + c0, t0, b);
                         bulk_commit();
                     }
-                    if (p.stats != nullptr && p.stats_columns) {
-                        // batch statistics, column-parallel over the staged tile (every thread's row is there: barrier 3 above; the
+                    if (p.stats != nullptr) {
+                        // BatchNorm batch statistics of what was just stored (bf16-rounded; hi + lo in the split tier), valid rows
+                        // only, column-parallel over the staged tile (every thread's row is there: barrier 3 above; the
                         // buffer is rewritten two chunks from now, behind that chunk's barrier 2)
                         float cs, cq;
                         const int srows = min(max(p.T_out - t0, 0), kBlockM);
@@ -870,28 +772,6 @@ static int pick_block_n(int C_out, int epilogue, long long m_tiles, int num_sms)
 
 extern std::atomic<int64_t> g_launch_count;
 
-// Counters of the dynamic tile schedule: one int per launch out of a ring that is allocated once per process (the only
-// allocation this library makes; 64 K launches must be in flight before a slot could be reused).  Zeroed on the launch's
-// stream right before the kernel, so CUDA-graph replays re-zero their own slots.  OPT-IN (CONVASR_B200_DYNAMIC_TILES=1): the
-// same-box A/B on 8 x B200 (profiles/r02_tile_schedule_ab.md) measured the dynamic schedule 1 % slower at N = 1 and 3 % slower
-// at N = 8 than the static round-robin walk, so static stays the default.
-int* next_tile_counter(cudaStream_t stream) {
-    constexpr int kSlots = 1 << 16;
-    static int* ring = nullptr;
-    static std::atomic<unsigned> next{0};
-    static std::once_flag once;
-    static bool disabled = false;
-    std::call_once(once, [] {
-        const char* e = getenv("CONVASR_B200_DYNAMIC_TILES");
-        disabled = !(e && e[0] == '1');
-        if (!disabled && cudaMalloc(&ring, sizeof(int) * kSlots) != cudaSuccess) ring = nullptr;
-    });
-    if (disabled || ring == nullptr) return nullptr;
-    int* slot = ring + (next.fetch_add(1, std::memory_order_relaxed) % kSlots);
-    if (cudaMemsetAsync(slot, 0, sizeof(int), stream) != cudaSuccess) return nullptr;
-    return slot;
-}
-
 }  // namespace cab
 
 using namespace cab;
@@ -982,14 +862,6 @@ extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
         }
     }
     if (p.stats != nullptr) CAB_CHECK_CUDA(cudaMemsetAsync(p.stats, 0, sizeof(double) * 2 * ep->C_out, stream));
-    {
-        static int stats_columns = -1;  // CONVASR_B200_STATS_COLUMNS=0: the round-1 shuffle-butterfly statistics (A/B switch)
-        if (stats_columns < 0) {
-            const char* e = getenv("CONVASR_B200_STATS_COLUMNS");
-            stats_columns = (e && e[0] == '0') ? 0 : 1;
-        }
-        p.stats_columns = stats_columns;
-    }
     // folded BatchNorm-backward reduction (see ConvParams)
     p.bnr_partials = nullptr; p.bnr_ss = nullptr; p.bnr_xlen = nullptr; p.bnr_C = 0; p.bnr_act = CAB_ACT_NONE; p.bnr_a = 0.f; p.bnr_b = 0.f;
     if (ep->bnr_partials != nullptr) {
@@ -1054,7 +926,6 @@ extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
     CAB_CHECK_ARG(num_sms > 0, "no CUDA device");
     int grid = p.n_tiles < num_sms ? p.n_tiles : num_sms;
     if (p.mtile_major) grid = p.B * p.mtiles_per_b < num_sms ? p.B * p.mtiles_per_b : num_sms;
-    p.tile_counter = next_tile_counter(stream);
     conv1d_umma_kernel<<<grid, kNumThreads, kSmemBytes, stream>>>(p);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);

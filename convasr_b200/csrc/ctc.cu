@@ -15,7 +15,6 @@
 #include <atomic>
 #include <float.h>
 #include <cuda_fp16.h>
-#include <cstdlib>
 
 namespace cab {
 extern std::atomic<int64_t> g_launch_count;
@@ -188,9 +187,7 @@ __global__ void ctc_recursion_kernel(const float* __restrict__ lp, int64_t st, i
                         const float a3 = skip[i] ? prev[s] : -INFINITY;
                         const float v = lse3_fast(a1, a2, a3) + e;
                         cur[s + 2] = v;
-#ifndef CAB_EXPERIMENT_CTC_NO_STORE
                         wsp[sr[i]] = v;
-#endif
                         vlast[i] = v;
                     }
                 }
@@ -1153,12 +1150,6 @@ entropy_kernel(const float* __restrict__ lp, const int64_t* __restrict__ lengths
 }
 
 static int ctc_threads(int S_max) {
-    static int forced = -1;
-    if (forced < 0) {
-        const char* e = getenv("CONVASR_B200_CTC_THREADS");
-        forced = e ? atoi(e) : 0;
-    }
-    if (forced > 0 && S_max <= kCtcMaxPer * forced) return forced;
     // measured on B200 (S = 339, t = 753): 128 threads 609 us, 192: 422, 256: 375, 384: 267 --
     // the per-state lse chain is latency bound, so one state per thread wins while it fits
     int th = (S_max + 31) / 32 * 32;

@@ -13,7 +13,6 @@
 #include "common.cuh"
 #include "../../include/convasr_b200.h"
 #include <atomic>
-#include <cstdlib>
 
 namespace cab {
 extern std::atomic<int64_t> g_launch_count;
@@ -615,14 +614,10 @@ instnorm_pack_kernel(const float* __restrict__ feat, const float* __restrict__ x
     }
 }
 
-// which STFT kernel: the radix-16 x radix-16 kernel (nfft = 256) unless CONVASR_B200_FRONTEND=radix2 asks for the round-1 one (A/B)
+// which STFT kernel: the radix-16 x radix-16 kernel covers nfft = 256 with windows of at most 256 samples; every other
+// nfft or longer window runs the radix-2 logmel_kernel
 static bool use_fft16(int nfft, int win, int hop) {
-    static int forced = -1;
-    if (forced < 0) {
-        const char* e = getenv("CONVASR_B200_FRONTEND");
-        forced = (e && e[0] == 'r') ? 1 : 0;
-    }
-    return !forced && nfft == 256 && win <= 256 && hop > 0;
+    return nfft == 256 && win <= 256 && hop > 0;
 }
 
 static size_t fft16_smem_bytes(int win, int hop, int n_mels) {

@@ -10,7 +10,6 @@
 #include "common.cuh"
 #include "../../include/convasr_b200.h"
 #include <atomic>
-#include <cstdlib>
 
 namespace cab {
 extern std::atomic<int64_t> g_launch_count;
@@ -607,15 +606,9 @@ bn_stream_kernel(const StreamArgs p) {
 static bool stream_geometry(int R, int ld, int n_inputs, StreamArgs& a, int& threads, int& grid, size_t& smem) {
     if (ld % 8 != 0 || R <= 0) return false;
     const int vectors = ld / 8;
-    static int target_threads = 0, stage_budget = 0;
-    if (target_threads == 0) {  // tuning knobs (A/B runs): CTA size and bytes of stages per CTA
-        const char* e = getenv("CONVASR_B200_BN_THREADS");
-        target_threads = e ? atoi(e) : 256;
-        if (target_threads < 32 || target_threads > kStreamMaxThreads) target_threads = 256;
-        e = getenv("CONVASR_B200_BN_STAGE_KB");
-        stage_budget = (e ? atoi(e) : 48) * 1024;
-        if (stage_budget < 16 * 1024 || stage_budget > 200 * 1024) stage_budget = 48 * 1024;
-    }
+    // CTA size and bytes of stages per CTA: the fastest backward of the 128-512 thread x 32-96 KB sweep over the BatchNorm layers
+    // of the training step (profiles/r02b_bn_geometry.log)
+    constexpr int target_threads = 256, stage_budget = 48 * 1024;
     int lanes = target_threads / vectors;  // ~256 threads: the kernels are register-heavy, more CTAs per SM beat bigger CTAs
     if (lanes < 1) lanes = 1;
     while ((vectors * lanes) % 32 != 0) ++lanes;
@@ -637,16 +630,6 @@ static bool stream_geometry(int R, int ld, int n_inputs, StreamArgs& a, int& thr
     if (smem > 220 * 1024) return false;
     grid = 0;  // sized by stream_launch from the occupancy of the instantiation
     return true;
-}
-
-// CONVASR_B200_BN_ORDER=0 restores the ascending walk everywhere (A/B switch); default: L2-aware order
-static int bn_l2_order() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("CONVASR_B200_BN_ORDER");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v;
 }
 
 static int num_sms() {
@@ -1051,7 +1034,7 @@ extern "C" int cab_bn_act_mask_fwd(const void* y, const void* y_lo, const float*
         sa.y_lo = static_cast<const __nv_bfloat16*>(y_lo); sa.out_lo = static_cast<__nv_bfloat16*>(out_lo);
         sa.seed_ptr = reinterpret_cast<const long long*>(seed); sa.salt = (unsigned long long)salt;
         sa.a = act_a; sa.bb = act_b; sa.drop_p = dropout_p; sa.B = B; sa.T = T; sa.C = C; sa.ld = ld; sa.act = act;
-        sa.reverse = bn_l2_order();  // the conv that produced y finished with the high rows
+        sa.reverse = 1;  // the conv that produced y finished with the high rows
         if (split) CAB_CHECK_CUDA((stream_launch<0, true>(sa, threads, grid_s, smem, stream)));
         else CAB_CHECK_CUDA((stream_launch<0, false>(sa, threads, grid_s, smem, stream)));
         g_launch_count.fetch_add(1, std::memory_order_relaxed);
@@ -1093,7 +1076,7 @@ extern "C" int cab_bn_act_mask_fwd_stats(const void* y, const void* y_lo, const 
     sa.raw_sums = raw_sums; sa.sums_ld = sums_ld; sa.gamma = gamma; sa.beta = beta; sa.running_mean = running_mean; sa.running_var = running_var;
     sa.ss_out = out_ss; sa.n_rows = (float)n_rows; sa.inv_n_rows = 1.0 / (double)(float)n_rows; sa.eps = eps; sa.momentum = momentum;
     sa.a = act_a; sa.bb = act_b; sa.drop_p = dropout_p; sa.B = B; sa.T = T; sa.C = C; sa.ld = ld; sa.act = act;
-    sa.reverse = bn_l2_order();
+    sa.reverse = 1;
     if (split) CAB_CHECK_CUDA((stream_launch<0, true>(sa, threads, grid_s, smem, stream)));
     else CAB_CHECK_CUDA((stream_launch<0, false>(sa, threads, grid_s, smem, stream)));
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
@@ -1124,7 +1107,7 @@ static int bn_bwd_impl(const void* y, const void* y_lo, const void* grad_out, co
             sa.B = B; sa.T = T; sa.C = C; sa.ld = ld; sa.act = act;
             if (partials_ready) {
                 // the dgrad GEMM that produced grad_out also accumulated the sums and finished with the high rows: descend
-                sa.reverse = bn_l2_order();
+                sa.reverse = 1;
                 if (split) CAB_CHECK_CUDA((stream_launch<2, true>(sa, threads, grid_s, smem, stream)));
                 else CAB_CHECK_CUDA((stream_launch<2, false>(sa, threads, grid_s, smem, stream)));
                 g_launch_count.fetch_add(1, std::memory_order_relaxed);
@@ -1134,7 +1117,7 @@ static int bn_bwd_impl(const void* y, const void* y_lo, const void* grad_out, co
             // reduce pass: descending (the dgrad GEMM that produced grad_out finished with the high rows); apply pass: ascending
             // (the reduce pass finished with the low rows)
             StreamArgs sr = sa;
-            sr.reverse = bn_l2_order();
+            sr.reverse = 1;
             sa.reverse = 0;
             if (split) {
                 CAB_CHECK_CUDA((stream_launch<1, true>(sr, threads, grid_s, smem, stream)));

@@ -12,7 +12,8 @@
 // (block_n/64 atoms), K = 64 frames per pipeline stage (4 MMAs of K=16).  Each TMA box is
 // {64 channels, 64 frames} = 8 KB with the 128-byte swizzle; frames outside [0, T) are zero-filled
 // by the TMA unit, which implements both the conv zero padding and the ragged tile tail.
-// Work item = (tap, m-tile, n-tile, batch split); partial sums of different splits are combined
+// Work item = (tap, m-tile, n-tile, batch split), CTA i takes items i, i + gridDim.x, ... (the static
+// schedule of conv1d_umma_kernel); partial sums of different splits are combined
 // with fp32 reductions in L2 (red.global.add), so dW must be zero-initialised by the caller when
 // n_splits > 1 (the host wrapper does it).
 #include "common.cuh"
@@ -22,7 +23,6 @@
 
 namespace cab {
 extern std::atomic<int64_t> g_launch_count;
-int* next_tile_counter(cudaStream_t stream);  // conv_gemm.cu
 
 namespace wg {
 constexpr int kBlockM = 128;
@@ -51,41 +51,7 @@ struct alignas(64) Params {
     int accumulate;         // use reductions instead of stores
     const float* skip_frac; // frames >= ceil(skip_frac[b] * skip_T) + skip_margin contribute zeros: not contracted
     int skip_T, skip_margin;
-    int* item_counter;      // dynamic item schedule (see conv_gemm.cu: a late CTA claims fewer items); null = static
 };
-
-constexpr int kSched = 4;
-struct SchedRing {
-    int* unit;
-    uint64_t* full;
-    uint64_t* empty;
-};
-// The producer claims one unit AHEAD: the atomicAdd for unit j + 1 is issued when unit j is published and its result is first
-// needed a whole tile later, so the ~1 us round trip of the global atomic never sits on the producer's critical path.
-__device__ __forceinline__ int sched_produce(const Params& p, const SchedRing& r, int j, int& ahead) {
-    if (p.item_counter == nullptr) return blockIdx.x + j * gridDim.x;
-    const int slot = j % kSched;
-    const int u = j == 0 ? atomicAdd(p.item_counter, 1) : ahead;
-    mbar_wait(&r.empty[slot], ((j / kSched) & 1) ^ 1);
-    r.unit[slot] = u;
-    mbar_arrive(&r.full[slot]);  // release: the slot's value is visible to whoever acquires the barrier
-    ahead = atomicAdd(p.item_counter, 1);
-    return u;
-}
-template <bool WARP>
-__device__ __forceinline__ int sched_consume(const Params& p, const SchedRing& r, int j, int lane) {
-    if (p.item_counter == nullptr) return blockIdx.x + j * gridDim.x;
-    const int slot = j % kSched;
-    mbar_wait(&r.full[slot], (j / kSched) & 1);
-    const int u = r.unit[slot];
-    if (WARP) {
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&r.empty[slot]);
-    } else {
-        mbar_arrive(&r.empty[slot]);
-    }
-    return u;
-}
 
 // 64-frame K chunks of utterance b that can hold non-zero products
 __device__ __forceinline__ int live_chunks(const Params& p, int b) {
@@ -117,11 +83,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) wgrad_umma_kernel(const __grid
     uint64_t* empty_bar = full_bar + kStages;
     uint64_t* tmem_full = empty_bar + kStages;
     uint64_t* tmem_empty = tmem_full + kAccStages;
-    SchedRing ring;
-    ring.full = tmem_empty + kAccStages;
-    ring.empty = ring.full + kSched;
-    ring.unit = reinterpret_cast<int*>(ring.empty + kSched);
-    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(ring.unit + kSched);
+    uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(tmem_empty + kAccStages);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (warp == 0 && lane == 0) {
@@ -131,7 +93,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) wgrad_umma_kernel(const __grid
     if (warp == 1 && lane == 0) {
         for (int i = 0; i < kStages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
         for (int i = 0; i < kAccStages; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 4); }
-        for (int i = 0; i < kSched; ++i) { mbar_init(&ring.full[i], 1); mbar_init(&ring.empty[i], 5); }
         mbar_fence_init();
     }
     if (warp == 2) {
@@ -165,10 +126,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) wgrad_umma_kernel(const __grid
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            int ahead = 0;
-            for (int j = 0;; ++j) {
-                const int item = sched_produce(p, ring, j, ahead);
-                if (item >= p.n_items) break;
+            for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
                 int tap, mt, nt, b0, b1;
                 decode(item, tap, mt, nt, b0, b1);
                 const int m0 = mt * kBlockM, n0 = nt * block_n;
@@ -197,9 +155,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) wgrad_umma_kernel(const __grid
             uint32_t phase = 0;
             int acc = 0;
             uint32_t acc_phase = 0;
-            for (int j = 0;; ++j) {
-                const int item = sched_consume<false>(p, ring, j, 0);
-                if (item >= p.n_items) break;
+            for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
                 int tap, mt, nt, b0, b1;
                 decode(item, tap, mt, nt, b0, b1);
                 mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
@@ -233,9 +189,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) wgrad_umma_kernel(const __grid
         const int row = q * 32 + lane;
         int acc = 0;
         uint32_t acc_phase = 0;
-        for (int j = 0;; ++j) {
-            const int item = sched_consume<true>(p, ring, j, lane);
-            if (item >= p.n_items) break;
+        for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
             int tap, mt, nt, b0, b1;
             decode(item, tap, mt, nt, b0, b1);
             const int m = mt * kBlockM + row;
@@ -376,7 +330,6 @@ extern "C" int cab_conv1d_wgrad(const void* a, int a_T, int a_T_rows, int a_ld, 
     p.accumulate = (n_splits > 1 || accumulate_into) ? 1 : 0;
     if (p.accumulate && !accumulate_into) CAB_CHECK_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)taps * M_total * out_ld, stream));
     const int grid = p.n_items < num_sms ? p.n_items : num_sms;
-    p.item_counter = next_tile_counter(stream);
     wg::wgrad_umma_kernel<<<grid, wg::kNumThreads, wg::kSmemBytes, stream>>>(p);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);

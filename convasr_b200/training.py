@@ -39,10 +39,11 @@ import torch.nn as nn
 from . import _lib, engine, ops
 
 BF16 = torch.bfloat16
-_SEPARATE_BN_STATS = os.environ.get('CONVASR_B200_SEPARATE_BN_STATS', '0') == '1'
-_SKIP_PADDING = os.environ.get('CONVASR_B200_SKIP_PADDING', '1') == '1'  # A/B switch: leave tiles of pure padding out
+# Tests and tools/trace_train_layers.py set these two to False to run the other path as a reference; that path also runs for
+# unmasked inputs and for repeats the fold does not cover.
+_SKIP_PADDING = True  # leave tiles of pure padding out
 # BatchNorm-backward channel sums accumulated by the dgrad GEMM's epilogue instead of a separate pass over (y, g)
-_FOLD_BN_REDUCE = os.environ.get('CONVASR_B200_FOLD_BN_REDUCE', '1') == '1'
+_FOLD_BN_REDUCE = True
 _GRAD_BUCKET_MB = int(os.environ.get('CONVASR_B200_GRAD_BUCKET_MB', '64'))  # data-parallel gradient bucket size; 0 = one collective per layer
 
 
@@ -290,7 +291,7 @@ class NativeStack(torch.autograd.Function):
 			mask_ptr = ops._p(xlen if rep.mask else None)
 			if not rep.res:
 				# one BatchNorm branch: streamed kernel, the BN finalize (mean / invstd / running statistics) folded in
-				if ss is None and not _SEPARATE_BN_STATS:
+				if ss is None:
 					ss = torch.empty(4, cv.C_out, dtype = torch.float32, device = dev)
 					bn = rep.bn
 					rc = lib.cab_bn_act_mask_fwd_stats(
@@ -300,8 +301,7 @@ class NativeStack(torch.autograd.Function):
 					)
 					_lib.check(rc, 'cab_bn_act_mask_fwd_stats')
 				else:
-					if ss is None:
-						ss = _bn_finalize(sums, B * T_out, cv.C_out, rep.bn)
+					# frozen BatchNorm: ss holds the coefficients of the running statistics
 					rc = lib.cab_bn_act_mask_fwd(ops._p(y.hi), ops._p(y.lo), ops._p(ss), B, T_out, cv.C_out, cv.co_alloc, code, a, b, mask_ptr, ops._p(out.hi), ops._p(out.lo), rep.dropout, ops._p(holder['seed']), rep.salt, ops._stream())
 					_lib.check(rc, 'cab_bn_act_mask_fwd')
 				rec.update(y = y, ss = ss, branches = None)

@@ -33,5 +33,4 @@ for C, count in ((256, 4), (384, 3), (512, 3), (640, 3), (768, 3), (896, 1), (10
 	mb = y.numel() * 2 / 1e6
 	rows.append(f'C={C}: fwd {t_f:.1f} us ({2 * mb / t_f:.2f} TB/s) bwd {t_b:.1f} apply {t_a:.1f} us ({3 * mb / t_a:.2f} TB/s)')
 	tot['fwd'] += count * t_f; tot['bwd'] += count * t_b; tot['apply'] += count * t_a
-tag = f"threads={os.environ.get('CONVASR_B200_BN_THREADS', '256')} stage_kb={os.environ.get('CONVASR_B200_BN_STAGE_KB', '48')}"
-print(f'[{tag}] 18-layer totals: fwd {tot["fwd"]:.0f} us, bwd(reduce+apply) {tot["bwd"]:.0f} us, apply-only {tot["apply"]:.0f} us | ' + ' | '.join(rows))
+print(f'18-layer totals: fwd {tot["fwd"]:.0f} us, bwd(reduce+apply) {tot["bwd"]:.0f} us, apply-only {tot["apply"]:.0f} us | ' + ' | '.join(rows))
