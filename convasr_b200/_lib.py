@@ -67,6 +67,9 @@ SIGNATURES = {
 	'cab_instnorm_pack': [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_int, c_int, c_int, c_void_p, c_void_p,
 						c_void_p, c_void_p, c_void_p],
 	'cab_conv1d_fused': [ctypes.POINTER(ConvSource), c_int, ctypes.POINTER(ConvEpilogue), c_void_p],
+	'cab_conv1d_fused_fp8': [ctypes.POINTER(ConvSource), c_int, ctypes.POINTER(ConvEpilogue), c_void_p, c_float, c_void_p],
+	'cab_absmax_bf16': [c_void_p, c_i64, c_void_p, c_void_p],
+	'cab_quantize_e4m3': [c_void_p, c_i64, c_float, c_void_p, c_void_p],
 	'cab_conv1d_wgrad': [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
 						c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p],
 	'cab_bn_batch_stats': [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_float, c_void_p, c_void_p,
@@ -92,6 +95,8 @@ SIGNATURES = {
 							c_void_p, c_void_p, c_void_p, c_float, c_float, c_float, c_float, c_float, c_int, c_float, c_void_p, c_void_p, c_void_p],
 	'cab_grouped_conv1d': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int,
 								c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p],
+	'cab_grouped_conv1d_fp8': [c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
+								c_void_p, c_int, c_int, c_float, c_void_p],
 	'cab_grouped_conv1d_wgrad': [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
 								c_void_p, c_void_p, c_void_p],
 	'cab_bn_act_mask_fwd_stats': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_float, c_float, c_void_p, c_void_p, c_void_p,

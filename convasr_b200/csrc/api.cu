@@ -24,7 +24,7 @@ void set_last_error(const char* fmt, ...) {
 // output channels; weights stay in L1.
 int grouped_conv_fast(const void* act, const void* act_lo, int B, int T, int T_rows, int C_in, int ld_in, const float* wgt,
                       const float* bias, int C_out, int groups, int k, int pad_left, void* out, void* out_lo,
-                      int out_T_rows, int ld_out, int relu, cudaStream_t stream);
+                      int out_T_rows, int ld_out, int relu, cudaStream_t stream, bool fp8, float in_scale, float out_inv);
 constexpr int kGcFrames = 8;
 __global__ void __launch_bounds__(256)
 grouped_conv_relu_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ x_lo, int T,
@@ -99,7 +99,7 @@ extern "C" int cab_grouped_conv1d(const void* act, const void* act_lo, int B, in
     CAB_CHECK_ARG(T_rows >= T && out_T_rows >= T, "row allocation smaller than T");
     CAB_CHECK_ARG(ld_in >= C_in && ld_out >= C_out, "row pitch smaller than channel count");
     {
-        const int rc = grouped_conv_fast(act, act_lo, B, T, T_rows, C_in, ld_in, wgt, bias, C_out, groups, k, pad_left, out, out_lo, out_T_rows, ld_out, relu, stream);
+        const int rc = grouped_conv_fast(act, act_lo, B, T, T_rows, C_in, ld_in, wgt, bias, C_out, groups, k, pad_left, out, out_lo, out_T_rows, ld_out, relu, stream, false, 1.f, 1.f);
         if (rc <= 0) return rc;  // launched (0) or failed (< 0); 1 = shape not covered by the FFMA2 kernel
     }
     dim3 grid((T + kGcFrames - 1) / kGcFrames, B);
@@ -110,4 +110,20 @@ extern "C" int cab_grouped_conv1d(const void* act, const void* act_lo, int B, in
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     return 0;
+}
+
+extern "C" int cab_grouped_conv1d_fp8(const void* act, int B, int T, int T_rows, int C_in, int ld_in, float in_scale,
+                                      const float* wgt, const float* bias, int C_out, int groups, int k, int pad_left,
+                                      void* out, int out_T_rows, int ld_out, float out_scale_inv, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CAB_CHECK_ARG(act && wgt && out, "null pointer argument");
+    CAB_CHECK_ARG(groups > 0 && C_in % groups == 0 && C_out % groups == 0, "channels not divisible by groups");
+    CAB_CHECK_ARG(T_rows >= T && out_T_rows >= T, "row allocation smaller than T");
+    CAB_CHECK_ARG(ld_in >= C_in && ld_out >= C_out, "row pitch smaller than channel count");
+    CAB_CHECK_ARG((reinterpret_cast<uintptr_t>(act) & 15) == 0, "act must be 16-byte aligned");
+    const int rc = grouped_conv_fast(act, nullptr, B, T, T_rows, C_in, ld_in, wgt, bias, C_out, groups, k, pad_left, out, nullptr,
+                                     out_T_rows, ld_out, 1, stream, true, in_scale, out_scale_inv);
+    CAB_CHECK_ARG(rc != 1, "E4M3 grouped conv: shape not covered (k=%d odd in 3..27, ld_in=%d a multiple of 16, input window of "
+                           "at most 208 channels per 64 outputs)", k, ld_in);
+    return rc;
 }

@@ -5,6 +5,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda.h>
 #include <stdint.h>
 #include <math.h>
@@ -194,6 +195,18 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint
         ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
         : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem], E4M3 inputs (K = 32 per instruction), fp32 accumulate, single CTA.
+__device__ __forceinline__ void umma_e4m3(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,
+                                          uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t"
+        "}\n"
+        ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
 // All previously issued MMAs of this thread arrive on `bar` when complete
 // (implies tcgen05.fence::before_thread_sync).
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
@@ -245,6 +258,24 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
 // both K-major (bits 15,16 = 0), N>>3 at bits 17-22, M>>4 at bits 24-28.
 __host__ __device__ __forceinline__ uint32_t umma_idesc_bf16(uint32_t M, uint32_t N) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+// Instruction descriptor, kind::f8f6f4: D=f32 (bits 4-5 = 1), A=B=E4M3 (format code 0 in bits 7-9 and 10-12),
+// both K-major, N>>3 at bits 17-22, M>>4 at bits 24-28.
+__host__ __device__ __forceinline__ uint32_t umma_idesc_e4m3(uint32_t M, uint32_t N) {
+    return (1u << 4) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+// two fp32 -> two E4M3 (round to nearest even, saturating to +-448); `lo` lands in the low byte (lower address)
+__device__ __forceinline__ uint16_t pack_e4m3x2(float lo, float hi) {
+    uint16_t r;
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+// two E4M3 (low byte first) -> float2, exact
+__device__ __forceinline__ float2 unpack_e4m3x2(uint16_t v) {
+    uint32_t h;
+    asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(h) : "h"(v));
+    const __half2 hh = *reinterpret_cast<const __half2*>(&h);
+    return __half22float2(hh);
 }
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {

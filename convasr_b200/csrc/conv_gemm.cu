@@ -15,6 +15,10 @@
 //   tcgen05.mma.cta_group::1.kind::f16 (M=128, N=block_n, K=16) accumulating fp32 in TMEM.
 //   TMEM holds two 256-column accumulators so the epilogue of tile i overlaps the MMAs of
 //   tile i+1.
+//   E4M3 operand mode (conv1d_umma_kernel<true>, cab_conv1d_fused_fp8): the same tiles with 1-byte
+//   elements -- a 128-byte swizzle row holds 128 channels, so a stage carries K = 128 and the same four
+//   MMAs per row are tcgen05.mma.kind::f8f6f4 with K = 32; the epilogue scales the accumulator by a
+//   per-column alpha[n] before the bias, and the activation epilogue stores E4M3 (x 1/s_out, saturating).
 // Warp roles (256 threads): warp0 = TMA producer, warp1 = MMA issuer, warp2 = TMEM allocator,
 //   warps4-7 = epilogue (TMEM lane quarter = warp_idx % 4).
 #include "common.cuh"
@@ -88,6 +92,9 @@ struct alignas(64) ConvParams {
     double* bnr_partials;    // null = no fold
     int bnr_C, bnr_act;
     float bnr_a, bnr_b;
+    // E4M3 mode: per-column multiplier of the accumulator [C_out], and 1/scale of the stored E4M3 activation
+    const float* alpha;
+    float out_inv;
 };
 
 // Tile schedule.  Only M tiles that hold at least one live row are enumerated ("compacted" index am), so
@@ -189,6 +196,26 @@ __device__ __forceinline__ void epi_chunk(const uint32_t (&v)[32], const float* 
     }
 }
 
+// E4M3 twin of epi_chunk: acc * alpha + bias -> activation -> mask -> x 1/s_out -> E4M3 (saturating), the thread's
+// 32-byte row into an unswizzled [128 rows][32 B] staging tile.
+template <int ACT>
+__device__ __forceinline__ void epi_chunk_e4m3(const uint32_t (&v)[32], const float* __restrict__ sb, const float* __restrict__ sa,
+                                               float a, float b, bool keep, float inv, int row, uint8_t* st) {
+    uint32_t q[8];
+#pragma unroll
+    for (int j = 0; j < 32; j += 4) {
+        float x[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            x[i] = act_t<ACT>(fmaf(__uint_as_float(v[j + i]), sa[j + i], sb[j + i]), a, b);
+            x[i] = keep ? x[i] * inv : 0.f;
+        }
+        q[j >> 2] = (uint32_t)pack_e4m3x2(x[0], x[1]) | ((uint32_t)pack_e4m3x2(x[2], x[3]) << 16);
+    }
+    *reinterpret_cast<uint4*>(st + row * 32) = make_uint4(q[0], q[1], q[2], q[3]);
+    *reinterpret_cast<uint4*>(st + row * 32 + 16) = make_uint4(q[4], q[5], q[6], q[7]);
+}
+
 // Folded BatchNorm-backward reduction over one staged chunk: g and y are bf16 [128 rows][32 cols] tiles in the 64B-swizzled
 // staging layout.  Thread = (column et % 32, row group et / 32): the per-channel coefficients are two scalars, the 32 lanes of
 // a warp read the 64 contiguous (swizzled) bytes of one row -- conflict free -- and no cross-lane reduction is needed; the
@@ -239,8 +266,11 @@ __device__ __forceinline__ void stats_column_pass(const uint8_t* __restrict__ st
     q_out = q;
 }
 
+// FP8: E4M3 operands (kind::f8f6f4); the stage layout and byte counts are those of the bf16 mode.
+template <bool FP8>
 __global__ void __launch_bounds__(kNumThreads, 1)
 conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
+    constexpr int kChunk = FP8 ? 2 * kBlockK : kBlockK;  // channels per 128-byte swizzle row
     extern __shared__ uint8_t smem_raw[];
     // 1024-byte alignment required by the 128B swizzle atoms
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
@@ -317,9 +347,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                             uint8_t* b_dst = a_dst + kATileBytes;
                             mbar_expect_tx(&full_bar[stage], stage_tx_bytes);
                             tma_load_3d(a_dst, &p.amap[s], &full_bar[stage],
-                                        sd.a_ch_off + ch * kBlockK, trow, b);
+                                        sd.a_ch_off + ch * kChunk, trow, b);
                             tma_load_3d(b_dst, &p.wmap[s], &full_bar[stage],
-                                        sd.w_ch_off + ch * kBlockK, n0, tap);
+                                        sd.w_ch_off + ch * kChunk, n0, tap);
                             if (++stage == kStages) { stage = 0; phase ^= 1; }
                         }
                     }
@@ -329,7 +359,7 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
     } else if (warp == 1) {
         // ===================== MMA issuer =====================
         if (lane == 0) {
-            const uint32_t idesc = umma_idesc_bf16(kBlockM, block_n);
+            const uint32_t idesc = FP8 ? umma_idesc_e4m3(kBlockM, block_n) : umma_idesc_bf16(kBlockM, block_n);
             int stage = 0;
             uint32_t phase = 0;
             int acc = 0;
@@ -356,8 +386,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                         const uint64_t b_desc = umma_desc_sw128(b_addr);
 #pragma unroll
                         for (int k = 0; k < kBlockK / 16; ++k) {
-                            // +32 bytes per K=16 slice inside the 128B swizzle row (>>4 => +2)
-                            umma_bf16(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, accumulate);
+                            // +32 bytes per K=16 (bf16) / K=32 (E4M3) slice inside the 128B swizzle row (>>4 => +2)
+                            if (FP8) umma_e4m3(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, accumulate);
+                            else umma_bf16(d_tmem, a_desc + 2 * k, b_desc + 2 * k, idesc, accumulate);
                             accumulate = 1;
                         }
                         umma_commit(&empty_bar[stage]);  // frees the smem slot when MMAs retire
@@ -419,9 +450,12 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                 }
                 // stage this tile's bias (zeros past C_out / without bias)
                 epi_bar(1);  // previous tile's readers are done with s_bias
+                // E4M3 mode: alpha goes where the lo staging pair would be (no lo output, no folded reduction there)
+                float* const s_alpha = reinterpret_cast<float*>(smem + kOffStageOut + 2 * kEpiTileBytes);
                 for (int i = et; i < block_n; i += 128) {
                     const int n = n0 + i;
                     s_bias[i] = (p.bias != nullptr && n < p.C_out) ? __ldg(p.bias + n) : 0.f;
+                    if (FP8) s_alpha[i] = n < p.C_out ? __ldg(p.alpha + n) : 0.f;
                 }
                 epi_bar(1);
                 mbar_wait(&tmem_full[acc], acc_phase);  // bias staging above overlaps the MMAs
@@ -459,7 +493,8 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                     }
                     const float* sb = s_bias + c0;
 #define CAB_EPI_CALL(ACT)                                                                          \
-    if (has_lo) epi_chunk<ACT, true>(v, sb, p.act_a, p.act_b, keep, row, st_hi, st_lo);            \
+    if (FP8) epi_chunk_e4m3<ACT>(v, sb, s_alpha + c0, p.act_a, p.act_b, keep, p.out_inv, row, st_hi); \
+    else if (has_lo) epi_chunk<ACT, true>(v, sb, p.act_a, p.act_b, keep, row, st_hi, st_lo);       \
     else epi_chunk<ACT, false>(v, sb, p.act_a, p.act_b, keep, row, st_hi, st_lo);
                     switch (p.act) {
                         case CAB_ACT_RELU: CAB_EPI_CALL(CAB_ACT_RELU) break;
@@ -539,8 +574,9 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                     int ci = 0;
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
-                        x[j] = __uint_as_float(v[j]) + s_bias[c0 + j];
                         const bool in = n0 + c0 + j < C;
+                        if (FP8) x[j] = fmaf(__uint_as_float(v[j]), in ? __ldg(p.alpha + n0 + c0 + j) : 0.f, s_bias[c0 + j]);
+                        else x[j] = __uint_as_float(v[j]) + s_bias[c0 + j];
                         if (in && x[j] > cm) { cm = x[j]; ci = n0 + c0 + j; }
                     }
                     if (cm > run_m) {  // strict: ties keep the lowest class id (classes are visited in increasing order)
@@ -588,7 +624,7 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                     for (int j = 0; j < 16; ++j) {
                         const int c = c0 + j;
                         if (c < C) {
-                            float x = __uint_as_float(v[j]) + (p.bias ? __ldg(p.bias + c) : 0.f);
+                            float x = (FP8 ? __uint_as_float(v[j]) * __ldg(p.alpha + c) : __uint_as_float(v[j])) + (p.bias ? __ldg(p.bias + c) : 0.f);
                             if (x > vmax) { vmax = x; imax = c; }
                         }
                     }
@@ -602,7 +638,7 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                     for (int j = 0; j < 16; ++j) {
                         const int c = c0 + j;
                         if (c < C) {
-                            float x = __uint_as_float(v[j]) + (p.bias ? __ldg(p.bias + c) : 0.f);
+                            float x = (FP8 ? __uint_as_float(v[j]) * __ldg(p.alpha + c) : __uint_as_float(v[j])) + (p.bias ? __ldg(p.bias + c) : 0.f);
                             ssum += expf(x - vmax);
                         }
                     }
@@ -617,7 +653,7 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                         for (int j = 0; j < 16; ++j) {
                             const int c = c0 + j;
                             if (c < C) {
-                                float x = __uint_as_float(v[j]) + (p.bias ? __ldg(p.bias + c) : 0.f);
+                                float x = (FP8 ? __uint_as_float(v[j]) * __ldg(p.alpha + c) : __uint_as_float(v[j])) + (p.bias ? __ldg(p.bias + c) : 0.f);
                                 const size_t o = (size_t(b) * C + c) * p.T_out + t;  // lanes -> consecutive t
                                 if (p.logits) p.logits[o] = x;
                                 if (p.log_probs) p.log_probs[o] = x - lse;
@@ -637,7 +673,7 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                         for (int j = 0; j < 16; ++j) {
                             const int c = n0 + c0 + j;
                             if (c < C) {
-                                float x = __uint_as_float(v[j]) + (p.bias ? __ldg(p.bias + c) : 0.f);
+                                float x = (FP8 ? __uint_as_float(v[j]) * __ldg(p.alpha + c) : __uint_as_float(v[j])) + (p.bias ? __ldg(p.bias + c) : 0.f);
                                 p.logits[(size_t(b) * C + c) * p.T_out + t] = apply_act(x, p.act, p.act_a, p.act_b);
                             }
                         }
@@ -675,10 +711,10 @@ conv1d_umma_kernel(const __grid_constant__ ConvParams p) {
                     uint8_t* st_lo = stage + (2 + buf) * kEpiTileBytes;
                     if (et == 0) bulk_wait_read<1>();
                     epi_bar(2);
-                    uint4* zh = reinterpret_cast<uint4*>(st_hi + row * 64);
+                    uint4* zh = reinterpret_cast<uint4*>(st_hi + row * (FP8 ? 32 : 64));
                     uint4* zl = reinterpret_cast<uint4*>(st_lo + row * 64);
 #pragma unroll
-                    for (int qd = 0; qd < 4; ++qd) {
+                    for (int qd = 0; qd < (FP8 ? 2 : 4); ++qd) {
                         zh[qd] = make_uint4(0, 0, 0, 0);
                         if (has_lo) zl[qd] = make_uint4(0, 0, 0, 0);
                     }
@@ -726,17 +762,18 @@ static EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-// 3-D bf16 map: dims (innermost first) {d0, d1, d2}, row pitch / slab pitch in elements.
+// 3-D bf16 (elem_bytes 2) or E4M3 (elem_bytes 1, mapped as bytes) map: dims (innermost first) {d0, d1, d2}, row pitch /
+// slab pitch in elements.
 static int encode_map_3d(CUtensorMap* map, const void* base, uint64_t d0, uint64_t d1, uint64_t d2,
                          uint64_t pitch1_elems, uint64_t pitch2_elems, uint32_t box0,
-                         uint32_t box1, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
+                         uint32_t box1, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B, int elem_bytes = 2) {
     EncodeTiledFn enc = get_encode_fn();
     CAB_CHECK_ARG(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
     cuuint64_t dims[3] = {d0, d1, d2};
-    cuuint64_t strides[2] = {pitch1_elems * 2, pitch2_elems * 2};
+    cuuint64_t strides[2] = {pitch1_elems * elem_bytes, pitch2_elems * elem_bytes};
     cuuint32_t box[3] = {box0, box1, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims,
+    CUresult r = enc(map, elem_bytes == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims,
                      strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -776,9 +813,12 @@ extern std::atomic<int64_t> g_launch_count;
 
 using namespace cab;
 
-extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
-                                const cab_conv_epilogue_t* ep, cab_stream_t stream_) {
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+// FP8: E4M3 sources and (ACT_BF16 epilogue) E4M3 output; alpha [C_out] scales the accumulator, out_inv the stored value
+template <bool FP8>
+static int conv1d_launch(const cab_conv_source_t* srcs, int n_src, const cab_conv_epilogue_t* ep, const float* alpha,
+                         float out_inv, cudaStream_t stream) {
+    constexpr int kChunk = FP8 ? 2 * kBlockK : kBlockK;
+    constexpr int kElem = FP8 ? 1 : 2;
     CAB_CHECK_ARG(srcs && ep, "null sources/epilogue");
     CAB_CHECK_ARG(n_src >= 1 && n_src <= CAB_MAX_CONV_SOURCES, "n_sources=%d out of [1,%d]", n_src,
                   CAB_MAX_CONV_SOURCES);
@@ -839,6 +879,15 @@ extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
     p.stats = ep->epilogue == CAB_EPI_ACT_BF16 ? ep->stats : nullptr;
     p.lse = ep->epilogue == CAB_EPI_LOGITS_ROWS ? ep->log_probs : nullptr;  // the log_probs slot carries the [B, T_out] log-sum-exp output
     p.mtile_major = ep->epilogue == CAB_EPI_LOGITS_ROWS ? 1 : 0;
+    p.alpha = alpha;
+    p.out_inv = out_inv;
+    if (FP8) {
+        CAB_CHECK_ARG(alpha != nullptr, "alpha is null");
+        CAB_CHECK_ARG(ep->out_lo == nullptr && ep->stats == nullptr && ep->bnr_partials == nullptr && ep->skip_frac == nullptr,
+                      "the E4M3 mode has no lo output, no statistics, no folded reduction and no explicit skip rows");
+        if (ep->epilogue == CAB_EPI_ACT_BF16)
+            CAB_CHECK_ARG(ep->out_ld_ch % 16 == 0, "E4M3 output: out_ld_ch=%d must be a multiple of 16", ep->out_ld_ch);
+    }
     if (ep->epilogue == CAB_EPI_LOGITS_ROWS) {
         EncodeTiledFn enc = get_encode_fn();
         CAB_CHECK_ARG(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
@@ -878,9 +927,10 @@ extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
     }
     if (ep->epilogue == CAB_EPI_ACT_BF16) {
         CAB_CHECK_ARG(ep->out_lo == nullptr || (reinterpret_cast<uintptr_t>(ep->out_lo) & 15) == 0, "out_lo must be 16-byte aligned");
+        // E4M3: 32-byte staging rows, unswizzled
         int rc = encode_map_3d(&p.omap_hi, ep->out_hi, (uint64_t)ep->out_ld_ch, (uint64_t)ep->T_out, (uint64_t)ep->B,
                                (uint64_t)ep->out_ld_ch, (uint64_t)ep->out_T_rows * ep->out_ld_ch, kEpiCols, kBlockM,
-                               CU_TENSOR_MAP_SWIZZLE_64B);
+                               FP8 ? CU_TENSOR_MAP_SWIZZLE_NONE : CU_TENSOR_MAP_SWIZZLE_64B, kElem);
         if (rc) return rc;
         if (ep->out_lo != nullptr) {
             rc = encode_map_3d(&p.omap_lo, ep->out_lo, (uint64_t)ep->out_ld_ch, (uint64_t)ep->T_out, (uint64_t)ep->B,
@@ -893,21 +943,21 @@ extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
     for (int s = 0; s < n_src; ++s) {
         const cab_conv_source_t& c = srcs[s];
         CAB_CHECK_ARG(c.act && c.wgt, "source %d: null pointer", s);
-        CAB_CHECK_ARG(c.C_in > 0 && c.C_in % kBlockK == 0, "source %d: C_in=%d must be a multiple of 64", s, c.C_in);
-        CAB_CHECK_ARG(c.ch_off >= 0 && c.ch_off + c.C_in <= c.ld_ch && c.ld_ch % 8 == 0, "source %d: bad channel window off=%d C_in=%d ld=%d", s, c.ch_off, c.C_in, c.ld_ch);
-        CAB_CHECK_ARG(c.w_ch_off >= 0 && c.w_ch_off + c.C_in <= c.w_ld_ch && c.w_ld_ch % 8 == 0, "source %d: bad weight channel window", s);
+        CAB_CHECK_ARG(c.C_in > 0 && c.C_in % kChunk == 0, "source %d: C_in=%d must be a multiple of %d", s, c.C_in, kChunk);
+        CAB_CHECK_ARG(c.ch_off >= 0 && c.ch_off + c.C_in <= c.ld_ch && c.ld_ch % (16 / kElem) == 0, "source %d: bad channel window off=%d C_in=%d ld=%d", s, c.ch_off, c.C_in, c.ld_ch);
+        CAB_CHECK_ARG(c.w_ch_off >= 0 && c.w_ch_off + c.C_in <= c.w_ld_ch && c.w_ld_ch % (16 / kElem) == 0, "source %d: bad weight channel window", s);
         CAB_CHECK_ARG(c.taps >= 1 && c.dilation >= 1, "source %d: taps=%d dilation=%d", s, c.taps, c.dilation);
         CAB_CHECK_ARG(c.T_in >= 1 && c.T_rows >= c.T_in, "source %d: T_in=%d T_rows=%d", s, c.T_in, c.T_rows);
         CAB_CHECK_ARG((reinterpret_cast<uintptr_t>(c.act) & 15) == 0 && (reinterpret_cast<uintptr_t>(c.wgt) & 15) == 0, "source %d: pointers must be 16-byte aligned", s);
         int rc = encode_map_3d(&p.amap[s], c.act, (uint64_t)c.ld_ch, (uint64_t)c.T_in, (uint64_t)ep->B,
-                               (uint64_t)c.ld_ch, (uint64_t)c.T_rows * c.ld_ch, kBlockK, kBlockM);
+                               (uint64_t)c.ld_ch, (uint64_t)c.T_rows * c.ld_ch, kChunk, kBlockM, CU_TENSOR_MAP_SWIZZLE_128B, kElem);
         if (rc) return rc;
         rc = encode_map_3d(&p.wmap[s], c.wgt, (uint64_t)c.w_ld_ch, (uint64_t)c.w_rows, (uint64_t)c.taps,
-                           (uint64_t)c.w_ld_ch, (uint64_t)c.w_rows * c.w_ld_ch, kBlockK, (uint32_t)bn);
+                           (uint64_t)c.w_ld_ch, (uint64_t)c.w_rows * c.w_ld_ch, kChunk, (uint32_t)bn, CU_TENSOR_MAP_SWIZZLE_128B, kElem);
         if (rc) return rc;
         p.src[s].a_ch_off = c.ch_off;
         p.src[s].w_ch_off = c.w_ch_off;
-        p.src[s].n_chunks = c.C_in / kBlockK;
+        p.src[s].n_chunks = c.C_in / kChunk;
         p.src[s].taps = c.taps;
         p.src[s].dil = c.dilation;
         p.src[s].pad_left = c.pad_left;
@@ -920,14 +970,24 @@ extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
         int dev = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
-        attr_err = cudaFuncSetAttribute(conv1d_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+        attr_err = cudaFuncSetAttribute(conv1d_umma_kernel<FP8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     });
     CAB_CHECK_ARG(attr_err == cudaSuccess, "cudaFuncSetAttribute(smem=%d) failed: %s", kSmemBytes, cudaGetErrorString(attr_err));
     CAB_CHECK_ARG(num_sms > 0, "no CUDA device");
     int grid = p.n_tiles < num_sms ? p.n_tiles : num_sms;
     if (p.mtile_major) grid = p.B * p.mtiles_per_b < num_sms ? p.B * p.mtiles_per_b : num_sms;
-    conv1d_umma_kernel<<<grid, kNumThreads, kSmemBytes, stream>>>(p);
+    conv1d_umma_kernel<FP8><<<grid, kNumThreads, kSmemBytes, stream>>>(p);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     return 0;
+}
+
+extern "C" int cab_conv1d_fused(const cab_conv_source_t* srcs, int n_src,
+                                const cab_conv_epilogue_t* ep, cab_stream_t stream) {
+    return conv1d_launch<false>(srcs, n_src, ep, nullptr, 1.f, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int cab_conv1d_fused_fp8(const cab_conv_source_t* srcs, int n_src, const cab_conv_epilogue_t* ep,
+                                    const float* alpha, float out_scale_inv, cab_stream_t stream) {
+    return conv1d_launch<true>(srcs, n_src, ep, alpha, out_scale_inv, static_cast<cudaStream_t>(stream));
 }

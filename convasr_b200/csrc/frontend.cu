@@ -784,3 +784,52 @@ extern "C" int cab_instnorm_pack(const float* feat, const float* xlen_frac, int 
     }
     return 0;
 }
+
+// ------------------------------------------------------------------------------------------
+// FP8 inference tier: calibration abs-max of a bf16 activation, and the E4M3 quantisation of the packed features
+// ------------------------------------------------------------------------------------------
+namespace cab {
+// 16 elements per thread: two 16-byte bf16 loads -> one 16-byte E4M3 store; q = satfinite(rn(x * scale_inv))
+__global__ void quantize_e4m3_kernel(const uint4* __restrict__ x, int64_t n16, float scale_inv, uint4* __restrict__ out) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n16; i += (int64_t)gridDim.x * blockDim.x) {
+        const uint4 a = x[2 * i], b = x[2 * i + 1];
+        const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+        uint32_t q[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const float2 lo = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[2 * k]));
+            const float2 hi = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[2 * k + 1]));
+            q[k] = (uint32_t)pack_e4m3x2(lo.x * scale_inv, lo.y * scale_inv) | ((uint32_t)pack_e4m3x2(hi.x * scale_inv, hi.y * scale_inv) << 16);
+        }
+        out[i] = make_uint4(q[0], q[1], q[2], q[3]);
+    }
+}
+}  // namespace cab
+
+extern "C" int cab_absmax_bf16(const void* x, int64_t n, float* out, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CAB_CHECK_ARG(x != nullptr && out != nullptr, "null pointer argument");
+    CAB_CHECK_ARG(n >= 0 && n <= INT32_MAX, "n=%lld out of [0, 2^31)", (long long)n);
+    CAB_CHECK_CUDA(cudaMemsetAsync(out, 0, sizeof(float), stream));
+    if (n == 0) return 0;
+    const dim3 grid((unsigned)((n + 256 * 16 - 1) / (256 * 16)), 1);
+    absmax_kernel<__nv_bfloat16><<<grid, 256, 0, stream>>>(static_cast<const __nv_bfloat16*>(x), (int)n, out);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
+
+extern "C" int cab_quantize_e4m3(const void* x, int64_t n, float scale_inv, void* out, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CAB_CHECK_ARG(x != nullptr && out != nullptr, "null pointer argument");
+    CAB_CHECK_ARG(n >= 0 && n % 16 == 0, "n=%lld must be a multiple of 16", (long long)n);
+    CAB_CHECK_ARG((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, "x and out must be 16-byte aligned");
+    if (n == 0) return 0;
+    const int64_t n16 = n / 16;
+    const int64_t blocks = (n16 + 255) / 256;
+    quantize_e4m3_kernel<<<(unsigned)(blocks < 148 * 8 ? blocks : 148 * 8), 256, 0, stream>>>(static_cast<const uint4*>(x), n16, scale_inv,
+                                                                                             static_cast<uint4*>(out));
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}

@@ -14,6 +14,9 @@
 //   x tile: the input channels those 64 outputs need (<= 104), 64 + K - 1 frames, raw bf16 in smem,
 //           double buffered with cp.async (zero fill = conv padding): the next tile lands during
 //           the current tile's math; bf16 -> fp32 is a shift at load time.
+//   FP8 (inference tier): x and the output are E4M3 -- the tile holds raw bytes (16 channels per 16-byte vector), a channel
+//           pair is dequantised with one cvt (x = q * in_scale, the scale applied once to the sum), and the output is
+//           stored as satfinite(rn(v / s_out)).
 #include "common.cuh"
 #include "../../include/convasr_b200.h"
 #include <atomic>
@@ -51,6 +54,7 @@ struct GroupedArgs {
     int ld_dy, dy_T_rows;
     float* dw;          // wgrad: fp32 [C_out][cin_g][K], zeroed by the host wrapper
     float* db;          // wgrad: fp32 [C_out] or null
+    float in_scale, out_inv;  // FP8: x = q * in_scale; stored q = v * out_inv
 };
 
 __device__ __forceinline__ void cp_async_16(uint32_t smem_dst, const void* gsrc, bool valid) {
@@ -72,12 +76,21 @@ __device__ __forceinline__ float2 load_pair(const unsigned char* p) {
     return make_float2(__uint_as_float(a << 16), __uint_as_float(b << 16));
 }
 
-template <int K, bool HAS_LO, bool ALIGNED>
+// two adjacent E4M3 channels -> float2 (exact)
+template <bool ALIGNED>
+__device__ __forceinline__ float2 load_pair_e4m3(const unsigned char* p) {
+    if (ALIGNED) return unpack_e4m3x2(*reinterpret_cast<const uint16_t*>(p));
+    return unpack_e4m3x2((uint16_t)(p[0] | (p[1] << 8)));
+}
+
+template <int K, bool HAS_LO, bool ALIGNED, bool FP8 = false>
 __global__ void __launch_bounds__(kGcThreads, 2)
 grouped_conv_ffma2_kernel(const GroupedArgs p) {
     constexpr int kRows = kGcTile + K - 1;   // frames in the x tile
     constexpr int kWin = kGcTT + K - 1;      // frames one thread slides over
     constexpr int NT = HAS_LO ? 2 : 1;       // tensors per tile (hi, lo)
+    constexpr int E = FP8 ? 1 : 2;           // bytes per element
+    constexpr int kVecCh = 16 / E;           // channels per 16-byte vector
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int cin_g = p.C_in / p.groups, cout_g = p.C_out / p.groups;
     const int n_jp = (cin_g + 1) / 2;
@@ -94,9 +107,9 @@ grouped_conv_ffma2_kernel(const GroupedArgs p) {
     const int co_last = min(cb * kGcCo + kGcCo, p.C_out) - 1;
     const int ci_first = co_last >= cb * kGcCo ? (cb * kGcCo / cout_g) * cin_g : 0;
     const int ci_end = co_last >= cb * kGcCo ? (co_last / cout_g + 1) * cin_g + 1 : 8;  // +1: pad channel of an odd cin_g
-    const int ci_lo = ci_first & ~7;
-    const int cols = ((ci_end - ci_lo + 7) & ~7);
-    const int n_vec = cols / 8;
+    const int ci_lo = ci_first & ~(kVecCh - 1);
+    const int cols = ((ci_end - ci_lo + kVecCh - 1) & ~(kVecCh - 1));
+    const int n_vec = cols / kVecCh;
     constexpr int pitch = kGcMaxCols * 2;  // bytes, compile-time: the window loads below use immediate offsets
 
     // weights -> smem, paired over input channels: ws[jp][k][co] = (w[co][2jp][k], w[co][2jp+1][k] or 0)
@@ -112,6 +125,7 @@ grouped_conv_ffma2_kernel(const GroupedArgs p) {
     }
     const float bv = (live && p.bias) ? p.bias[co] : 0.f;
     const int col0 = live ? (co / cout_g) * cin_g - ci_lo : 0;
+    const unsigned char* const xg = reinterpret_cast<const unsigned char*>(p.x);
 
     const int total_vec = kRows * n_vec;
     auto issue = [&](int item, int buf) {
@@ -122,11 +136,11 @@ grouped_conv_ffma2_kernel(const GroupedArgs p) {
             const int idx = tid + v * kGcThreads;
             if (idx >= total_vec) break;
             const int r = idx / n_vec, cvec = idx - r * n_vec;
-            const int u = t0 - p.pad + r, ch = ci_lo + cvec * 8;
+            const int u = t0 - p.pad + r, ch = ci_lo + cvec * kVecCh;
             const bool ok = u >= 0 && u < p.T && ch < p.ld_in;
             const size_t off = ok ? ((size_t)b * p.T_rows + u) * p.ld_in + ch : 0;
             const uint32_t dst = base + r * pitch + cvec * 16;
-            cp_async_16(dst, p.x + off, ok);
+            cp_async_16(dst, xg + off * E, ok);
             if (HAS_LO) cp_async_16(dst + tile_bytes, p.x_lo + off, ok);
         }
         cp_async_commit();
@@ -143,15 +157,16 @@ grouped_conv_ffma2_kernel(const GroupedArgs p) {
         const int b = item / p.tiles_per_utt, t0 = (item - b * p.tiles_per_utt) * kGcTile;
         float2 acc[kGcTT];
 #pragma unroll
-        for (int i = 0; i < kGcTT; ++i) acc[i] = make_float2(bv, 0.f);
+        for (int i = 0; i < kGcTT; ++i) acc[i] = make_float2(FP8 ? 0.f : bv, 0.f);
         if (live) {
-            const unsigned char* xt = xs + buf * NT * tile_bytes + (strip * kGcTT) * pitch + col0 * 2;
+            const unsigned char* xt = xs + buf * NT * tile_bytes + (strip * kGcTT) * pitch + col0 * E;
             for (int jp = 0; jp < n_jp; ++jp) {
-                const unsigned char* xr = xt + jp * 4;
+                const unsigned char* xr = xt + jp * 2 * E;
                 float2 xw[kWin];
 #pragma unroll
                 for (int m = 0; m < kWin; ++m) {
-                    xw[m] = load_pair<ALIGNED>(xr + m * pitch);
+                    if (FP8) xw[m] = load_pair_e4m3<ALIGNED>(xr + m * pitch);
+                    else xw[m] = load_pair<ALIGNED>(xr + m * pitch);
                     if (HAS_LO) {  // split-bf16 ("fp32 tier"): value = hi + lo
                         const float2 l = load_pair<ALIGNED>(xr + tile_bytes + m * pitch);
                         xw[m].x += l.x;
@@ -167,7 +182,18 @@ grouped_conv_ffma2_kernel(const GroupedArgs p) {
                 }
             }
         }
-        if (co < p.ld_out) {
+        if (FP8 && co < p.ld_out) {
+            const int t_first = t0 + strip * kGcTT;
+            unsigned char* o = reinterpret_cast<unsigned char*>(p.out) + ((size_t)b * p.out_T_rows + t_first) * p.ld_out + co;
+            const int n_t = min(kGcTT, p.T - t_first);
+#pragma unroll
+            for (int i = 0; i < kGcTT; ++i) {
+                if (i < n_t) {
+                    const float v = live ? (p.relu ? fmaxf(fmaf(acc[i].x + acc[i].y, p.in_scale, bv), 0.f) : fmaf(acc[i].x + acc[i].y, p.in_scale, bv)) : 0.f;
+                    o[(size_t)i * p.ld_out] = (unsigned char)(pack_e4m3x2(v * p.out_inv, 0.f) & 0xffu);
+                }
+            }
+        } else if (co < p.ld_out) {
             const int t_first = t0 + strip * kGcTT;
             __nv_bfloat16* o_hi = p.out + ((size_t)b * p.out_T_rows + t_first) * p.ld_out + co;
             __nv_bfloat16* o_lo = HAS_LO && p.out_lo ? p.out_lo + ((size_t)b * p.out_T_rows + t_first) * p.ld_out + co : nullptr;
@@ -197,36 +223,39 @@ static int gc_num_sms() {
     return n;
 }
 
-static size_t grouped_smem_bytes(int cin_g, int K, int cols_max, bool has_lo) {
+static size_t grouped_smem_bytes(int cin_g, int K, int cols_max, bool has_lo) {  // (the tile's byte size is the same for E4M3)
     return sizeof(float2) * ((cin_g + 1) / 2) * K * kGcCo + (size_t)2 * (has_lo ? 2 : 1) * (kGcTile + K - 1) * kGcMaxCols * 2;
 }
 
-template <int K, bool HAS_LO, bool ALIGNED>
+template <int K, bool HAS_LO, bool ALIGNED, bool FP8 = false>
 static int launch_grouped_t(const GroupedArgs& a, int n_cb, cudaStream_t stream) {
     const size_t smem = grouped_smem_bytes(a.C_in / a.groups, K, a.cols_max, HAS_LO);
     static size_t smem_set = 0;
     if (smem > smem_set) {
-        CAB_CHECK_CUDA(cudaFuncSetAttribute(grouped_conv_ffma2_kernel<K, HAS_LO, ALIGNED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CAB_CHECK_CUDA(cudaFuncSetAttribute(grouped_conv_ffma2_kernel<K, HAS_LO, ALIGNED, FP8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         smem_set = smem;
     }
-    grouped_conv_ffma2_kernel<K, HAS_LO, ALIGNED><<<dim3(n_cb, a.parts), kGcThreads, smem, stream>>>(a);
+    grouped_conv_ffma2_kernel<K, HAS_LO, ALIGNED, FP8><<<dim3(n_cb, a.parts), kGcThreads, smem, stream>>>(a);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     return 0;
 }
 
 template <int K>
-static int launch_grouped(const GroupedArgs& a, int n_cb, cudaStream_t stream) {
+static int launch_grouped(const GroupedArgs& a, int n_cb, cudaStream_t stream, bool fp8 = false) {
     const bool aligned = (a.C_in / a.groups) % 2 == 0;
+    if (fp8) return aligned ? launch_grouped_t<K, false, true, true>(a, n_cb, stream) : launch_grouped_t<K, false, false, true>(a, n_cb, stream);
     if (a.x_lo) return aligned ? launch_grouped_t<K, true, true>(a, n_cb, stream) : launch_grouped_t<K, true, false>(a, n_cb, stream);
     return aligned ? launch_grouped_t<K, false, true>(a, n_cb, stream) : launch_grouped_t<K, false, false>(a, n_cb, stream);
 }
 
 // returns 1 when this shape is not covered (caller runs the generic kernel), 0 on launch, < 0 on error
+// fp8: E4M3 act and out (act_lo / out_lo null), x = q * in_scale, stored q = v * out_inv
 int grouped_conv_fast(const void* act, const void* act_lo, int B, int T, int T_rows, int C_in, int ld_in, const float* wgt,
                       const float* bias, int C_out, int groups, int k, int pad_left, void* out, void* out_lo,
-                      int out_T_rows, int ld_out, int relu, cudaStream_t stream) {
-    if (ld_in % 8 != 0 || C_in % groups != 0 || C_out % groups != 0) return 1;
+                      int out_T_rows, int ld_out, int relu, cudaStream_t stream, bool fp8, float in_scale, float out_inv) {
+    const int vec_ch = fp8 ? 16 : 8;  // channels per 16-byte vector
+    if (ld_in % vec_ch != 0 || C_in % groups != 0 || C_out % groups != 0) return 1;
     const int cin_g = C_in / groups, cout_g = C_out / groups;
     const int n_cb = (ld_out + kGcCo - 1) / kGcCo;
     // widest input window over the channel blocks, and the prefetch budget
@@ -235,11 +264,11 @@ int grouped_conv_fast(const void* act, const void* act_lo, int B, int T, int T_r
         const int co_last = (cb * kGcCo + kGcCo < C_out ? cb * kGcCo + kGcCo : C_out) - 1;
         if (co_last < cb * kGcCo) continue;
         const int ci_first = (cb * kGcCo / cout_g) * cin_g, ci_end = (co_last / cout_g + 1) * cin_g + 1;
-        const int cols = ((ci_end - (ci_first & ~7)) + 7) & ~7;
+        const int cols = ((ci_end - (ci_first & ~(vec_ch - 1))) + vec_ch - 1) & ~(vec_ch - 1);
         cols_max = cols > cols_max ? cols : cols_max;
     }
-    if (cols_max > kGcMaxCols) return 1;
-    if ((kGcTile + k - 1) * (cols_max / 8) > kGcMaxVec * kGcThreads) return 1;
+    if (cols_max * (fp8 ? 1 : 2) > kGcMaxCols * 2) return 1;  // tile row: kGcMaxCols * 2 bytes
+    if ((kGcTile + k - 1) * (cols_max / vec_ch) > kGcMaxVec * kGcThreads) return 1;
     const size_t smem = grouped_smem_bytes(cin_g, k, cols_max, act_lo != nullptr);
     if (smem > 200 * 1024) return 1;
     const int ctas_per_sm = smem > 113 * 1024 ? 1 : 2;
@@ -247,7 +276,7 @@ int grouped_conv_fast(const void* act, const void* act_lo, int B, int T, int T_r
     a.x = static_cast<const __nv_bfloat16*>(act); a.x_lo = static_cast<const __nv_bfloat16*>(act_lo); a.w = wgt; a.bias = bias;
     a.out = static_cast<__nv_bfloat16*>(out); a.out_lo = static_cast<__nv_bfloat16*>(out_lo);
     a.B = B; a.T = T; a.T_rows = T_rows; a.C_in = C_in; a.ld_in = ld_in; a.C_out = C_out; a.ld_out = ld_out; a.out_T_rows = out_T_rows;
-    a.groups = groups; a.pad = pad_left; a.cols_max = cols_max; a.relu = relu;
+    a.groups = groups; a.pad = pad_left; a.cols_max = cols_max; a.relu = relu; a.in_scale = in_scale; a.out_inv = out_inv;
     a.tiles_per_utt = (T + kGcTile - 1) / kGcTile;
     a.n_items = B * a.tiles_per_utt;
     // one wave: every CTA must be resident at once (2 per SM), a 297th CTA would run alone afterwards
@@ -255,19 +284,19 @@ int grouped_conv_fast(const void* act, const void* act_lo, int B, int T, int T_r
     parts = parts < 1 ? 1 : parts;
     a.parts = parts < a.n_items ? parts : a.n_items;
     switch (k) {
-        case 3: return launch_grouped<3>(a, n_cb, stream);
-        case 5: return launch_grouped<5>(a, n_cb, stream);
-        case 7: return launch_grouped<7>(a, n_cb, stream);
-        case 9: return launch_grouped<9>(a, n_cb, stream);
-        case 11: return launch_grouped<11>(a, n_cb, stream);
-        case 13: return launch_grouped<13>(a, n_cb, stream);
-        case 15: return launch_grouped<15>(a, n_cb, stream);
-        case 17: return launch_grouped<17>(a, n_cb, stream);
-        case 19: return launch_grouped<19>(a, n_cb, stream);
-        case 21: return launch_grouped<21>(a, n_cb, stream);
-        case 23: return launch_grouped<23>(a, n_cb, stream);
-        case 25: return launch_grouped<25>(a, n_cb, stream);
-        case 27: return launch_grouped<27>(a, n_cb, stream);
+        case 3: return launch_grouped<3>(a, n_cb, stream, fp8);
+        case 5: return launch_grouped<5>(a, n_cb, stream, fp8);
+        case 7: return launch_grouped<7>(a, n_cb, stream, fp8);
+        case 9: return launch_grouped<9>(a, n_cb, stream, fp8);
+        case 11: return launch_grouped<11>(a, n_cb, stream, fp8);
+        case 13: return launch_grouped<13>(a, n_cb, stream, fp8);
+        case 15: return launch_grouped<15>(a, n_cb, stream, fp8);
+        case 17: return launch_grouped<17>(a, n_cb, stream, fp8);
+        case 19: return launch_grouped<19>(a, n_cb, stream, fp8);
+        case 21: return launch_grouped<21>(a, n_cb, stream, fp8);
+        case 23: return launch_grouped<23>(a, n_cb, stream, fp8);
+        case 25: return launch_grouped<25>(a, n_cb, stream, fp8);
+        case 27: return launch_grouped<27>(a, n_cb, stream, fp8);
         default: return 1;
     }
 }

@@ -10,6 +10,12 @@ bias/activation/mask run in the TMEM epilogue.
 HBM layout: activations are bf16 channels-last [B, T, C_alloc] (C_alloc = C rounded up to 64),
 weights are bf16 tap-major [taps, C_out, C_in_alloc].  The "fp32" precision tier keeps every
 activation and weight as a (hi, lo) bf16 pair and accumulates hi*hi + hi*lo + lo*hi in fp32.
+
+The "fp8" tier (inference only) stores every activation as E4M3 with one static fp32 scale per tensor (from a
+calibration run of the bf16 plan, keyed by the launch that produces the tensor) and every weight as E4M3 with one
+scale per output channel.  The sources of a launch share one accumulator: source j's weights absorb its input scale s_j,
+W~_j = e4m3(W_j * s_j / alpha[n]) with alpha[n] = max_j(s_j * max|W_j[n]|) / 448, and the epilogue multiplies by
+alpha[n].  Contracted widths are multiples of 128 there (C_alloc = C rounded up to 128).
 """
 import torch
 import torch.nn as nn
@@ -17,6 +23,8 @@ import torch.nn as nn
 from . import _lib, ops
 
 BF16 = torch.bfloat16
+FP8 = torch.float8_e4m3fn
+E4M3_MAX = 448.0
 
 
 def _ceil_to(x, m):
@@ -86,11 +94,37 @@ def act_code(nonlinearity):
 	return _ACT_CODES[name], 0.0, 0.0
 
 
+def e4m3(x):
+	"""fp32 -> E4M3 with saturation at +-448 (torch's float8_e4m3fn cast turns values past the largest finite into NaN;
+	cvt.rn.satfinite, which the kernels use, clamps)"""
+	return x.clamp(-E4M3_MAX, E4M3_MAX).to(FP8)
+
+
+def fp8_scale(amax):
+	"""per-tensor activation scale: x / scale spans the E4M3 range; an all-zero tensor gets 1"""
+	amax = float(amax)
+	return amax / E4M3_MAX if amax > 0 else 1.0
+
+
+def quantize_sources_fp8(ws, scales):
+	"""E4M3 weights of one launch's sources sharing an accumulator.  ws: fp32 packed weights [taps, rows, c_in] (rows may
+	differ), scales: the input scale of each source.  Returns ([W~_j], alpha fp32 [max rows]) with
+	alpha[n] = max_j(s_j * max|W_j[n]|) / 448 (1 where every weight of row n is zero) and W~_j = e4m3(W_j * s_j / alpha[n])."""
+	rows = max(w.shape[1] for w in ws)
+	peak = torch.zeros(rows, dtype = torch.float32, device = ws[0].device)
+	for w, s in zip(ws, scales):
+		peak[:w.shape[1]] = torch.maximum(peak[:w.shape[1]], w.abs().amax(dim = (0, 2)) * s)
+	alpha = torch.where(peak > 0, peak / E4M3_MAX, torch.ones_like(peak))
+	return [e4m3(w * (s / alpha[:w.shape[1]]).view(1, -1, 1)).contiguous() for w, s in zip(ws, scales)], alpha.contiguous()
+
+
 class _Weights:
-	"""a packed weight in the active precision tier"""
+	"""a packed weight in the active precision tier ('fp8': the fp32 packing is kept until the plan quantises it)"""
 
 	def __init__(self, w_f32, fp32_tier):
-		if fp32_tier:
+		if fp32_tier == 'fp8':
+			self.f32, self.hi, self.lo = w_f32, None, None
+		elif fp32_tier:
 			self.hi, self.lo = _split(w_f32)
 			self.hi, self.lo = self.hi.contiguous(), self.lo.contiguous()
 		else:
@@ -125,6 +159,20 @@ class _Launch:
 		self.stride2 = None  # (k, pad) of the original strided conv
 		self.grouped = None  # (weight fp32, bias fp32, groups, pad_left, C_mid, C_mid_alloc)
 		self.epilogue = _lib.EPI_ACT_BF16
+		self.key = self.tmp_key = None  # calibration keys of the output / grouped-conv activation
+		self.alpha = None  # fp8 tier: per-column accumulator multiplier [C_alloc]
+		self.in_scale = self.tmp_scale = self.out_scale = 1.0  # fp8 tier: scales of the running input, grouped output, output
+
+
+def next_residuals(i, n_blocks, plan, residuals, x):
+	"""residual bookkeeping of JasperNet.forward after block i (models.py:306-313)"""
+	if i >= n_blocks - plan.num_epilogue_modules - 1:
+		return []
+	if plan.residual_mode == 'dense':
+		return residuals + [x]
+	if plan.residual_mode:
+		return [x]
+	return []
 
 
 class StackPlan:
@@ -132,16 +180,59 @@ class StackPlan:
 
 	_epochs = 0
 
-	def __init__(self, model, fp32_tier):
+	def __init__(self, model, fp32_tier, fp8_scales = None):
+		"""fp8_scales: {activation key: scale} from a calibration run (JasperNet.calibrate_fp8) selects the fp8 tier"""
 		StackPlan._epochs += 1
 		self.epoch = StackPlan._epochs  # monotonically increasing identity (id() can be reused after a plan is freed)
-		self.fp32_tier = fp32_tier
+		self.fp8 = fp8_scales is not None
+		self.fp32_tier = fp32_tier and not self.fp8
+		self._wmode = 'fp8' if self.fp8 else self.fp32_tier
+		self.align = 128 if self.fp8 else 64  # channel allocation granularity (one 128-byte swizzle row of the operand)
 		self.blocks = []  # list of list of _Launch (one list per ConvBn1d)
 		self.residual_mode = model.residual
 		self.num_epilogue_modules = model.num_epilogue_modules
 		for block in model.backbone:
 			self.blocks.append(self._plan_convbn(block))
 		self.heads = self._plan_decoder(model.decoder)
+		# the features are packed 64 wide for a stride-2 prologue (its frame-pair view is then 128 wide), else like every activation
+		self.feat_align = 64 if self.blocks[0][0].stride2 is not None else self.align
+		self._assign_keys()
+		if self.fp8:
+			self._quantize_fp8(fp8_scales)
+
+	def _assign_keys(self):
+		"""name every activation by the launch that produces it ('feat' for the packed features); record each source's key"""
+		x, residuals = 'feat', []
+		for i, launches in enumerate(self.blocks):
+			for j, L in enumerate(launches):
+				L.key, L.tmp_key, L.in_key = ('block', i, j), ('grouped', i, j), x
+				for g in L.gemms:
+					g.in_key = x if g.src == 'x' else L.tmp_key if g.src == 'tmp' else residuals[g.src]
+				x = L.key
+			residuals = next_residuals(i, len(self.blocks), self, residuals, x)
+		for h, chain in enumerate(self.heads):
+			hx = x
+			for j, L in enumerate(chain):
+				L.key, L.tmp_key, L.in_key = ('head', h, j), ('head_grouped', h, j), hx
+				for g in L.gemms:
+					g.in_key = hx if g.src == 'x' else L.tmp_key
+				hx = L.key
+
+	def launches(self):
+		return [L for launches in self.blocks for L in launches] + [L for chain in self.heads for L in chain]
+
+	def _quantize_fp8(self, scales):
+		missing = sorted({g.in_key for L in self.launches() for g in L.gemms if g.in_key not in scales}, key = str)
+		if missing:
+			raise RuntimeError(f'convasr_b200: no fp8 calibration scale for activations {missing}; call model.calibrate_fp8(x, xlen)')
+		for L in self.launches():
+			wq, alpha = quantize_sources_fp8([g.weights.f32 for g in L.gemms], [scales[g.in_key] for g in L.gemms])
+			for g, w in zip(L.gemms, wq):
+				g.weights.hi, g.weights.f32 = w, None
+			L.alpha = torch.cat([alpha, torch.ones(max(L.C_alloc - alpha.numel(), 0), device = alpha.device)]).contiguous()
+			L.in_scale = scales[L.in_key]
+			L.tmp_scale = scales.get(L.tmp_key, 1.0)
+			L.out_scale = scales.get(L.key, 1.0)
 
 	# -- planning ---------------------------------------------------------------------------
 	def _plan_convbn(self, m, final_logits = False, mask = None):
@@ -154,19 +245,19 @@ class StackPlan:
 			k, stride, dil = first.kernel_size[0], first.stride[0], first.dilation[0]
 			pad = first.padding[0]
 			C_in, C_out = first.in_channels, seq[-1].out_channels
-			c_in_alloc = _ceil_to(C_in, 64)
-			L.C_out, L.C_alloc = C_out, _ceil_to(C_out, 64)
+			c_in_alloc = _ceil_to(C_in, 64 if stride == 2 else self.align)  # stride 2: the pair view doubles it
+			L.C_out, L.C_alloc = C_out, _ceil_to(C_out, self.align)
 			L.dT = 2 * pad - dil * (k - 1)
 			bias = torch.zeros(L.C_alloc, dtype = torch.float32, device = first.weight.device)
 			if len(seq) == 3:  # separable: grouped conv + bias + ReLU, then pointwise (+BN)
 				if stride != 1 or dil != 1:
 					raise NotImplementedError('convasr_b200: strided/dilated separable conv')
 				C_mid = first.out_channels
-				c_mid_alloc = _ceil_to(C_mid, 64)
+				c_mid_alloc = _ceil_to(C_mid, self.align)
 				gb = first.bias.detach().float().contiguous() if first.bias is not None else None
 				L.grouped = (first.weight.detach().float().contiguous(), gb, first.groups, pad, C_mid, c_mid_alloc, C_in)
 				w, b = fold_bn(seq[2].weight, seq[2].bias, m.bn[j])
-				L.gemms.append(_Gemm('tmp', _Weights(pack_taps(w, c_mid_alloc), self.fp32_tier), c_mid_alloc, 1, 1, 0))
+				L.gemms.append(_Gemm('tmp', _Weights(pack_taps(w, c_mid_alloc), self._wmode), c_mid_alloc, 1, 1, 0))
 			else:
 				if first.groups != 1:
 					raise NotImplementedError('convasr_b200: grouped non-separable conv')
@@ -176,9 +267,9 @@ class StackPlan:
 						raise NotImplementedError('convasr_b200: dilated strided conv')
 					wp, taps, pad_left = pack_taps_stride2(w, pad, c_in_alloc)
 					L.stride2 = (k, pad)
-					L.gemms.append(_Gemm('x', _Weights(wp, self.fp32_tier), 2 * c_in_alloc, taps, 1, pad_left, pair_view = True))
+					L.gemms.append(_Gemm('x', _Weights(wp, self._wmode), 2 * c_in_alloc, taps, 1, pad_left, pair_view = True))
 				elif stride == 1:
-					L.gemms.append(_Gemm('x', _Weights(pack_taps(w, c_in_alloc), self.fp32_tier), c_in_alloc, k, dil, pad))
+					L.gemms.append(_Gemm('x', _Weights(pack_taps(w, c_in_alloc), self._wmode), c_in_alloc, k, dil, pad))
 				else:
 					raise NotImplementedError(f'convasr_b200: conv stride {stride}')
 			bias[:C_out] += b
@@ -186,11 +277,11 @@ class StackPlan:
 				for r, (rc, rbn) in enumerate(zip(m.conv_residual, m.bn_residual)):
 					if isinstance(rc, nn.Identity):  # 'flat' residual: identity 1x1
 						w = torch.eye(C_out, device = bias.device).unsqueeze(-1)
-						L.gemms.append(_Gemm(r, _Weights(pack_taps(w, L.C_alloc), self.fp32_tier), L.C_alloc, 1, 1, 0))
+						L.gemms.append(_Gemm(r, _Weights(pack_taps(w, L.C_alloc), self._wmode), L.C_alloc, 1, 1, 0))
 					else:
 						w, b = fold_bn(rc.weight, rc.bias, rbn)
-						rc_in_alloc = _ceil_to(rc.in_channels, 64)
-						L.gemms.append(_Gemm(r, _Weights(pack_taps(w, rc_in_alloc), self.fp32_tier), rc_in_alloc, 1, 1, 0))
+						rc_in_alloc = _ceil_to(rc.in_channels, self.align)
+						L.gemms.append(_Gemm(r, _Weights(pack_taps(w, rc_in_alloc), self._wmode), rc_in_alloc, 1, 1, 0))
 						bias[:C_out] += b
 			L.bias = bias.contiguous()
 			act = m.activation.nonlinearity
@@ -206,8 +297,8 @@ class StackPlan:
 		conv0 = decoder[0]
 		L = _Launch()
 		w, b = fold_bn(conv0.weight, conv0.bias, None)
-		c_in_alloc = _ceil_to(conv0.in_channels, 64)
-		L.gemms.append(_Gemm('x', _Weights(pack_taps(w, c_in_alloc), self.fp32_tier), c_in_alloc, conv0.kernel_size[0], 1, conv0.padding[0]))
+		c_in_alloc = _ceil_to(conv0.in_channels, self.align)
+		L.gemms.append(_Gemm('x', _Weights(pack_taps(w, c_in_alloc), self._wmode), c_in_alloc, conv0.kernel_size[0], 1, conv0.padding[0]))
 		L.bias = b.contiguous()
 		L.C_out = L.C_alloc = conv0.out_channels
 		L.dT = 2 * conv0.padding[0] - (conv0.kernel_size[0] - 1)
@@ -259,13 +350,18 @@ class StackPlan:
 			srcs = [ops.Source(part_hi, eye, C_alloc, 1, 1, 0, T_in = T_out)] + ([ops.Source(part_lo, eye, C_alloc, 1, 1, 0, T_in = T_out)] if part_lo is not None else []) + srcs
 		return srcs
 
-	def _run_launch(self, L, x, residuals, xlen, B):
+	def _run_launch(self, L, x, residuals, xlen, B, observe = None):
 		dev = x.hi.device
 		tmp = None
 		if L.grouped is not None:
 			gw, gb, groups, gpad, C_mid, c_mid_alloc, C_in = L.grouped
-			t_hi, t_lo = ops.grouped_conv1d_relu(x.hi, x.T, C_in, gw, gb, groups, gpad, ld_out = c_mid_alloc, act_lo = x.lo, want_lo = self.fp32_tier)
+			if self.fp8:
+				t_hi, t_lo = ops.grouped_conv1d_fp8(x.hi, x.T, C_in, L.in_scale, gw, gb, groups, gpad, c_mid_alloc, L.tmp_scale), None
+			else:
+				t_hi, t_lo = ops.grouped_conv1d_relu(x.hi, x.T, C_in, gw, gb, groups, gpad, ld_out = c_mid_alloc, act_lo = x.lo, want_lo = self.fp32_tier)
 			tmp = _Act(t_hi, t_lo, x.T, C_mid)
+			if observe is not None:
+				observe(L.tmp_key, t_hi)
 		if L.stride2 is not None:
 			k, pad = L.stride2
 			T_out = (x.T + 2 * pad - (k - 1) - 1) // 2 + 1
@@ -273,6 +369,8 @@ class StackPlan:
 			T_out = x.T + L.dT
 		srcs = self._sources(L, x, tmp, residuals)
 		code, a, b = L.act
+		if self.fp8:
+			return self._run_epilogue_fp8(L, srcs, xlen, B, T_out, dev)
 		if L.epilogue == _lib.EPI_ACT_BF16:
 			srcs = self._fold_excess_sources(srcs, B, T_out, L.C_alloc, dev)
 			out_hi = torch.empty(B, T_out, L.C_alloc, dtype = BF16, device = dev)
@@ -292,30 +390,50 @@ class StackPlan:
 			log_probs, argmax = ops.log_softmax_argmax(logits)
 		return logits, log_probs, argmax
 
-	def run(self, feats, xlen):
-		"""feats: _Act holding the normalised features [B, F_pad, C_alloc]; returns per head
-		(logits, log_probs, argmax)."""
+	def _run_epilogue_fp8(self, L, srcs, xlen, B, T_out, dev):
+		if len(srcs) > _lib.MAX_CONV_SOURCES:
+			raise NotImplementedError(f'convasr_b200: {len(srcs)} operand pairs in one fp8 launch (at most {_lib.MAX_CONV_SOURCES})')
+		code, a, b = L.act
+		if L.epilogue == _lib.EPI_ACT_BF16:
+			out = torch.empty(B, T_out, L.C_alloc, dtype = FP8, device = dev)
+			ops.conv1d_fused_fp8(srcs, B, T_out, L.C_alloc, L.alpha, 1.0 / L.out_scale, bias = L.bias, act = code, act_a = a, act_b = b, xlen = xlen if L.mask else None, out = out)
+			return _Act(out, None, T_out, L.C_out)
+		if L.epilogue == _lib.EPI_LOGSOFTMAX:
+			logits = torch.empty(B, L.C_out, T_out, dtype = torch.float32, device = dev)
+			log_probs = torch.empty_like(logits)
+			argmax = torch.empty(B, T_out, dtype = torch.int32, device = dev)
+			ops.conv1d_fused_fp8(srcs, B, T_out, L.C_out, L.alpha, bias = L.bias, logits = logits, log_probs = log_probs, argmax = argmax, epilogue = _lib.EPI_LOGSOFTMAX)
+		elif code == _lib.ACT_NONE:
+			return ops.large_vocab_head(srcs, B, T_out, L.C_out, L.bias, alpha = L.alpha)
+		else:
+			logits = torch.empty(B, L.C_out, T_out, dtype = torch.float32, device = dev)
+			ops.conv1d_fused_fp8(srcs, B, T_out, L.C_out, L.alpha, bias = L.bias, act = code, act_a = a, act_b = b, logits = logits, epilogue = _lib.EPI_LOGITS_F32)
+			log_probs, argmax = ops.log_softmax_argmax(logits)
+		return logits, log_probs, argmax
+
+	def run(self, feats, xlen, observe = None):
+		"""feats: _Act holding the normalised features [B, F_pad, C_alloc] (E4M3 in the fp8 tier, already divided by the
+		'feat' scale); returns per head (logits, log_probs, argmax).  observe(key, tensor): called with every activation the
+		plan produces (calibration)."""
 		B = feats.hi.shape[0]
 		x = feats
+		if observe is not None:
+			observe('feat', feats.hi)
 		residuals = []
 		n_blocks = len(self.blocks)
 		for i, launches in enumerate(self.blocks):
 			for L in launches:
-				x = self._run_launch(L, x, residuals, xlen, B)
-			# residual bookkeeping of JasperNet.forward, models.py:306-313
-			if i >= n_blocks - self.num_epilogue_modules - 1:
-				residuals = []
-			elif self.residual_mode == 'dense':
-				residuals.append(x)
-			elif self.residual_mode:
-				residuals = [x]
-			else:
-				residuals = []
+				x = self._run_launch(L, x, residuals, xlen, B, observe)
+				if observe is not None:
+					observe(L.key, x.hi)
+			residuals = next_residuals(i, n_blocks, self, residuals, x)
 		outs = []
 		for chain in self.heads:
 			h = x
 			for L in chain:
-				h = self._run_launch(L, h, [], None, B)
+				h = self._run_launch(L, h, [], None, B, observe)
+				if observe is not None and isinstance(h, _Act):
+					observe(L.key, h.hi)
 			outs.append(h)
 		return outs
 

@@ -358,8 +358,9 @@ class JasperNet(nn.Module):
 		self.dict = dict
 		self.bpe_only = bpe_only
 		self.check_time_dim_padded = check_time_dim_padded
-		self.precision = precision  # None = follow the parameter dtype; 'bf16' | 'fp32'
+		self.precision = precision  # None = follow the parameter dtype; 'bf16' | 'fp32' | 'fp8' (eval only)
 		self._plan = None
+		self._fp8_calibration = None  # (parameter signature, {activation key: scale}); deliberately not in state_dict
 		self._graphs_enabled = os.environ.get('CONVASR_B200_CUDA_GRAPHS', '0') == '1'
 		self._graphs_max = 4
 		self._graphs = {}
@@ -367,9 +368,10 @@ class JasperNet(nn.Module):
 	# -- precision tier -------------------------------------------------------------------
 	def set_precision(self, precision):
 		"""'bf16': single bf16 operands (speed tier).  'fp32': split-bf16 hi/lo operands with fp32
-		accumulation (matches the reference's fp32 path to ~1e-5).  None: decide from the
+		accumulation (matches the reference's fp32 path to ~1e-5).  'fp8': eval-only serving tier, E4M3
+		activations and weights with fp32 accumulation; needs calibrate_fp8() first.  None: decide from the
 		parameter dtype (fp32 params -> 'fp32', half/bfloat16 params -> 'bf16')."""
-		assert precision in (None, 'bf16', 'fp32')
+		assert precision in (None, 'bf16', 'fp32', 'fp8')
 		self.precision = precision
 		self._plan = None
 		return self
@@ -381,15 +383,57 @@ class JasperNet(nn.Module):
 		w = self.decoder[0].weight
 		return 'fp32' if w.dtype == torch.float32 else 'bf16'
 
-	def _get_plan(self):
-		prec = self._active_precision()
+	def train(self, mode = True):
+		if mode and self._active_precision() == 'fp8':
+			raise RuntimeError("convasr_b200: the fp8 tier is inference only (there is no fp8 training); call set_precision('bf16') or set_precision('fp32') before model.train()")
+		return super().train(mode)
+
+	def _params_sig(self):
 		# _state_epoch: bumped by everything that writes parameters / running statistics through raw pointers without
 		# touching a tensor version (native training forward, CUDA-graph replays of a training step)
-		sig = (prec, getattr(self, '_state_epoch', 0), engine.params_signature(self.backbone), engine.params_signature(self.decoder))
+		return (getattr(self, '_state_epoch', 0), engine.params_signature(self.backbone), engine.params_signature(self.decoder))
+
+	def _get_plan(self):
+		prec = self._active_precision()
+		sig = (prec, ) + self._params_sig()
 		if self._plan is None or self._plan[0] != sig:
+			scales = None
+			if prec == 'fp8':
+				if self._fp8_calibration is None:
+					raise RuntimeError('convasr_b200: the fp8 tier needs activation scales; call model.calibrate_fp8(x, xlen) first')
+				if self._fp8_calibration[0] != self._params_sig():
+					raise RuntimeError('convasr_b200: parameters or running statistics changed since the fp8 calibration; call model.calibrate_fp8(x, xlen) again')
+				scales = self._fp8_calibration[1]
 			with torch.no_grad():
-				self._plan = (sig, engine.StackPlan(self, fp32_tier = prec == 'fp32'))
+				self._plan = (sig, engine.StackPlan(self, fp32_tier = prec == 'fp32', fp8_scales = scales))
 		return self._plan[1]
+
+	@torch.no_grad()
+	def calibrate_fp8(self, x, xlen = None):
+		"""Static activation scales of the fp8 tier: runs the bf16 plan once on (x, xlen) -- inputs as for forward -- and
+		records max |a| of every activation it produces (features, every launch output, every grouped-conv output) with
+		one abs-max kernel each; scale = max / 448.  The scales belong to the current parameters: after a training step or
+		any parameter change the fp8 forward raises until this is called again.  They are not part of state_dict."""
+		if not x.is_cuda:
+			raise RuntimeError('convasr_b200: model inputs must be CUDA tensors (there is no CPU fallback)')
+		if xlen is not None:
+			xlen = xlen.to(device = x.device, dtype = torch.float32).contiguous()
+		if self.frontend is not None:
+			x = x.squeeze(1) if x.ndim == 3 else x
+		plan = engine.StackPlan(self, fp32_tier = False)
+		keys, amax = [], []
+
+		def observe(key, t):
+			keys.append(key)
+			amax.append(ops.absmax_bf16(t))
+
+		hi, _, Fr, C = self._packed_features(x, xlen, False)
+		plan.run(engine._Act(hi, None, Fr, C), xlen, observe = observe)
+		values = torch.cat(amax).tolist()  # one device -> host copy
+		self._fp8_calibration = (self._params_sig(), {k: engine.fp8_scale(v) for k, v in zip(keys, values)})
+		self._plan = None
+		self._graphs = {}
+		return self
 
 	# -- forward --------------------------------------------------------------------------
 	def forward(self, x, xlen = None, y = None, ylen = None):
@@ -407,6 +451,8 @@ class JasperNet(nn.Module):
 		assert (not self.check_time_dim_padded) or (n_frames % 32 == 0), 'Shape of features after frontend is not divisible by 32'
 
 		if self.training:
+			if self._active_precision() == 'fp8':
+				raise RuntimeError("convasr_b200: the fp8 tier is inference only (there is no fp8 training); call model.eval()")
 			from . import training
 			why = training.unsupported_reason(self)
 			if why is not None:
@@ -462,7 +508,7 @@ class JasperNet(nn.Module):
 		graph.replay()
 		return [(lg.clone(), lp.clone(), am.clone()) for lg, lp, am in outs]
 
-	def _packed_features(self, x, xlen, want_lo):
+	def _packed_features(self, x, xlen, want_lo, c_align = 64):
 		"""raw input (signal when the frontend is in the model, else fp32 features [B, C, F]) -> (bf16 hi, lo or None, frames, channels):
 		log-mel frontend + masked instance norm + channels-last packing (models.py:286-301)"""
 		nf = self.normalize_features
@@ -471,19 +517,21 @@ class JasperNet(nn.Module):
 		stride = self.backbone[0].conv[0][0].stride[0]
 		if self.frontend is not None and isinstance(self.frontend, LogFilterBankFrontend) and self.frontend.nfft == 256:
 			C = self.frontend.mel.weight.shape[0]
-			hi, lo, Fr = self.frontend.features(x, xlen, nf, stride == 2, engine._ceil_to(C, 64), want_lo)
+			hi, lo, Fr = self.frontend.features(x, xlen, nf, stride == 2, engine._ceil_to(C, c_align), want_lo)
 			return hi, lo, Fr, C
 		feats = self.frontend(x, xlen = xlen) if self.frontend is not None else x
 		B, C, Fr = feats.shape
 		F_pad = Fr + (Fr % 2) if stride == 2 else Fr
 		norm_xlen = xlen if (nf is not None and nf.temporal_mask) else None
-		hi, lo, _ = ops.instnorm_pack(feats, norm_xlen, nf.eps if nf is not None else -1.0, F_pad = F_pad, C_pad = engine._ceil_to(C, 64), want_lo = want_lo, normalize = nf is not None)
+		hi, lo, _ = ops.instnorm_pack(feats, norm_xlen, nf.eps if nf is not None else -1.0, F_pad = F_pad, C_pad = engine._ceil_to(C, c_align), want_lo = want_lo, normalize = nf is not None)
 		return hi, lo, Fr, C
 
 	def _raw_to_outputs(self, x, xlen):
 		"""raw input (signal or features) -> per head (logits, log_probs, argmax); kernels only"""
 		plan = self._get_plan()
-		hi, lo, Fr, C = self._packed_features(x, xlen, plan.fp32_tier)
+		hi, lo, Fr, C = self._packed_features(x, xlen, plan.fp32_tier, plan.feat_align)
+		if plan.fp8:
+			hi = ops.quantize_e4m3(hi, plan.blocks[0][0].in_scale)
 		return plan.run(engine._Act(hi, lo, Fr, C), xlen)
 
 	def _forward_native(self, x, xlen):

@@ -11,6 +11,7 @@ import torch
 from . import _lib
 
 BF16 = torch.bfloat16
+FP8 = torch.float8_e4m3fn
 
 
 def _stream():
@@ -140,8 +141,8 @@ class Source:
 	"""One (activation, packed weight) operand pair of the fused conv GEMM."""
 
 	def __init__(self, act, wgt, C_in, taps, dilation, pad_left, T_in = None, ch_off = 0, w_ch_off = 0):
-		# act: bf16 [B, T_rows, ld_ch]; wgt: bf16 [taps, w_rows, w_ld_ch]
-		assert act.dtype == BF16 and wgt.dtype == BF16 and act.is_contiguous() and wgt.is_contiguous()
+		# act: bf16 [B, T_rows, ld_ch]; wgt: bf16 [taps, w_rows, w_ld_ch] (both E4M3 for conv1d_fused_fp8)
+		assert act.dtype in (BF16, FP8) and wgt.dtype == act.dtype and act.is_contiguous() and wgt.is_contiguous()
 		self.act, self.wgt = act, wgt
 		self.C_in, self.taps, self.dilation, self.pad_left = C_in, taps, dilation, pad_left
 		self.T_in = act.shape[1] if T_in is None else T_in
@@ -165,6 +166,7 @@ def conv1d_fused(
 	[BN_SUM_REPLICAS, 2, C]): the launch is the dgrad GEMM producing dL/d(out) of a ConvBn1d repeat; its epilogue also
 	accumulates that repeat's BatchNorm-backward channel sums (cab_conv_epilogue_t.bnr_*)"""
 	_need_cuda(*(s.act for s in sources), bias, xlen, out_hi, out_lo, logits, log_probs, argmax)
+	assert all(s.act.dtype == BF16 for s in sources), 'E4M3 sources run on conv1d_fused_fp8'
 	n = len(sources)
 	arr = (_lib.ConvSource * n)(*[s.to_c() for s in sources])
 	ep = _lib.ConvEpilogue()
@@ -196,6 +198,54 @@ def conv1d_fused(
 		ep.bnr_C, ep.bnr_act, ep.bnr_act_a, ep.bnr_act_b = int(C), int(b_act), float(b_a), float(b_b)
 	rc = _lib.load().cab_conv1d_fused(arr, n, ctypes.byref(ep), _stream())
 	_lib.check(rc, 'cab_conv1d_fused')
+
+
+def conv1d_fused_fp8(
+	sources, B, T_out, C_out, alpha, out_scale_inv = 1.0, bias = None, act = _lib.ACT_NONE, act_a = 0.0, act_b = 0.0, xlen = None,
+	out = None, logits = None, log_probs = None, argmax = None, epilogue = _lib.EPI_ACT_BF16, block_n = 0
+):
+	"""cab_conv1d_fused_fp8: E4M3 sources (weights already carry their source's activation scale over alpha), fp32 alpha
+	[C_out] applied to the accumulator before the bias; EPI_ACT_BF16 stores E4M3 `out` [B, T_rows, ld] = act(.) *
+	out_scale_inv, the other epilogues write fp32 exactly as in conv1d_fused"""
+	_need_cuda(*(s.act for s in sources), alpha, bias, xlen, out, logits, log_probs, argmax)
+	assert all(s.act.dtype == FP8 for s in sources) and alpha.dtype == torch.float32 and alpha.is_contiguous() and alpha.numel() >= C_out
+	n = len(sources)
+	arr = (_lib.ConvSource * n)(*[s.to_c() for s in sources])
+	ep = _lib.ConvEpilogue()
+	ep.B, ep.T_out, ep.C_out, ep.block_n, ep.epilogue, ep.act = B, T_out, C_out, block_n, epilogue, act
+	ep.act_a, ep.act_b = float(act_a), float(act_b)
+	ep.bias = None if bias is None else bias.data_ptr()
+	ep.xlen_frac = None if xlen is None else xlen.data_ptr()
+	if out is not None:
+		assert out.dtype == FP8 and out.is_contiguous()
+		ep.out_hi = out.data_ptr()
+		ep.out_T_rows, ep.out_ld_ch = out.shape[1], out.shape[2]
+	if epilogue == _lib.EPI_LOGITS_ROWS:
+		assert logits is not None and logits.ndim == 3 and logits.is_contiguous() and logits.shape[1] == T_out
+		ep.out_T_rows, ep.out_ld_ch = T_out, logits.shape[2]
+	ep.logits = None if logits is None else logits.data_ptr()
+	ep.log_probs = None if log_probs is None else log_probs.data_ptr()
+	ep.argmax = None if argmax is None else argmax.data_ptr()
+	rc = _lib.load().cab_conv1d_fused_fp8(arr, n, ctypes.byref(ep), _p(alpha), float(out_scale_inv), _stream())
+	_lib.check(rc, 'cab_conv1d_fused_fp8')
+
+
+def absmax_bf16(x):
+	"""max |x| of a bf16 tensor as a device fp32 [1] (calibration of the FP8 tier)"""
+	_need_cuda(x)
+	assert x.dtype == BF16 and x.is_contiguous()
+	out = torch.empty(1, dtype = torch.float32, device = x.device)
+	_lib.check(_lib.load().cab_absmax_bf16(_p(x), x.numel(), _p(out), _stream()), 'cab_absmax_bf16')
+	return out
+
+
+def quantize_e4m3(x, scale):
+	"""bf16 -> E4M3 of x / scale, saturating at +-448, same shape"""
+	_need_cuda(x)
+	assert x.dtype == BF16 and x.is_contiguous()
+	out = torch.empty(x.shape, dtype = FP8, device = x.device)
+	_lib.check(_lib.load().cab_quantize_e4m3(_p(x), x.numel(), 1.0 / float(scale), _p(out), _stream()), 'cab_quantize_e4m3')
+	return out
 
 
 def conv1d_wgrad(a, a_T, M_total, bx, b_T, N_total, taps, dilation, pad_left, n_splits = 0, skip = None, out = None, alloc = None):
@@ -239,6 +289,22 @@ def grouped_conv1d_relu(act, T, C_in, wgt, bias, groups, pad_left, ld_out = None
 	return grouped_conv1d(act, T, C_in, wgt, bias, groups, pad_left, ld_out = ld_out, act_lo = act_lo, want_lo = want_lo, relu = True)
 
 
+def grouped_conv1d_fp8(act, T, C_in, in_scale, wgt, bias, groups, pad_left, ld_out, out_scale):
+	"""grouped conv + bias + ReLU of the FP8 tier: E4M3 [B, T_rows, ld_in] (value = q * in_scale) -> E4M3 [B, T, ld_out]
+	(value / out_scale, saturating)"""
+	_need_cuda(act, wgt, bias)
+	assert act.dtype == FP8 and act.is_contiguous()
+	B, T_rows, ld_in = act.shape
+	C_out, _, k = wgt.shape
+	out = torch.empty(B, T, ld_out, dtype = FP8, device = act.device)
+	rc = _lib.load().cab_grouped_conv1d_fp8(
+		_p(act), B, T, T_rows, C_in, ld_in, float(in_scale), _p(wgt), _p(bias), C_out, groups, k, pad_left, _p(out), out.shape[1], out.shape[2],
+		1.0 / float(out_scale), _stream()
+	)
+	_lib.check(rc, 'cab_grouped_conv1d_fp8')
+	return out
+
+
 def grouped_conv1d_wgrad(dy, T, x, x_T, C_in, C_out, groups, k, pad_left, db = None):
 	"""dy, x: engine._Act-like (hi, lo) bf16 channels-last; returns dW fp32 [C_out, C_in / groups, k]; db (fp32 [C_out]) is filled"""
 	_need_cuda(dy.hi, x.hi)
@@ -267,17 +333,21 @@ def log_softmax_argmax(logits, want_log_probs = True, want_argmax = True):
 	return lp, am
 
 
-def large_vocab_head(sources, B, T_out, C, bias):
+def large_vocab_head(sources, B, T_out, C, bias, alpha = None):
 	"""Decoder 1x1 conv + log_softmax + argmax for large vocabularies (models.py:26,316; transcript_generators.py:27):
 	one GEMM launch whose epilogue writes the fp32 logits once (class-contiguous rows, TMA stores) and keeps an online
 	softmax per frame across the N tiles, then one streaming pass log_probs = logits - lse.  Returns (logits, log_probs,
-	argmax) with logits / log_probs as [B, C, T] VIEWS of class-contiguous [B, T, C] memory."""
+	argmax) with logits / log_probs as [B, C, T] VIEWS of class-contiguous [B, T, C] memory.  alpha given: E4M3 sources
+	(conv1d_fused_fp8)."""
 	dev = sources[0].act.device
 	ld = (C + 3) // 4 * 4
 	logits = torch.empty(B, T_out, ld, dtype = torch.float32, device = dev)
 	lse = torch.empty(B, T_out, dtype = torch.float32, device = dev)
 	argmax = torch.empty(B, T_out, dtype = torch.int32, device = dev)
-	conv1d_fused(sources, B, T_out, C, bias = bias, logits = logits, log_probs = lse, argmax = argmax, epilogue = _lib.EPI_LOGITS_ROWS)
+	if alpha is None:
+		conv1d_fused(sources, B, T_out, C, bias = bias, logits = logits, log_probs = lse, argmax = argmax, epilogue = _lib.EPI_LOGITS_ROWS)
+	else:
+		conv1d_fused_fp8(sources, B, T_out, C, alpha, bias = bias, logits = logits, log_probs = lse, argmax = argmax, epilogue = _lib.EPI_LOGITS_ROWS)
 	log_probs = torch.empty_like(logits)
 	rc = _lib.load().cab_log_softmax_rows(_p(logits), _p(lse), B * T_out, C, ld, _p(log_probs), _stream())
 	_lib.check(rc, 'cab_log_softmax_rows')

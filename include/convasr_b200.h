@@ -167,6 +167,23 @@ typedef struct {
 int cab_conv1d_fused(const cab_conv_source_t* sources_host, int n_sources,
                      const cab_conv_epilogue_t* epilogue_host, cab_stream_t stream);
 
+/* FP8 inference tier: the same launch with E4M3 operands (tcgen05.mma kind::f8f6f4, fp32 accumulation in TMEM).
+ *   Sources: act and wgt are E4M3 (1 byte per element); C_in a multiple of 128; ld_ch, w_ld_ch multiples of 16.
+ *   Each source j carries activation scale s_j folded into its weights by the caller:
+ *   wgt_j = e4m3(W_j * s_j / alpha[n]), alpha[n] = max_j(s_j * max|W_j[n, :]|) / 448, so that
+ *   acc[t, n] * alpha[n] = sum_j s_j * x_q_j . W_j  (x_q_j: the stored E4M3 activation).
+ *   alpha: fp32 [C_out], applied to the accumulator before the bias in every epilogue.
+ *   CAB_EPI_ACT_BF16 here stores E4M3: out_hi = e4m3(act(acc * alpha + bias) * mask * out_scale_inv), saturating to
+ *   +-448 (cvt.rn.satfinite), out_ld_ch a multiple of 16.  LOGSOFTMAX / LOGITS_F32 / LOGITS_ROWS write fp32 as above.
+ *   Not available here: out_lo, stats, skip_frac, the folded BatchNorm-backward reduction. */
+int cab_conv1d_fused_fp8(const cab_conv_source_t* sources_host, int n_sources,
+                         const cab_conv_epilogue_t* epilogue_host, const float* alpha, float out_scale_inv,
+                         cab_stream_t stream);
+/* calibration of the FP8 tier: out[0] = max |x| over n bf16 elements (n < 2^31) */
+int cab_absmax_bf16(const void* x, int64_t n, float* out, cab_stream_t stream);
+/* out = e4m3(x * scale_inv) elementwise, saturating to +-448 (cvt.rn.satfinite); x bf16, n a multiple of 16, both 16-byte aligned */
+int cab_quantize_e4m3(const void* x, int64_t n, float scale_inv, void* out, cab_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------
  * Training: Conv1d weight gradient (autograd's wgrad behind loss.backward(), train.py:770-774)
  *   out[tap][m][n] = sum_{b,t} a[b, t, m] * bx[b, t + tap*dilation - pad_left, n]
@@ -328,6 +345,11 @@ int cab_grouped_conv1d(const void* act, const void* act_lo, int B, int T, int T_
                        int ld_in, const float* wgt, const float* bias, int C_out, int groups,
                        int k, int pad_left, void* out, void* out_lo, int out_T_rows, int ld_out, int relu,
                        cab_stream_t stream);
+/* FP8 inference tier: the same grouped conv + bias + ReLU with E4M3 input (x = q * in_scale, ld_in a multiple of 16) and
+ * E4M3 output e4m3(v * out_scale_inv), saturating; odd k in 3..27 with the input window of 64 outputs at most 208 channels. */
+int cab_grouped_conv1d_fp8(const void* act, int B, int T, int T_rows, int C_in, int ld_in, float in_scale,
+                           const float* wgt, const float* bias, int C_out, int groups, int k, int pad_left,
+                           void* out, int out_T_rows, int ld_out, float out_scale_inv, cab_stream_t stream);
 /* training: weight / bias gradient of that grouped conv (autograd's grouped wgrad behind loss.backward(),
  * train.py:770-774):  dw[co, j, k] = sum_{b,t} dy[b,t,co] * x[b, t + k - pad, g(co)*cin_g + j]  (fp32 [C_out, C_in/groups, k],
  * zeroed by the call), db[co] = sum_{b,t} dy[b,t,co] (fp32 [C_out] or NULL).  Odd k with pad = k / 2. */
