@@ -124,8 +124,12 @@ SIGNATURES = {
 							c_void_p, c_int, c_void_p, c_void_p],
 	'cab_top2_probs': [c_void_p, c_i64, c_i64, c_i64, c_int, c_int, c_int, c_void_p, c_void_p],
 	'cab_entropy': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+	'cab_ctc_beam_search_workspace': [c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, ctypes.POINTER(c_i64)],
+	'cab_ctc_beam_search': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, c_void_p, c_i64,
+							c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
 }
-HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace', 'cab_ctc_loss_one_cta_covers', 'cab_ctc_loss_long_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
+HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace', 'cab_ctc_loss_one_cta_covers', 'cab_ctc_loss_long_workspace',
+			'cab_ctc_beam_search_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
 INTROSPECTION = {'cab_abi_version': c_int, 'cab_last_error': ctypes.c_char_p, 'cab_launch_count': c_i64}
 
 

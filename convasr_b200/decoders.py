@@ -1,10 +1,13 @@
-"""Drop-in replacement for the reference's `decoders` module (decoders.py:5-16).
+"""Drop-in replacement for the reference's `decoders` module (decoders.py:5-55).
 
 GreedyDecoder: per-frame top-K class ids truncated to the output length -- NO blank/repeat
 collapse (that lives in transcript_generators.GreedyCTCGenerator).  K=1 is the fused argmax
 (ties -> lowest id, as torch.argmax); K>1 is the native top-K kernel (K <= 8).
-BeamSearchDecoder wraps the external ctcdecode C++ library and is out of scope (SURVEY.md 2.1).
+BeamSearchDecoder: CTC prefix beam search on the GPU (csrc/beam.cu) without a language model;
+LM decoding (ctcdecode + KenLM) is not built.
 """
+import math
+
 import torch
 
 from . import ops
@@ -25,5 +28,49 @@ class GreedyDecoder:
 
 
 class BeamSearchDecoder:
-	def __init__(self, *args, **kwargs):
-		raise NotImplementedError('convasr_b200: BeamSearchDecoder (external ctcdecode + KenLM) is outside the hot path; use GreedyDecoder')
+	"""CTC prefix beam search over [B, C, T] log_probs, argument names as ctcdecode's CTCBeamDecoder.
+
+	Acoustic scores only: `lm_path`, or a nonzero `beam_alpha` / `beam_beta`, raises NotImplementedError (KenLM
+	decoding is not built).  Each frame keeps its `cutoff_top_n` most probable classes and, with `cutoff_prob` < 1,
+	only those (most probable first) until their probability sums to `cutoff_prob`; `beam_width` (at most 128)
+	prefixes survive each frame, ranked by log(p_blank + p_nonblank).  `blank_id` None means the last class (C - 1),
+	the model's convention.  `num_workers` is accepted for compatibility; the search runs on the GPU.
+
+	`topk` means the k most probable hypotheses, best first.  Whether the reference's `decoded_scores.topk(...)` line
+	selects the same ones depends on the sign of ctcdecode's scores and cannot be checked here."""
+
+	def __init__(self, labels, lm_path = None, beam_width = 100, beam_alpha = 0, beam_beta = 0, cutoff_top_n = 40, cutoff_prob = 1.0,
+				num_workers = 1, topk = 1, blank_id = None):
+		if lm_path is not None or beam_alpha != 0 or beam_beta != 0:
+			raise NotImplementedError('convasr_b200: BeamSearchDecoder with a language model (ctcdecode + KenLM: lm_path, beam_alpha, beam_beta) is not built; '
+									'the acoustic beam search runs with lm_path=None and beam_alpha = beam_beta = 0')
+		if not 1 <= int(beam_width) <= ops.BEAM_MAX_WIDTH:
+			raise ValueError(f'convasr_b200: beam_width={beam_width} out of [1, {ops.BEAM_MAX_WIDTH}]')
+		if not 1 <= int(topk) <= int(beam_width):
+			raise ValueError(f'convasr_b200: topk={topk} out of [1, beam_width={beam_width}]')
+		if int(cutoff_top_n) < 1:
+			raise ValueError(f'convasr_b200: cutoff_top_n={cutoff_top_n} must be positive')
+		if not 0.0 < float(cutoff_prob) <= 1.0:
+			raise ValueError(f'convasr_b200: cutoff_prob={cutoff_prob} out of (0, 1]')
+		self.labels = labels
+		self.beam_width, self.cutoff_top_n, self.cutoff_prob = int(beam_width), int(cutoff_top_n), float(cutoff_prob)
+		self.num_workers, self.topk, self.blank_id = num_workers, int(topk), blank_id
+
+	def decode_nbest(self, log_probs, output_lengths = None):
+		"""Device tensors for rescoring and timestamps: dict(tokens int32 [B, topk, T], frames int32 [B, topk, T] (the frame
+		at which each token was emitted), lengths int32 [B, topk], scores fp32 [B, topk] = log(p_blank + p_nonblank)).
+		Tokens and frames are -1 past each length; a hypothesis the search did not keep has score -inf and length 0."""
+		tokens, frames, lengths, scores = ops.ctc_beam_search(
+			log_probs, output_lengths, beam_width = self.beam_width, cutoff_top_n = self.cutoff_top_n, cutoff_prob = self.cutoff_prob,
+			topk = self.topk, blank = self.blank_id
+		)
+		return dict(tokens = tokens, frames = frames, lengths = lengths, scores = scores)
+
+	def decode(self, log_probs, output_lengths = None):
+		"""topk = 1: one token list per utterance; topk > 1: per utterance, up to topk token lists, best first."""
+		r = self.decode_nbest(log_probs, output_lengths)
+		lengths, scores = r['lengths'].cpu().tolist(), r['scores'].cpu().tolist()
+		n_max = max([max(l) for l in lengths], default = 0)
+		tokens = r['tokens'][:, :, :n_max].cpu().tolist()
+		out = [[tok[:l] for tok, l, s in zip(tb, lb, sb) if s > -math.inf] for tb, lb, sb in zip(tokens, lengths, scores)]
+		return [o[0] if o else [] for o in out] if self.topk == 1 else out

@@ -416,6 +416,48 @@ def top2_probs(log_probs):
 	return out
 
 
+BEAM_MAX_WIDTH = 128  # beams per utterance the search kernel holds in shared memory
+BEAM_MAX_CLASSES = 64  # classes per frame after pruning (min(cutoff_top_n, C))
+
+
+def ctc_beam_search(log_probs, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0, topk = 1, blank = None):
+	"""CTC prefix beam search without a language model on fp32 [B, C, T] log_probs (any strides, e.g. the class-contiguous
+	views of the large-vocabulary head).  blank None: C - 1.  Returns device tensors (tokens int32 [B, topk, T], frames int32
+	[B, topk, T], lengths int32 [B, topk], scores fp32 [B, topk]): the topk most probable hypotheses best first, the frame at
+	which each token was emitted, and log(p_blank + p_nonblank) at the last frame (-inf, length 0 where the search kept fewer
+	than topk hypotheses).  Tokens and frames are -1 past each hypothesis' length."""
+	_need_cuda(log_probs)
+	lp = log_probs if log_probs.dtype == torch.float32 else log_probs.float()
+	B, C, T = lp.shape
+	blank = C - 1 if blank is None else int(blank)
+	N = min(int(cutoff_top_n), C)
+	W, K = int(beam_width), int(topk)
+	dev = lp.device
+	if output_lengths is None:
+		olen = torch.full((B, ), T, dtype = torch.int64, device = dev)
+	else:
+		olen = torch.as_tensor(output_lengths, device = dev).to(torch.int64).contiguous()
+	if B == 0 or T == 0:  # nothing to search: the empty hypothesis, probability one
+		tokens = torch.full((B, K, T), -1, dtype = torch.int32, device = dev)
+		scores = torch.full((B, K), -math.inf, dtype = torch.float32, device = dev)
+		scores[:, 0] = 0.0
+		return tokens, tokens.clone(), torch.zeros(B, K, dtype = torch.int32, device = dev), scores
+	lib = _lib.load()
+	nbytes = ctypes.c_int64()
+	_lib.check(lib.cab_ctc_beam_search_workspace(B, T, C, N, W, K, blank, float(cutoff_prob), ctypes.byref(nbytes)), 'cab_ctc_beam_search_workspace')
+	ws = torch.empty(nbytes.value, dtype = torch.uint8, device = dev)
+	tokens = torch.empty(B, K, T, dtype = torch.int32, device = dev)
+	frames = torch.empty_like(tokens)
+	lengths = torch.empty(B, K, dtype = torch.int32, device = dev)
+	scores = torch.empty(B, K, dtype = torch.float32, device = dev)
+	rc = lib.cab_ctc_beam_search(
+		_p(lp), lp.stride(0), lp.stride(1), lp.stride(2), _p(olen), B, T, C, N, float(cutoff_prob), blank, W, K, _p(ws), nbytes.value,
+		_p(tokens), _p(frames), T, _p(lengths), _p(scores), _stream()
+	)
+	_lib.check(rc, 'cab_ctc_beam_search')
+	return tokens, frames, lengths, scores
+
+
 def entropy(log_probs, lengths = None, eps_id = -1):
 	_need_cuda(log_probs, lengths)
 	log_probs = log_probs.to(torch.float32).contiguous()

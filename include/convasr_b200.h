@@ -496,6 +496,32 @@ int cab_top2_probs(const float* log_probs, int64_t stride_b, int64_t stride_c, i
 int cab_entropy(const float* log_probs, const int64_t* lengths, int B, int C, int T, int eps_id,
                 float* out_entropy, float* out_weighted_entropy, cab_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------
+ * CTC prefix beam search without a language model (decoders.BeamSearchDecoder; the acoustic
+ *   part of ctcdecode's CTCBeamDecoder, alpha = beta = 0).  fp32 log domain, full-precision
+ *   expf / logf: the result of an utterance does not depend on the batch it is in.
+ *   log_probs [B, C, T] through element strides; output_lengths int64 [B] (frames searched,
+ *   clamped to [0, T]).  Per frame the top N = min(cutoff_top_n, C) classes are kept (ties ->
+ *   lower class id), then, with cutoff_prob < 1, only those (by descending probability) until
+ *   the fp32 running sum of probabilities reaches cutoff_prob, the class that crosses it
+ *   included.  W beams per utterance; candidates are ranked by log(p_blank + p_nonblank), ties
+ *   to the lower (source beam rank, class id); probability zero is never a candidate.
+ *   out_tokens / out_frames: int32 [B, K, L_cap], the K best hypotheses best first, with the
+ *   frame at which each token's prefix was created; -1 past the hypothesis' length.
+ *   out_lengths: int32 [B, K]; out_scores: fp32 [B, K] = log(p_blank + p_nonblank) at the last
+ *   frame, -inf (length 0) where fewer than K hypotheses have nonzero probability.
+ *   Refused before any launch: W outside [1, 128], N outside [1, 64] or above C, K outside
+ *   [1, W], blank outside [0, C), cutoff_prob outside (0, 1], a workspace smaller than
+ *   cab_ctc_beam_search_workspace reports (host only, no device work).  Three launches.
+ * ------------------------------------------------------------------------------------- */
+int cab_ctc_beam_search_workspace(int B, int T, int C, int N, int W, int K, int blank, float cutoff_prob,
+                                  int64_t* bytes);
+int cab_ctc_beam_search(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                        const int64_t* output_lengths, int B, int T, int C, int N, float cutoff_prob,
+                        int blank, int W, int K, void* workspace, int64_t workspace_bytes,
+                        int32_t* out_tokens, int32_t* out_frames, int L_cap, int32_t* out_lengths,
+                        float* out_scores, cab_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
