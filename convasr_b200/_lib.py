@@ -49,6 +49,14 @@ class BnBranch(ctypes.Structure):
 	_fields_ = [('y', c_void_p), ('y_lo', c_void_p), ('ss', c_void_p)]
 
 
+NGRAM_MAX_ORDER = 6  # CAB_NGRAM_MAX_ORDER
+
+
+class NgramLM(ctypes.Structure):  # cab_ngram_lm_t
+	_fields_ = [('order', c_i32), ('num_classes', c_i32), ('num_nodes', c_i32), ('bos', c_i32), ('tables', c_void_p * NGRAM_MAX_ORDER),
+				('sizes', c_i64 * NGRAM_MAX_ORDER), ('child', c_void_p), ('word', c_void_p)]
+
+
 ACT_NONE, ACT_RELU, ACT_HARDTANH, ACT_LEAKY_RELU = 0, 1, 2, 3
 EPI_ACT_BF16, EPI_LOGSOFTMAX, EPI_LOGITS_F32, EPI_LOGITS_ROWS = 0, 1, 2, 3
 MAX_CONV_SOURCES = 18
@@ -127,6 +135,8 @@ SIGNATURES = {
 	'cab_ctc_beam_search_workspace': [c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_float, ctypes.POINTER(c_i64)],
 	'cab_ctc_beam_search': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, c_void_p, c_i64,
 							c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
+	'cab_ctc_beam_search_lm': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, c_void_p, c_i64,
+								c_void_p, c_void_p, c_int, c_void_p, c_void_p, ctypes.POINTER(NgramLM), c_float, c_float, c_int, c_void_p],
 }
 HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace', 'cab_ctc_loss_one_cta_covers', 'cab_ctc_loss_long_workspace',
 			'cab_ctc_beam_search_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)

@@ -1,18 +1,22 @@
-// CTC prefix beam search without a language model (decoders.BeamSearchDecoder, the acoustic part of ctcdecode's
-// CTCBeamDecoder: lm_path = None, alpha = beta = 0).
+// CTC prefix beam search (decoders.BeamSearchDecoder, ctcdecode's CTCBeamDecoder), acoustic only or with a word n-gram
+// language model fused in (ctcdecode's word-level scorer rules, tables built by convasr_b200/lm.py).
 //
 // Three launches per call:
 //   beam_prune_kernel      one warp per frame: the top N = min(cutoff_top_n, C) classes by log-prob (ties -> lower class
 //                          id), cut further by cutoff_prob as ctcdecode does, written in ascending class order.
 //   beam_search_kernel     one CTA per utterance, T sequential frames: W <= 128 beams in shared memory, candidates scored,
 //                          extensions merged into existing beams, the top W selected by a block-wide radix select, and
-//                          one node (parent, class) allocated per surviving new prefix in a [T, W] table.
+//                          one node (parent, class) allocated per surviving new prefix in a [T, W] table.  The LM
+//                          instance also holds each beam's trie node and word context, refuses extensions that leave
+//                          the dictionary, adds the word score when a space completes a word, and adds the last word's
+//                          score and re-ranks after the last frame.
 //   beam_backtrace_kernel  one thread per hypothesis walks the parent chain into tokens and emission frames.
 //
 // Log domain in fp32 with full-precision expf / logf, so the result is deterministic and does not depend on the batch.
 #include "common.cuh"
 #include "../../include/convasr_b200.h"
 #include <atomic>
+#include <cmath>
 
 namespace cab {
 extern std::atomic<int64_t> g_launch_count;
@@ -194,10 +198,90 @@ struct BeamNode {
     int cls;
 };
 
+// ------------------------------------------------------------------------------------------
+// Word n-gram LM (the LM instance).  A beam also holds the trie node of its current word, the last order - 1 completed
+// words (oldest first, <s>-padded) and the bonus that the extension creating its prefix carried (nonzero only when that
+// extension was a space; step (1)'s merge into the beam adds it again).  Per frame, before step (2):
+//  (a) when `space` is among the frame's classes and the beam's node spells a word w, the space bonus
+//      alpha * lm(w | context) + beta; otherwise a space is not a candidate of that beam;
+//  (b) a non-space class c is a candidate only if child[node][c] >= 0.
+// A new prefix takes node' = child[node][c], or after a space the root and the context shifted by w.
+// ------------------------------------------------------------------------------------------
+constexpr int kLmMaxOrder = CAB_NGRAM_MAX_ORDER;
+constexpr float kLmOovScore = -1000.f;  // ctcdecode's OOV_SCORE (natural log, before alpha)
+
+struct NgramEntry {
+    uint64_t key;  // 0 = empty slot
+    float log10_p;
+    float log10_bo;
+};
+
+struct BeamLm {
+    const NgramEntry* table[kLmMaxOrder];
+    uint64_t mask[kLmMaxOrder];
+    const int* child;
+    const int* word;
+    int order, C, space, bos;
+    float alpha, beta;
+};
+
+// linear probing from the first probe e (slot key & mask) until the key or an empty slot; at most one pass over the
+// table, so a table without an empty slot ends the search as "not listed" instead of spinning
+__device__ __forceinline__ NgramEntry ngram_probe(const NgramEntry* table, uint64_t mask, uint64_t key, NgramEntry e) {
+    uint64_t slot = key & mask;
+    for (uint64_t i = 0; i < mask && e.key != key && e.key != 0; ++i) {
+        slot = (slot + 1) & mask;
+        e = table[slot];
+    }
+    return e;
+}
+
+// lm(w | ctx) in natural log: ARPA back-off over the order tables.  Every first probe (n for log10 p of the suffixes
+// (ctx[n-k..], w), n - 1 for the back-offs of the context suffixes) is issued before any is used; keys are folded
+// newest first, so each suffix's key extends the next shorter one's.
+__device__ float lm_word_score(const BeamLm& lm, const int* ctx, int w) {
+    const int n = lm.order;
+    uint64_t pk[kLmMaxOrder], bk[kLmMaxOrder];
+    NgramEntry pe[kLmMaxOrder], be[kLmMaxOrder];
+    pk[0] = beam_hash(0, w);
+    bk[0] = 0;
+#pragma unroll
+    for (int k = 1; k < kLmMaxOrder; ++k) {
+        if (k < n) {
+            const int id = ctx[n - 1 - k];
+            pk[k] = beam_hash(pk[k - 1], id);
+            bk[k] = beam_hash(bk[k - 1], id);
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < kLmMaxOrder; ++k) {
+        if (k < n) pe[k] = lm.table[k][pk[k] & lm.mask[k]];
+        if (k >= 1 && k < n) be[k] = lm.table[k - 1][bk[k] & lm.mask[k - 1]];
+    }
+    float p = 0.f, bo = 0.f;
+    bool found = false;
+#pragma unroll
+    for (int k = kLmMaxOrder - 1; k >= 0; --k) {
+        if (k < n && !found) {
+            // (ctx[n-1-k..], w) at order k + 1; back-off of the context suffix of length k (order k)
+            const NgramEntry e = ngram_probe(lm.table[k], lm.mask[k], pk[k], pe[k]);
+            if (e.key == pk[k]) {
+                p = e.log10_p;
+                found = true;
+            } else if (k >= 1) {
+                const NgramEntry c = ngram_probe(lm.table[k - 1], lm.mask[k - 1], bk[k], be[k]);
+                if (c.key == bk[k]) bo += c.log10_bo;
+            }
+        }
+    }
+    return found ? 2.302585093f * (bo + p) : kLmOovScore;
+}
+
+template <bool LM>
 __global__ void __launch_bounds__(kBeamThreads, 1)
 beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp, const int* __restrict__ p_cnt,
                    const int64_t* __restrict__ lengths, int T, int N, int blank, int W, int K,
-                   BeamNode* __restrict__ nodes, int* __restrict__ final_node, float* __restrict__ out_scores) {
+                   BeamNode* __restrict__ nodes, int* __restrict__ final_node, float* __restrict__ out_scores, const BeamLm lm) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int b = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -226,11 +310,23 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
     int& s_nsel = s_misc[kWarps + 1];
     int& s_prefix = s_misc[kWarps + 2];
     int& s_need = s_misc[kWarps + 3];
+    // LM instance only, after the acoustic layout
+    constexpr int kCtx = kLmMaxOrder - 1;
+    int* s_tnode = reinterpret_cast<int*>(s_keys + W * (N + 1));  // [2][W] trie node of the current word
+    int* s_ctx = s_tnode + 2 * W;                                   // [2][W][kCtx] completed words, oldest first
+    float* s_bonus = reinterpret_cast<float*>(s_ctx + 2 * W * kCtx);  // [2][W] bonus of the extension that made the prefix
+    float* s_spb = s_bonus + 2 * W;                                  // [W] this frame's space bonus, -inf = no space
+    int* s_word = reinterpret_cast<int*>(s_spb + W);                // [W] word id of the beam's node, or -1
 
     const int64_t len64 = lengths ? lengths[b] : T;
     const int len = len64 < 0 ? 0 : (len64 > T ? T : (int)len64);
     if (tid == 0) {
         s_hash[0] = 0; s_phash[0] = 0; s_pb[0] = 0.f; s_pnb[0] = -INFINITY; s_last[0] = -1; s_node[0] = -1; s_prank[0] = -1;
+        if constexpr (LM) {
+            s_tnode[0] = 0;
+            s_bonus[0] = 0.f;
+            for (int k = 0; k < kCtx; ++k) s_ctx[k] = lm.bos;
+        }
     }
     int cur = 0, nb = 1;
     const size_t frame0 = (size_t)b * T;
@@ -271,11 +367,23 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
             float x = kl >= 0 ? pnb[j] + s_flp[kl] : -INFINITY;
             const int p = s_prank[cur * W + j];
             if (p >= 0 && kl >= 0) {
-                const float e = (last[p] == lj ? pb[p] : beam_lse(pb[p], pnb[p])) + s_flp[kl];
+                float e = (last[p] == lj ? pb[p] : beam_lse(pb[p], pnb[p])) + s_flp[kl];
+                if constexpr (LM) e += s_bonus[cur * W + j];
                 x = beam_lse(x, e);
                 s_merged[p * N + kl] = (int16_t)j;
             }
             s_kpnb[j] = x;
+        }
+        if constexpr (LM) {
+            // (a) the space bonus, by the threads step (1) leaves idle
+            const int j = tid - kBeamMaxW;
+            if (j >= 0 && j < nb) {
+                bool has_space = false;
+                for (int k = 0; k < n; ++k) has_space |= s_fcls[k] == lm.space;
+                const int w = lm.word[s_tnode[cur * W + j]];
+                s_word[j] = w;
+                s_spb[j] = has_space && w >= 0 ? lm.alpha * lm_word_score(lm, s_ctx + (cur * W + j) * kCtx, w) + lm.beta : -INFINITY;
+            }
         }
         __syncthreads();
         // (2) candidate keys; the first radix pass's histogram on the way
@@ -290,6 +398,11 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
                 const int k = s - 1, c = s_fcls[k];
                 if (c == blank || s_merged[i * N + k] >= 0) v = -INFINITY;
                 else v = (c == last[i] ? pb[i] : beam_lse(pb[i], pnb[i])) + s_flp[k];
+                if constexpr (LM) {
+                    // (b) the dictionary constraint; a space carries the word's bonus (-inf: no word to end)
+                    if (c == lm.space) v += s_spb[i];
+                    else if (c != blank && lm.child[(size_t)s_tnode[cur * W + i] * lm.C + c] < 0) v = -INFINITY;
+                }
             }
             const uint32_t key = beam_ckey(v);
             s_keys[q] = key;
@@ -395,10 +508,32 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
                 s_hash[nxt * W + r] = s_hash[cur * W + i];
                 s_phash[nxt * W + r] = s_phash[cur * W + i];
                 s_newrank[i] = r;
+                if constexpr (LM) {
+                    s_tnode[nxt * W + r] = s_tnode[cur * W + i];
+                    s_bonus[nxt * W + r] = s_bonus[cur * W + i];
+                    for (int k = 0; k < lm.order - 1; ++k) s_ctx[(nxt * W + r) * kCtx + k] = s_ctx[(cur * W + i) * kCtx + k];
+                }
             } else {
                 const int k = s - 1, c = s_fcls[k];
                 s_pb[nxt * W + r] = -INFINITY;
-                s_pnb[nxt * W + r] = (c == last[i] ? pb[i] : beam_lse(pb[i], pnb[i])) + s_flp[k];
+                float v = (c == last[i] ? pb[i] : beam_lse(pb[i], pnb[i])) + s_flp[k];
+                if constexpr (LM) {
+                    const int* ctx = s_ctx + (cur * W + i) * kCtx;
+                    int* nctx = s_ctx + (nxt * W + r) * kCtx;
+                    const int nc = lm.order - 1;
+                    if (c == lm.space) {
+                        v += s_spb[i];
+                        s_tnode[nxt * W + r] = 0;
+                        s_bonus[nxt * W + r] = s_spb[i];
+                        for (int m = 0; m + 1 < nc; ++m) nctx[m] = ctx[m + 1];
+                        if (nc > 0) nctx[nc - 1] = s_word[i];
+                    } else {
+                        s_tnode[nxt * W + r] = lm.child[(size_t)s_tnode[cur * W + i] * lm.C + c];
+                        s_bonus[nxt * W + r] = 0.f;
+                        for (int m = 0; m < nc; ++m) nctx[m] = ctx[m];
+                    }
+                }
+                s_pnb[nxt * W + r] = v;
                 s_last[nxt * W + r] = c;
                 const int id = t * W + r;
                 s_node[nxt * W + r] = id;
@@ -429,6 +564,34 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
         cur = nxt;
         __syncthreads();
         if (nb == 0) break;
+    }
+    if constexpr (LM) {
+        // the last word's term, then re-rank by counting (ties to the earlier rank); hypothesis r is beam s_order[r]
+        float* s_fin = s_kpb;
+        if (tid < nb) {
+            const int l = s_last[cur * W + tid];
+            float f = beam_lse(s_pb[cur * W + tid], s_pnb[cur * W + tid]);
+            if (l >= 0 && l != lm.space) {
+                const int w = lm.word[s_tnode[cur * W + tid]];
+                f += lm.alpha * (w >= 0 ? lm_word_score(lm, s_ctx + (cur * W + tid) * kCtx, w) : kLmOovScore) + lm.beta;
+            }
+            s_fin[tid] = f;
+        }
+        __syncthreads();
+        if (tid < nb) {
+            const float f = s_fin[tid];
+            int rank = 0;
+            for (int g = 0; g < nb; ++g) rank += s_fin[g] > f || (s_fin[g] == f && g < tid);
+            s_order[rank] = tid;
+        }
+        __syncthreads();
+        if (tid < K) {
+            const size_t o = (size_t)b * K + tid;
+            const int r = tid < nb ? s_order[tid] : -1;
+            final_node[o] = r >= 0 ? s_node[cur * W + r] : -2;
+            out_scores[o] = r >= 0 ? s_fin[r] : -INFINITY;
+        }
+        return;
     }
     // beams are in rank order: hypothesis r is beam r
     if (tid < K) {
@@ -482,10 +645,48 @@ static size_t beam_workspace_bytes(int B, int T, int N, int W) {
     return beam_align(off[4] + (size_t)B * W * 4);
 }
 
-static size_t beam_search_smem(int W, int N) {
+static size_t beam_search_smem(int W, int N, bool lm) {
     size_t bytes = 2 * W * 8 * 2 + 2 * W * 4 * 5 + W * 4 * 6 + N * 8 + 256 * 4 + (kBeamThreads / 32 + 8) * 4;
     bytes += (size_t)((W * N + 1) & ~1) * 2 + (size_t)W * (N + 1) * 4;
+    if (lm) bytes += (size_t)W * 4 * (2 + 2 * (kLmMaxOrder - 1) + 2 + 2);  // trie node, context, bonus; space bonus, word
     return bytes;
+}
+
+// prune -> search -> back-trace; the arguments are checked by the caller
+template <bool LM>
+static int beam_search_launch(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t, const int64_t* output_lengths,
+                              int B, int T, int C, int N, float cutoff_prob, int blank, int W, int K, void* workspace, int32_t* out_tokens,
+                              int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores, const BeamLm& lm,
+                              cudaStream_t stream) {
+    size_t off[5];
+    beam_workspace_layout(B, T, N, W, off);
+    unsigned char* ws = static_cast<unsigned char*>(workspace);
+    int* p_cls = reinterpret_cast<int*>(ws + off[0]);
+    float* p_lp = reinterpret_cast<float*>(ws + off[1]);
+    int* p_cnt = reinterpret_cast<int*>(ws + off[2]);
+    BeamNode* nodes = reinterpret_cast<BeamNode*>(ws + off[3]);
+    int* final_node = reinterpret_cast<int*>(ws + off[4]);
+
+    const size_t smem = beam_search_smem(W, N, LM);
+    static size_t smem_set = 0;
+    if (smem > 48 * 1024 && smem > smem_set) {
+        CAB_CHECK_CUDA(cudaFuncSetAttribute(beam_search_kernel<LM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                            (int)beam_search_smem(kBeamMaxW, kBeamMaxN, LM)));
+        smem_set = beam_search_smem(kBeamMaxW, kBeamMaxN, LM);
+    }
+    dim3 pgrid((T + kPruneWarps - 1) / kPruneWarps, B);
+    beam_prune_kernel<<<pgrid, kPruneWarps * 32, 0, stream>>>(log_probs, stride_b, stride_c, stride_t, C, T, N, cutoff_prob, p_cls,
+                                                               p_lp, p_cnt);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    beam_search_kernel<LM><<<B, kBeamThreads, smem, stream>>>(p_cls, p_lp, p_cnt, output_lengths, T, N, blank, W, K, nodes, final_node,
+                                                              out_scores, lm);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    beam_backtrace_kernel<<<B, kBeamMaxW, 0, stream>>>(nodes, final_node, T, W, K, L_cap, out_tokens, out_frames, out_lengths);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
 }
 
 }  // namespace cab
@@ -500,6 +701,13 @@ using namespace cab;
     CAB_CHECK_ARG(blank >= 0 && blank < C, "blank=%d out of range (C=%d)", blank, C);                                  \
     CAB_CHECK_ARG(cutoff_prob > 0.f && cutoff_prob <= 1.f, "cutoff_prob=%g out of (0, 1]", (double)cutoff_prob)
 
+#define CAB_BEAM_CHECK_CALL()                                                                                          \
+    CAB_CHECK_ARG(log_probs && workspace && out_tokens && out_frames && out_lengths && out_scores, "null pointer argument"); \
+    CAB_BEAM_CHECK_ARGS();                                                                                             \
+    CAB_CHECK_ARG(L_cap >= 1, "L_cap=%d must be positive", L_cap);                                                     \
+    CAB_CHECK_ARG(workspace_bytes >= (int64_t)beam_workspace_bytes(B, T, N, W), "workspace of %lld bytes is too small (%lld needed)", \
+                  (long long)workspace_bytes, (long long)beam_workspace_bytes(B, T, N, W))
+
 extern "C" int cab_ctc_beam_search_workspace(int B, int T, int C, int N, int W, int K, int blank, float cutoff_prob, int64_t* bytes) {
     CAB_CHECK_ARG(bytes != nullptr, "null output");
     CAB_BEAM_CHECK_ARGS();
@@ -512,39 +720,43 @@ extern "C" int cab_ctc_beam_search(const float* log_probs, int64_t stride_b, int
                                    int W, int K, void* workspace, int64_t workspace_bytes, int32_t* out_tokens,
                                    int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores,
                                    cab_stream_t stream_) {
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    CAB_CHECK_ARG(log_probs && workspace && out_tokens && out_frames && out_lengths && out_scores, "null pointer argument");
-    CAB_BEAM_CHECK_ARGS();
-    CAB_CHECK_ARG(L_cap >= 1, "L_cap=%d must be positive", L_cap);
-    CAB_CHECK_ARG(workspace_bytes >= (int64_t)beam_workspace_bytes(B, T, N, W), "workspace of %lld bytes is too small (%lld needed)",
-                  (long long)workspace_bytes, (long long)beam_workspace_bytes(B, T, N, W));
-    size_t off[5];
-    beam_workspace_layout(B, T, N, W, off);
-    unsigned char* ws = static_cast<unsigned char*>(workspace);
-    int* p_cls = reinterpret_cast<int*>(ws + off[0]);
-    float* p_lp = reinterpret_cast<float*>(ws + off[1]);
-    int* p_cnt = reinterpret_cast<int*>(ws + off[2]);
-    BeamNode* nodes = reinterpret_cast<BeamNode*>(ws + off[3]);
-    int* final_node = reinterpret_cast<int*>(ws + off[4]);
+    CAB_BEAM_CHECK_CALL();
+    return beam_search_launch<false>(log_probs, stride_b, stride_c, stride_t, output_lengths, B, T, C, N, cutoff_prob, blank, W, K,
+                                     workspace, out_tokens, out_frames, L_cap, out_lengths, out_scores, BeamLm{},
+                                     static_cast<cudaStream_t>(stream_));
+}
 
-    const size_t smem = beam_search_smem(W, N);
-    static size_t smem_set = 0;
-    if (smem > 48 * 1024 && smem > smem_set) {
-        CAB_CHECK_CUDA(cudaFuncSetAttribute(beam_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)beam_search_smem(kBeamMaxW, kBeamMaxN)));
-        smem_set = beam_search_smem(kBeamMaxW, kBeamMaxN);
+extern "C" int cab_ctc_beam_search_lm(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                                      const int64_t* output_lengths, int B, int T, int C, int N, float cutoff_prob, int blank,
+                                      int W, int K, void* workspace, int64_t workspace_bytes, int32_t* out_tokens,
+                                      int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores,
+                                      const cab_ngram_lm_t* lm, float alpha, float beta, int space, cab_stream_t stream_) {
+    CAB_BEAM_CHECK_CALL();
+    CAB_CHECK_ARG(lm != nullptr, "null lm");
+    CAB_CHECK_ARG(lm->order >= 1 && lm->order <= kLmMaxOrder, "lm order=%d out of [1, %d]", lm->order, kLmMaxOrder);
+    CAB_CHECK_ARG(lm->num_classes == C, "lm trie has %d classes, log_probs %d", lm->num_classes, C);
+    CAB_CHECK_ARG(lm->num_nodes >= 1 && lm->child && lm->word, "lm trie: %d nodes, child %p, word %p", lm->num_nodes,
+                  (const void*)lm->child, (const void*)lm->word);
+    CAB_CHECK_ARG(lm->bos >= 0, "lm bos=%d negative", lm->bos);
+    CAB_CHECK_ARG(space >= 0 && space < C && space != blank, "space=%d out of range (C=%d) or equal to blank=%d", space, C, blank);
+    CAB_CHECK_ARG(std::isfinite(alpha) && std::isfinite(beta), "alpha=%g / beta=%g not finite", (double)alpha, (double)beta);
+    BeamLm v{};
+    for (int k = 0; k < lm->order; ++k) {
+        const int64_t n = lm->sizes[k];
+        CAB_CHECK_ARG(lm->tables[k] != nullptr, "lm table of order %d is null", k + 1);
+        CAB_CHECK_ARG(n > 0 && (n & (n - 1)) == 0, "lm table of order %d: size %lld is not a power of two", k + 1, (long long)n);
+        v.table[k] = static_cast<const NgramEntry*>(lm->tables[k]);
+        v.mask[k] = (uint64_t)(n - 1);
     }
-    dim3 pgrid((T + kPruneWarps - 1) / kPruneWarps, B);
-    beam_prune_kernel<<<pgrid, kPruneWarps * 32, 0, stream>>>(log_probs, stride_b, stride_c, stride_t, C, T, N, cutoff_prob, p_cls,
-                                                               p_lp, p_cnt);
-    CAB_CHECK_LAUNCH();
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    beam_search_kernel<<<B, kBeamThreads, smem, stream>>>(p_cls, p_lp, p_cnt, output_lengths, T, N, blank, W, K, nodes, final_node,
-                                                          out_scores);
-    CAB_CHECK_LAUNCH();
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    beam_backtrace_kernel<<<B, kBeamMaxW, 0, stream>>>(nodes, final_node, T, W, K, L_cap, out_tokens, out_frames, out_lengths);
-    CAB_CHECK_LAUNCH();
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return 0;
+    v.child = lm->child;
+    v.word = lm->word;
+    v.order = lm->order;
+    v.C = C;
+    v.space = space;
+    v.bos = lm->bos;
+    v.alpha = alpha;
+    v.beta = beta;
+    return beam_search_launch<true>(log_probs, stride_b, stride_c, stride_t, output_lengths, B, T, C, N, cutoff_prob, blank, W, K,
+                                    workspace, out_tokens, out_frames, L_cap, out_lengths, out_scores, v,
+                                    static_cast<cudaStream_t>(stream_));
 }

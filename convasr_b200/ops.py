@@ -420,12 +420,17 @@ BEAM_MAX_WIDTH = 128  # beams per utterance the search kernel holds in shared me
 BEAM_MAX_CLASSES = 64  # classes per frame after pruning (min(cutoff_top_n, C))
 
 
-def ctc_beam_search(log_probs, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0, topk = 1, blank = None):
-	"""CTC prefix beam search without a language model on fp32 [B, C, T] log_probs (any strides, e.g. the class-contiguous
-	views of the large-vocabulary head).  blank None: C - 1.  Returns device tensors (tokens int32 [B, topk, T], frames int32
+def ctc_beam_search(log_probs, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0, topk = 1, blank = None, lm = None,
+					alpha = 0.0, beta = 0.0):
+	"""CTC prefix beam search on fp32 [B, C, T] log_probs (any strides, e.g. the class-contiguous views of the
+	large-vocabulary head).  blank None: C - 1.  Returns device tensors (tokens int32 [B, topk, T], frames int32
 	[B, topk, T], lengths int32 [B, topk], scores fp32 [B, topk]): the topk most probable hypotheses best first, the frame at
 	which each token was emitted, and log(p_blank + p_nonblank) at the last frame (-inf, length 0 where the search kept fewer
-	than topk hypotheses).  Tokens and frames are -1 past each hypothesis' length."""
+	than topk hypotheses).  Tokens and frames are -1 past each hypothesis' length.
+
+	lm: an lm.NGramLM built for these labels and this blank.  Then only prefixes spelling words of the LM's vocabulary are
+	searched, a space that ends word w adds alpha * ln P(w | previous words) + beta, the last word gets the same term
+	(alpha * -1000 + beta if it is incomplete) and the scores are these fused ones (csrc/beam.cu, cab_ctc_beam_search_lm)."""
 	_need_cuda(log_probs)
 	lp = log_probs if log_probs.dtype == torch.float32 else log_probs.float()
 	B, C, T = lp.shape
@@ -450,11 +455,21 @@ def ctc_beam_search(log_probs, output_lengths = None, beam_width = 100, cutoff_t
 	frames = torch.empty_like(tokens)
 	lengths = torch.empty(B, K, dtype = torch.int32, device = dev)
 	scores = torch.empty(B, K, dtype = torch.float32, device = dev)
-	rc = lib.cab_ctc_beam_search(
-		_p(lp), lp.stride(0), lp.stride(1), lp.stride(2), _p(olen), B, T, C, N, float(cutoff_prob), blank, W, K, _p(ws), nbytes.value,
-		_p(tokens), _p(frames), T, _p(lengths), _p(scores), _stream()
-	)
-	_lib.check(rc, 'cab_ctc_beam_search')
+	if lm is None:
+		rc = lib.cab_ctc_beam_search(
+			_p(lp), lp.stride(0), lp.stride(1), lp.stride(2), _p(olen), B, T, C, N, float(cutoff_prob), blank, W, K, _p(ws), nbytes.value,
+			_p(tokens), _p(frames), T, _p(lengths), _p(scores), _stream()
+		)
+		_lib.check(rc, 'cab_ctc_beam_search')
+	else:
+		if lm.blank != blank:
+			raise ValueError(f'convasr_b200: the LM was built with blank={lm.blank}, the search uses blank={blank}')
+		rc = lib.cab_ctc_beam_search_lm(
+			_p(lp), lp.stride(0), lp.stride(1), lp.stride(2), _p(olen), B, T, C, N, float(cutoff_prob), blank, W, K, _p(ws), nbytes.value,
+			_p(tokens), _p(frames), T, _p(lengths), _p(scores), ctypes.byref(lm.device_struct(dev)), float(alpha), float(beta), lm.space,
+			_stream()
+		)
+		_lib.check(rc, 'cab_ctc_beam_search_lm')
 	return tokens, frames, lengths, scores
 
 

@@ -522,6 +522,49 @@ int cab_ctc_beam_search(const float* log_probs, int64_t stride_b, int64_t stride
                         int32_t* out_tokens, int32_t* out_frames, int L_cap, int32_t* out_lengths,
                         float* out_scores, cab_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------
+ * The same search with a word n-gram language model fused in (shallow fusion, ctcdecode's
+ *   word-level scorer rules; convasr_b200/lm.py builds the tables from an ARPA file).
+ *   Labels are single characters; `space` is the label that ends a word.
+ *   N-gram tables: one per order k = 1..order, open addressing with linear probing, `sizes[k-1]`
+ *   entries (a power of two) of 16 bytes {uint64 key, float log10 p, float log10 back-off};
+ *   key 0 marks an empty slot.  The key of the word-id sequence (w1 .. wk) folds the ids
+ *   newest first: h = 0; for id = wk .. w1: h = splitmix64(h + 0x9E3779B97F4A7C15 * (id + 1));
+ *   the slot probed first is key & (size - 1).  Each table needs at least one empty slot, or a
+ *   key it does not hold is only found absent after a full pass (lm.py builds at load <= 1/2).
+ *   Dictionary trie over label ids: child int32 [num_nodes, num_classes] (-1 = no child), node 0
+ *   the root; word int32 [num_nodes], the word id a node spells or -1.
+ *   A prefix is admissible when every run of labels a space follows is a word, the last run
+ *   is a prefix of a word, and no space is first or follows a space; other extensions are not
+ *   candidates.  Extending a beam whose current word w is complete by `space` adds
+ *   alpha * ln(10) * log10 P(w | last order-1 words, <s>-padded) + beta to the extension (and
+ *   to a merge into a beam holding that prefix).  After the last frame each non-empty beam
+ *   not ending in a space gets the same term for its last word (-1000 before alpha if that
+ *   word is incomplete), and the beams are re-ranked by it (ties to the earlier rank);
+ *   out_scores are these fused scores.  Uses cab_ctc_beam_search_workspace's workspace.
+ *   Refused before any launch, besides the checks above: a null lm or table, order outside
+ *   [1, 6], a table size that is not a power of two, num_classes != C, space outside [0, C)
+ *   or equal to blank, num_nodes < 1, a negative bos, non-finite alpha or beta.  Three launches.
+ * ------------------------------------------------------------------------------------- */
+#define CAB_NGRAM_MAX_ORDER 6
+typedef struct {
+    int32_t order;         /* n, 1..CAB_NGRAM_MAX_ORDER */
+    int32_t num_classes;   /* C of the trie */
+    int32_t num_nodes;
+    int32_t bos;           /* word id of <s> */
+    const void* tables[CAB_NGRAM_MAX_ORDER];  /* order k at [k - 1] */
+    int64_t sizes[CAB_NGRAM_MAX_ORDER];
+    const int32_t* child;  /* [num_nodes, num_classes] */
+    const int32_t* word;   /* [num_nodes] */
+} cab_ngram_lm_t;
+
+int cab_ctc_beam_search_lm(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                           const int64_t* output_lengths, int B, int T, int C, int N, float cutoff_prob,
+                           int blank, int W, int K, void* workspace, int64_t workspace_bytes,
+                           int32_t* out_tokens, int32_t* out_frames, int L_cap, int32_t* out_lengths,
+                           float* out_scores, const cab_ngram_lm_t* lm, float alpha, float beta, int space,
+                           cab_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
