@@ -57,6 +57,11 @@ class NgramLM(ctypes.Structure):  # cab_ngram_lm_t
 				('sizes', c_i64 * NGRAM_MAX_ORDER), ('child', c_void_p), ('word', c_void_p)]
 
 
+class BeamStreamRow(ctypes.Structure):  # cab_beam_stream_t
+	_fields_ = [('state', c_void_p), ('nodes', c_void_p), ('state_bytes', c_i64), ('capacity', c_i64), ('t0', c_i64), ('frames', c_i32),
+				('is_eos', c_i32), ('finished', c_i32), ('reserved', c_i32)]
+
+
 ACT_NONE, ACT_RELU, ACT_HARDTANH, ACT_LEAKY_RELU = 0, 1, 2, 3
 EPI_ACT_BF16, EPI_LOGSOFTMAX, EPI_LOGITS_F32, EPI_LOGITS_ROWS = 0, 1, 2, 3
 MAX_CONV_SOURCES = 18
@@ -137,9 +142,14 @@ SIGNATURES = {
 							c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
 	'cab_ctc_beam_search_lm': [c_void_p, c_i64, c_i64, c_i64, c_void_p, c_int, c_int, c_int, c_int, c_float, c_int, c_int, c_int, c_void_p, c_i64,
 								c_void_p, c_void_p, c_int, c_void_p, c_void_p, ctypes.POINTER(NgramLM), c_float, c_float, c_int, c_void_p],
+	'cab_ctc_beam_search_stream_state_bytes': [c_int, c_int, ctypes.POINTER(c_i64)],
+	'cab_ctc_beam_search_stream_workspace': [c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_i64)],
+	'cab_ctc_beam_search_stream': [c_void_p, c_i64, c_i64, c_i64, ctypes.POINTER(BeamStreamRow), c_int, c_int, c_int, c_int, c_float, c_int, c_int,
+									c_int, c_void_p, c_i64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, ctypes.POINTER(NgramLM), c_float, c_float,
+									c_int, c_void_p],
 }
 HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace', 'cab_ctc_loss_one_cta_covers', 'cab_ctc_loss_long_workspace',
-			'cab_ctc_beam_search_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
+			'cab_ctc_beam_search_workspace', 'cab_ctc_beam_search_stream_state_bytes', 'cab_ctc_beam_search_stream_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
 INTROSPECTION = {'cab_abi_version': c_int, 'cab_last_error': ctypes.c_char_p, 'cab_launch_count': c_i64}
 
 

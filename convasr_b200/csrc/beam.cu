@@ -277,11 +277,62 @@ __device__ float lm_word_score(const BeamLm& lm, const int* ctx, int w) {
     return found ? 2.302585093f * (bo + p) : kLmOovScore;
 }
 
-template <bool LM>
+// ------------------------------------------------------------------------------------------
+// Streaming instance (STREAM): row b continues the stream of rows[b].  The beam set a frame leaves behind is loaded from
+// the row's state block before the first frame (the root, the empty prefix, when the stream has consumed no frame) and
+// stored back after the last; node ids and the re-link test use the stream's absolute frame t0 + t, in the row's own
+// node table.  Everything that crosses a frame boundary is in the block, so the frames of a stream give the beams of
+// the one-shot search whatever the chunks.  The LM's end term and re-rank go to the outputs only.
+// ------------------------------------------------------------------------------------------
+struct BeamStreamState {  // views into a state block (layout: cab_ctc_beam_search_stream_state_bytes)
+    int* hdr;             // {t0, beam count, finished, 0}
+    uint64_t* hash;
+    uint64_t* phash;
+    float* pb;
+    float* pnb;
+    int* last;
+    int* node;
+    int* prank;
+    int* tnode;  // LM only
+    float* bonus;
+    int* ctx;    // [W][lm_order - 1]
+};
+
+__host__ __device__ __forceinline__ size_t beam_state_layout(unsigned char* base, int W, int lm_order, BeamStreamState* v) {
+    const size_t w = (size_t)W;
+    size_t o = 16;
+    const size_t o_hash = o; o += 8 * w;
+    const size_t o_phash = o; o += 8 * w;
+    const size_t o_pb = o; o += 4 * w;
+    const size_t o_pnb = o; o += 4 * w;
+    const size_t o_last = o; o += 4 * w;
+    const size_t o_node = o; o += 4 * w;
+    const size_t o_prank = o; o += 4 * w;
+    const size_t o_tnode = o; o += lm_order > 0 ? 4 * w : 0;
+    const size_t o_bonus = o; o += lm_order > 0 ? 4 * w : 0;
+    const size_t o_ctx = o; o += lm_order > 1 ? 4 * w * (size_t)(lm_order - 1) : 0;
+    if (v) {
+        v->hdr = reinterpret_cast<int*>(base);
+        v->hash = reinterpret_cast<uint64_t*>(base + o_hash);
+        v->phash = reinterpret_cast<uint64_t*>(base + o_phash);
+        v->pb = reinterpret_cast<float*>(base + o_pb);
+        v->pnb = reinterpret_cast<float*>(base + o_pnb);
+        v->last = reinterpret_cast<int*>(base + o_last);
+        v->node = reinterpret_cast<int*>(base + o_node);
+        v->prank = reinterpret_cast<int*>(base + o_prank);
+        v->tnode = reinterpret_cast<int*>(base + o_tnode);
+        v->bonus = reinterpret_cast<float*>(base + o_bonus);
+        v->ctx = reinterpret_cast<int*>(base + o_ctx);
+    }
+    return (o + 15) & ~(size_t)15;
+}
+
+template <bool LM, bool STREAM>
 __global__ void __launch_bounds__(kBeamThreads, 1)
 beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp, const int* __restrict__ p_cnt,
                    const int64_t* __restrict__ lengths, int T, int N, int blank, int W, int K,
-                   BeamNode* __restrict__ nodes, int* __restrict__ final_node, float* __restrict__ out_scores, const BeamLm lm) {
+                   BeamNode* __restrict__ nodes, int* __restrict__ final_node, float* __restrict__ out_scores, const BeamLm lm,
+                   const cab_beam_stream_t* __restrict__ rows) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int b = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -318,9 +369,31 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
     float* s_spb = s_bonus + 2 * W;                                  // [W] this frame's space bonus, -inf = no space
     int* s_word = reinterpret_cast<int*>(s_spb + W);                // [W] word id of the beam's node, or -1
 
+    int cur = 0, nb = 1;
     const int64_t len64 = lengths ? lengths[b] : T;
-    const int len = len64 < 0 ? 0 : (len64 > T ? T : (int)len64);
-    if (tid == 0) {
+    int len = len64 < 0 ? 0 : (len64 > T ? T : (int)len64);
+    int t0 = 0;
+    BeamStreamState ss;
+    if constexpr (STREAM) {
+        const cab_beam_stream_t row = rows[b];
+        beam_state_layout(static_cast<unsigned char*>(row.state), W, LM ? lm.order : 0, &ss);
+        t0 = ss.hdr[0];
+        nb = t0 > 0 ? ss.hdr[1] : 1;
+        // the caller checked t0 + frames against the capacity; the clamp only keeps a state out of step in bounds
+        const int64_t room = row.capacity - t0;
+        len = row.frames < 0 ? 0 : (row.frames > T ? T : row.frames);
+        if (len > room) len = room < 0 ? 0 : (int)room;
+        if (t0 > 0 && tid < nb) {
+            s_hash[tid] = ss.hash[tid]; s_phash[tid] = ss.phash[tid]; s_pb[tid] = ss.pb[tid]; s_pnb[tid] = ss.pnb[tid];
+            s_last[tid] = ss.last[tid]; s_node[tid] = ss.node[tid]; s_prank[tid] = ss.prank[tid];
+            if constexpr (LM) {
+                s_tnode[tid] = ss.tnode[tid];
+                s_bonus[tid] = ss.bonus[tid];
+                for (int k = 0; k < lm.order - 1; ++k) s_ctx[tid * kCtx + k] = ss.ctx[tid * (lm.order - 1) + k];
+            }
+        }
+    }
+    if (tid == 0 && t0 == 0) {
         s_hash[0] = 0; s_phash[0] = 0; s_pb[0] = 0.f; s_pnb[0] = -INFINITY; s_last[0] = -1; s_node[0] = -1; s_prank[0] = -1;
         if constexpr (LM) {
             s_tnode[0] = 0;
@@ -328,9 +401,9 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
             for (int k = 0; k < kCtx; ++k) s_ctx[k] = lm.bos;
         }
     }
-    int cur = 0, nb = 1;
     const size_t frame0 = (size_t)b * T;
     BeamNode* bnodes = nodes + frame0 * W;
+    if constexpr (STREAM) bnodes = static_cast<BeamNode*>(rows[b].nodes);
     // next frame's pruned classes, prefetched into registers by threads < N
     int nx_cls = -1, nx_cnt = 0;
     float nx_lp = -INFINITY;
@@ -535,7 +608,7 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
                 }
                 s_pnb[nxt * W + r] = v;
                 s_last[nxt * W + r] = c;
-                const int id = t * W + r;
+                const int id = (t0 + t) * W + r;
                 s_node[nxt * W + r] = id;
                 bnodes[id] = BeamNode{s_node[cur * W + i], c};
                 s_hash[nxt * W + r] = beam_hash(s_hash[cur * W + i], c);
@@ -553,7 +626,7 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
                     // the shorter prefix was not a beam before this frame: it may have come back as a new extension
                     const uint64_t ph = s_phash[nxt * W + r];
                     for (int f = 0; f < Kn; ++f)
-                        if (s_hash[nxt * W + f] == ph && s_node[nxt * W + f] == t * W + f) { pr = f; break; }
+                        if (s_hash[nxt * W + f] == ph && s_node[nxt * W + f] == (t0 + t) * W + f) { pr = f; break; }
                 }
             } else {
                 pr = s_newrank[src];
@@ -564,6 +637,26 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
         cur = nxt;
         __syncthreads();
         if (nb == 0) break;
+    }
+    if constexpr (STREAM) {
+        // store the beam set the last frame left; t0 advances by the frames consumed
+        __syncthreads();
+        if (tid < nb) {
+            ss.hash[tid] = s_hash[cur * W + tid]; ss.phash[tid] = s_phash[cur * W + tid];
+            ss.pb[tid] = s_pb[cur * W + tid]; ss.pnb[tid] = s_pnb[cur * W + tid];
+            ss.last[tid] = s_last[cur * W + tid]; ss.node[tid] = s_node[cur * W + tid]; ss.prank[tid] = s_prank[cur * W + tid];
+            if constexpr (LM) {
+                ss.tnode[tid] = s_tnode[cur * W + tid];
+                ss.bonus[tid] = s_bonus[cur * W + tid];
+                for (int k = 0; k < lm.order - 1; ++k) ss.ctx[tid * (lm.order - 1) + k] = s_ctx[(cur * W + tid) * kCtx + k];
+            }
+        }
+        if (tid == 0) {
+            ss.hdr[0] = t0 + len;
+            ss.hdr[1] = nb;
+            ss.hdr[2] = rows[b].is_eos != 0;
+            ss.hdr[3] = 0;
+        }
     }
     if constexpr (LM) {
         // the last word's term, then re-rank by counting (ties to the earlier rank); hypothesis r is beam s_order[r]
@@ -606,13 +699,18 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
     }
 }
 
-// back-trace: one thread per hypothesis; tokens in order, emission frame = the frame the prefix was created
+// back-trace: one thread per hypothesis; tokens in order, emission frame = the frame the prefix was created (STREAM:
+// in row b's own node table, frames counted from the stream's start)
+template <bool STREAM>
 __global__ void __launch_bounds__(kBeamMaxW)
 beam_backtrace_kernel(const BeamNode* __restrict__ nodes, const int* __restrict__ final_node, int T, int W, int K, int L_cap,
-                      int* __restrict__ out_tokens, int* __restrict__ out_frames, int* __restrict__ out_lengths) {
+                      int* __restrict__ out_tokens, int* __restrict__ out_frames, int* __restrict__ out_lengths,
+                      const cab_beam_stream_t* __restrict__ rows) {
     const int b = blockIdx.x, r = threadIdx.x;
     if (r >= K) return;
-    const BeamNode* bn = nodes + (size_t)b * T * W;
+    const BeamNode* bn;
+    if constexpr (STREAM) bn = static_cast<const BeamNode*>(rows[b].nodes);
+    else bn = nodes + (size_t)b * T * W;
     const size_t o = (size_t)b * K + r;
     const int start = final_node[o];
     int L = 0;
@@ -645,6 +743,22 @@ static size_t beam_workspace_bytes(int B, int T, int N, int W) {
     return beam_align(off[4] + (size_t)B * W * 4);
 }
 
+// streaming workspace: pruned classes, log-probs and counts of the chunk as above, final node int32 [B, K], and the
+// rows' descriptors copied to the device
+static void beam_stream_workspace_layout(int B, int T, int N, int K, size_t off[5]) {
+    const size_t BT = (size_t)B * T;
+    off[0] = 0;
+    off[1] = beam_align(off[0] + BT * N * 4);
+    off[2] = beam_align(off[1] + BT * N * 4);
+    off[3] = beam_align(off[2] + BT * 4);
+    off[4] = beam_align(off[3] + (size_t)B * K * 4);
+}
+static size_t beam_stream_workspace_bytes(int B, int T, int N, int K) {
+    size_t off[5];
+    beam_stream_workspace_layout(B, T, N, K, off);
+    return beam_align(off[4] + (size_t)B * sizeof(cab_beam_stream_t));
+}
+
 static size_t beam_search_smem(int W, int N, bool lm) {
     size_t bytes = 2 * W * 8 * 2 + 2 * W * 4 * 5 + W * 4 * 6 + N * 8 + 256 * 4 + (kBeamThreads / 32 + 8) * 4;
     bytes += (size_t)((W * N + 1) & ~1) * 2 + (size_t)W * (N + 1) * 4;
@@ -652,38 +766,52 @@ static size_t beam_search_smem(int W, int N, bool lm) {
     return bytes;
 }
 
-// prune -> search -> back-trace; the arguments are checked by the caller
-template <bool LM>
+// prune -> search -> back-trace; the arguments are checked by the caller.  STREAM: `rows` are the host descriptors,
+// copied into the workspace before the launches
+template <bool LM, bool STREAM = false>
 static int beam_search_launch(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t, const int64_t* output_lengths,
                               int B, int T, int C, int N, float cutoff_prob, int blank, int W, int K, void* workspace, int32_t* out_tokens,
                               int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores, const BeamLm& lm,
-                              cudaStream_t stream) {
+                              cudaStream_t stream, const cab_beam_stream_t* rows = nullptr) {
     size_t off[5];
-    beam_workspace_layout(B, T, N, W, off);
     unsigned char* ws = static_cast<unsigned char*>(workspace);
+    BeamNode* nodes = nullptr;
+    int* final_node;
+    const cab_beam_stream_t* d_rows = nullptr;
+    if constexpr (STREAM) {
+        beam_stream_workspace_layout(B, T, N, K, off);
+        final_node = reinterpret_cast<int*>(ws + off[3]);
+        cab_beam_stream_t* dr = reinterpret_cast<cab_beam_stream_t*>(ws + off[4]);
+        CAB_CHECK_CUDA(cudaMemcpyAsync(dr, rows, (size_t)B * sizeof(cab_beam_stream_t), cudaMemcpyHostToDevice, stream));
+        d_rows = dr;
+    } else {
+        beam_workspace_layout(B, T, N, W, off);
+        nodes = reinterpret_cast<BeamNode*>(ws + off[3]);
+        final_node = reinterpret_cast<int*>(ws + off[4]);
+    }
     int* p_cls = reinterpret_cast<int*>(ws + off[0]);
     float* p_lp = reinterpret_cast<float*>(ws + off[1]);
     int* p_cnt = reinterpret_cast<int*>(ws + off[2]);
-    BeamNode* nodes = reinterpret_cast<BeamNode*>(ws + off[3]);
-    int* final_node = reinterpret_cast<int*>(ws + off[4]);
 
     const size_t smem = beam_search_smem(W, N, LM);
     static size_t smem_set = 0;
     if (smem > 48 * 1024 && smem > smem_set) {
-        CAB_CHECK_CUDA(cudaFuncSetAttribute(beam_search_kernel<LM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        CAB_CHECK_CUDA(cudaFuncSetAttribute(beam_search_kernel<LM, STREAM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                             (int)beam_search_smem(kBeamMaxW, kBeamMaxN, LM)));
         smem_set = beam_search_smem(kBeamMaxW, kBeamMaxN, LM);
     }
     dim3 pgrid((T + kPruneWarps - 1) / kPruneWarps, B);
+    if (pgrid.x == 0) pgrid.x = 1;  // a streaming call of 0 frames: the prune warps find no frame
     beam_prune_kernel<<<pgrid, kPruneWarps * 32, 0, stream>>>(log_probs, stride_b, stride_c, stride_t, C, T, N, cutoff_prob, p_cls,
                                                                p_lp, p_cnt);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    beam_search_kernel<LM><<<B, kBeamThreads, smem, stream>>>(p_cls, p_lp, p_cnt, output_lengths, T, N, blank, W, K, nodes, final_node,
-                                                              out_scores, lm);
+    beam_search_kernel<LM, STREAM><<<B, kBeamThreads, smem, stream>>>(p_cls, p_lp, p_cnt, output_lengths, T, N, blank, W, K, nodes,
+                                                                      final_node, out_scores, lm, d_rows);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    beam_backtrace_kernel<<<B, kBeamMaxW, 0, stream>>>(nodes, final_node, T, W, K, L_cap, out_tokens, out_frames, out_lengths);
+    beam_backtrace_kernel<STREAM><<<B, kBeamMaxW, 0, stream>>>(nodes, final_node, T, W, K, L_cap, out_tokens, out_frames, out_lengths,
+                                                                d_rows);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     return 0;
@@ -726,12 +854,8 @@ extern "C" int cab_ctc_beam_search(const float* log_probs, int64_t stride_b, int
                                      static_cast<cudaStream_t>(stream_));
 }
 
-extern "C" int cab_ctc_beam_search_lm(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
-                                      const int64_t* output_lengths, int B, int T, int C, int N, float cutoff_prob, int blank,
-                                      int W, int K, void* workspace, int64_t workspace_bytes, int32_t* out_tokens,
-                                      int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores,
-                                      const cab_ngram_lm_t* lm, float alpha, float beta, int space, cab_stream_t stream_) {
-    CAB_BEAM_CHECK_CALL();
+// the LM arguments checked and turned into the kernel's view
+static int beam_lm_view(const cab_ngram_lm_t* lm, int C, int blank, float alpha, float beta, int space, BeamLm* out) {
     CAB_CHECK_ARG(lm != nullptr, "null lm");
     CAB_CHECK_ARG(lm->order >= 1 && lm->order <= kLmMaxOrder, "lm order=%d out of [1, %d]", lm->order, kLmMaxOrder);
     CAB_CHECK_ARG(lm->num_classes == C, "lm trie has %d classes, log_probs %d", lm->num_classes, C);
@@ -756,7 +880,81 @@ extern "C" int cab_ctc_beam_search_lm(const float* log_probs, int64_t stride_b, 
     v.bos = lm->bos;
     v.alpha = alpha;
     v.beta = beta;
+    *out = v;
+    return 0;
+}
+
+extern "C" int cab_ctc_beam_search_lm(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                                      const int64_t* output_lengths, int B, int T, int C, int N, float cutoff_prob, int blank,
+                                      int W, int K, void* workspace, int64_t workspace_bytes, int32_t* out_tokens,
+                                      int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores,
+                                      const cab_ngram_lm_t* lm, float alpha, float beta, int space, cab_stream_t stream_) {
+    CAB_BEAM_CHECK_CALL();
+    BeamLm v{};
+    const int rc = beam_lm_view(lm, C, blank, alpha, beta, space, &v);
+    if (rc != 0) return rc;
     return beam_search_launch<true>(log_probs, stride_b, stride_c, stride_t, output_lengths, B, T, C, N, cutoff_prob, blank, W, K,
                                     workspace, out_tokens, out_frames, L_cap, out_lengths, out_scores, v,
                                     static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int cab_ctc_beam_search_stream_state_bytes(int W, int lm_order, int64_t* bytes) {
+    CAB_CHECK_ARG(bytes != nullptr, "null output");
+    CAB_CHECK_ARG(W >= 1 && W <= kBeamMaxW, "beam_width=%d out of [1, %d]", W, kBeamMaxW);
+    CAB_CHECK_ARG(lm_order >= 0 && lm_order <= kLmMaxOrder, "lm_order=%d out of [0, %d] (0: no LM)", lm_order, kLmMaxOrder);
+    *bytes = (int64_t)beam_state_layout(nullptr, W, lm_order, nullptr);
+    return 0;
+}
+
+extern "C" int cab_ctc_beam_search_stream_workspace(int B, int T, int N, int W, int K, int64_t* bytes) {
+    CAB_CHECK_ARG(bytes != nullptr, "null output");
+    CAB_CHECK_ARG(B > 0 && T >= 0, "bad shape B=%d T=%d", B, T);
+    CAB_CHECK_ARG(W >= 1 && W <= kBeamMaxW, "beam_width=%d out of [1, %d]", W, kBeamMaxW);
+    CAB_CHECK_ARG(N >= 1 && N <= kBeamMaxN, "N=%d out of [1, %d]", N, kBeamMaxN);
+    CAB_CHECK_ARG(K >= 1 && K <= W, "K=%d out of [1, beam_width=%d]", K, W);
+    *bytes = (int64_t)beam_stream_workspace_bytes(B, T, N, K);
+    return 0;
+}
+
+extern "C" int cab_ctc_beam_search_stream(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                                          const cab_beam_stream_t* rows, int B, int T, int C, int N, float cutoff_prob, int blank,
+                                          int W, int K, void* workspace, int64_t workspace_bytes, int32_t* out_tokens,
+                                          int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores,
+                                          const cab_ngram_lm_t* lm, float alpha, float beta, int space, cab_stream_t stream_) {
+    CAB_CHECK_ARG(rows && workspace && out_tokens && out_frames && out_lengths && out_scores, "null pointer argument");
+    CAB_CHECK_ARG(B > 0 && T >= 0 && C > 0, "bad shape B=%d T=%d C=%d", B, T, C);
+    CAB_CHECK_ARG(T == 0 || log_probs, "null log_probs");
+    CAB_CHECK_ARG(W >= 1 && W <= kBeamMaxW, "beam_width=%d out of [1, %d]", W, kBeamMaxW);
+    CAB_CHECK_ARG(N >= 1 && N <= kBeamMaxN && N <= C, "N=%d out of [1, %d] (C=%d)", N, kBeamMaxN, C);
+    CAB_CHECK_ARG(K >= 1 && K <= W, "K=%d out of [1, beam_width=%d]", K, W);
+    CAB_CHECK_ARG(blank >= 0 && blank < C, "blank=%d out of range (C=%d)", blank, C);
+    CAB_CHECK_ARG(cutoff_prob > 0.f && cutoff_prob <= 1.f, "cutoff_prob=%g out of (0, 1]", (double)cutoff_prob);
+    CAB_CHECK_ARG(L_cap >= 1, "L_cap=%d must be positive", L_cap);
+    CAB_CHECK_ARG(workspace_bytes >= (int64_t)beam_stream_workspace_bytes(B, T, N, K), "workspace of %lld bytes is too small (%lld needed)",
+                  (long long)workspace_bytes, (long long)beam_stream_workspace_bytes(B, T, N, K));
+    BeamLm v{};
+    if (lm) {
+        const int rc = beam_lm_view(lm, C, blank, alpha, beta, space, &v);
+        if (rc != 0) return rc;
+    }
+    const int64_t need_state = (int64_t)beam_state_layout(nullptr, W, lm ? lm->order : 0, nullptr);
+    for (int b = 0; b < B; ++b) {
+        const cab_beam_stream_t& r = rows[b];
+        CAB_CHECK_ARG(r.state && r.nodes, "row %d: null state or node table", b);
+        CAB_CHECK_ARG(r.state_bytes >= need_state, "row %d: state block of %lld bytes, %lld needed", b, (long long)r.state_bytes,
+                      (long long)need_state);
+        CAB_CHECK_ARG(!r.finished, "row %d: the stream has ended (an earlier call had is_eos)", b);
+        CAB_CHECK_ARG(r.frames >= 0 && r.frames <= T, "row %d: frames=%d out of [0, T=%d]", b, r.frames, T);
+        CAB_CHECK_ARG(r.capacity >= 0 && r.capacity <= INT32_MAX / W, "row %d: node table capacity %lld frames out of [0, %d]", b,
+                      (long long)r.capacity, INT32_MAX / W);
+        CAB_CHECK_ARG(r.t0 >= 0 && r.t0 + r.frames <= r.capacity, "row %d: t0=%lld + frames=%d overruns the node table (%lld frames)", b,
+                      (long long)r.t0, r.frames, (long long)r.capacity);
+        for (int c = 0; c < b; ++c) CAB_CHECK_ARG(rows[c].state != r.state, "rows %d and %d share a state block", c, b);
+    }
+    if (lm) return beam_search_launch<true, true>(log_probs, stride_b, stride_c, stride_t, nullptr, B, T, C, N, cutoff_prob, blank, W, K,
+                                                  workspace, out_tokens, out_frames, L_cap, out_lengths, out_scores, v,
+                                                  static_cast<cudaStream_t>(stream_), rows);
+    return beam_search_launch<false, true>(log_probs, stride_b, stride_c, stride_t, nullptr, B, T, C, N, cutoff_prob, blank, W, K,
+                                           workspace, out_tokens, out_frames, L_cap, out_lengths, out_scores, v,
+                                           static_cast<cudaStream_t>(stream_), rows);
 }

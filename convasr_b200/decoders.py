@@ -5,6 +5,7 @@ collapse (that lives in transcript_generators.GreedyCTCGenerator).  K=1 is the f
 (ties -> lowest id, as torch.argmax); K>1 is the native top-K kernel (K <= 8).
 BeamSearchDecoder: CTC prefix beam search on the GPU (csrc/beam.cu), acoustic only or fused with a word n-gram LM read
 from an ARPA file (convasr_b200/lm.py); KenLM's binary format is not read.
+OnlineBeamSearchDecoder: the same search resumed chunk by chunk, one state per stream.
 """
 import math
 
@@ -82,9 +83,56 @@ class BeamSearchDecoder:
 
 	def decode(self, log_probs, output_lengths = None):
 		"""topk = 1: one token list per utterance; topk > 1: per utterance, up to topk token lists, best first."""
-		r = self.decode_nbest(log_probs, output_lengths)
+		return self._token_lists(self.decode_nbest(log_probs, output_lengths))
+
+	def _token_lists(self, r):
 		lengths, scores = r['lengths'].cpu().tolist(), r['scores'].cpu().tolist()
 		n_max = max([max(l) for l in lengths], default = 0)
 		tokens = r['tokens'][:, :, :n_max].cpu().tolist()
 		out = [[tok[:l] for tok, l, s in zip(tb, lb, sb) if s > -math.inf] for tb, lb, sb in zip(tokens, lengths, scores)]
 		return [o[0] if o else [] for o in out] if self.topk == 1 else out
+
+
+class OnlineBeamSearchDecoder(BeamSearchDecoder):
+	"""BeamSearchDecoder for posteriors that arrive over time (ctcdecode's OnlineCTCBeamDecoder): the same constructor
+	and search, resumed chunk by chunk per stream (ops.ctc_beam_search_stream, csrc/beam.cu).
+
+	    dec = OnlineBeamSearchDecoder(labels, beam_width = 100)
+	    state = dec.new_state()                             # one per stream
+	    for chunk, last in chunks:                          # chunk: [1, C, T_chunk] log_probs, any T_chunk >= 0
+	        partial = dec.decode(chunk, [state], is_eos = last)
+
+	After the chunk containing frame t the result is bit for bit BeamSearchDecoder's on frames 0..t of the stream
+	(with an LM, the last word's term and the re-rank included).  Each call may batch any streams in any rows; a row's
+	`output_lengths` entry is its frame count in this call (0 allowed).  A state belongs to the decoder that made it;
+	after an is_eos call it is finished and feeding it again raises."""
+
+	def new_state(self, capacity = 1024):
+		"""a new stream; `capacity` is the node table's first size in frames (it grows by doubling)"""
+		return ops.BeamStreamState(config = self._config(), capacity = capacity)
+
+	def _config(self):
+		return (tuple(self.labels), self.lm_path, self.beam_width, self.beam_alpha, self.beam_beta, self.cutoff_top_n, self.cutoff_prob,
+				self.topk, self.blank_id)
+
+	def decode_nbest(self, log_probs, states, is_eos, output_lengths = None):
+		"""device tensors as BeamSearchDecoder.decode_nbest, [B, topk, L] tokens and frames with L the longest stream's
+		frames so far; frames count from the stream's start"""
+		if any(s.finished for s in states if isinstance(s, ops.BeamStreamState)):
+			raise RuntimeError('convasr_b200: a stream of this call has ended (is_eos was set on an earlier call); start a new state')
+		if log_probs.shape[1] != len(self.labels):
+			raise ValueError(f'convasr_b200: log_probs have {log_probs.shape[1]} classes, the decoder {len(self.labels)} labels')
+		config = self._config()
+		for b, s in enumerate(states):
+			if not isinstance(s, ops.BeamStreamState) or s.config != config:
+				raise ValueError(f'convasr_b200: the stream state of row {b} was not made by this decoder configuration (new_state())')
+		tokens, frames, lengths, scores = ops.ctc_beam_search_stream(
+			log_probs, states, is_eos, output_lengths, beam_width = self.beam_width, cutoff_top_n = self.cutoff_top_n,
+			cutoff_prob = self.cutoff_prob, topk = self.topk, blank = self.blank_id, lm = self.lm, alpha = self.beam_alpha, beta = self.beam_beta
+		)
+		return dict(tokens = tokens, frames = frames, lengths = lengths, scores = scores)
+
+	def decode(self, log_probs, states, is_eos, output_lengths = None):
+		"""token lists as BeamSearchDecoder.decode, for each row's stream so far"""
+		r = self.decode_nbest(log_probs, states, is_eos, output_lengths)
+		return self._token_lists(r)

@@ -473,6 +473,114 @@ def ctc_beam_search(log_probs, output_lengths = None, beam_width = 100, cutoff_t
 	return tokens, frames, lengths, scores
 
 
+class BeamStreamState:
+	"""One stream of ctc_beam_search_stream: the device state block (the beam set between two frames), the node table
+	(W nodes of 8 bytes per frame, indexed by the stream's absolute frame, grown geometrically by copying), the frames
+	consumed so far and whether the stream has ended.  The search configuration (C, blank, beam width, pruning, topk, LM,
+	alpha, beta) is bound on the first call and a call with another one is refused; `config` is the configuration of the
+	decoder that made the state, if any (checked by that decoder).  `capacity`: the node table's first size in frames."""
+
+	def __init__(self, config = None, capacity = 1024):
+		self.config = config
+		self.search = None
+		self.t0 = 0
+		self.finished = False
+		self.initial_capacity = max(1, int(capacity))
+		self.state = None  # uint8 device tensor, zeroed: a fresh stream
+		self.nodes = None  # int32 device tensor [capacity, W, 2]
+
+	@property
+	def capacity(self):
+		return 0 if self.nodes is None else self.nodes.shape[0]
+
+	def _reserve(self, frames, W, state_bytes, dev):
+		if self.state is None:
+			self.state = torch.zeros(state_bytes, dtype = torch.uint8, device = dev)
+		need = self.t0 + frames
+		if self.nodes is None or need > self.capacity:
+			cap = max(need, 2 * self.capacity, self.initial_capacity)
+			nodes = torch.empty(cap, W, 2, dtype = torch.int32, device = dev)
+			if self.t0 > 0:
+				nodes[:self.t0].copy_(self.nodes[:self.t0])
+			self.nodes = nodes
+
+
+def beam_stream_state_bytes(beam_width, lm_order = 0):
+	"""bytes of one stream's state block (host-only query)"""
+	n = ctypes.c_int64()
+	_lib.check(_lib.load().cab_ctc_beam_search_stream_state_bytes(int(beam_width), int(lm_order), ctypes.byref(n)), 'cab_ctc_beam_search_stream_state_bytes')
+	return n.value
+
+
+def ctc_beam_search_stream(log_probs, states, is_eos, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0, topk = 1,
+							blank = None, lm = None, alpha = 0.0, beta = 0.0):
+	"""Streaming CTC prefix beam search: row b of fp32 [B, C, T] log_probs (any strides) holds the next output_lengths[b]
+	frames (None: T; 0 is allowed) of the stream states[b] (BeamStreamState, one per row, each at most once).  is_eos:
+	a bool, or one per row: that row's stream ends with this call.  Returns ctc_beam_search's tensors with [B, topk, L]
+	tokens and frames, L the longest stream's frames so far: the stream's current n-best list, frames counted from its
+	start, bit for bit what ctc_beam_search returns for the stream's frames so far with the same arguments (with an LM,
+	the last word's term and the re-rank included).  A finished stream, or a state bound to another configuration, is
+	refused."""
+	states = list(states)
+	for b, s in enumerate(states):
+		if s.finished:
+			raise RuntimeError(f'convasr_b200: the stream of row {b} has ended (is_eos was set on an earlier call); start a new state')
+	B, C, T = log_probs.shape
+	if len(states) != B:
+		raise ValueError(f'convasr_b200: {len(states)} stream states for a batch of {B}')
+	if len({id(s) for s in states}) != B:
+		raise ValueError('convasr_b200: one stream state appears in two rows of the call')
+	eos = [bool(is_eos)] * B if isinstance(is_eos, (bool, int)) else [bool(e) for e in torch.as_tensor(is_eos).reshape(-1).tolist()]
+	if len(eos) != B:
+		raise ValueError(f'convasr_b200: {len(eos)} is_eos flags for a batch of {B}')
+	frames = [T] * B if output_lengths is None else [min(max(int(n), 0), T) for n in torch.as_tensor(output_lengths).reshape(-1).tolist()]
+	if len(frames) != B:
+		raise ValueError(f'convasr_b200: {len(frames)} output lengths for a batch of {B}')
+	blank = C - 1 if blank is None else int(blank)
+	N = min(int(cutoff_top_n), C)
+	W, K = int(beam_width), int(topk)
+	if lm is not None and lm.blank != blank:
+		raise ValueError(f'convasr_b200: the LM was built with blank={lm.blank}, the search uses blank={blank}')
+	search = (C, blank, W, N, float(cutoff_prob), K, None if lm is None else id(lm), float(alpha), float(beta))
+	for b, s in enumerate(states):
+		if s.search is not None and s.search != search:
+			raise ValueError(f'convasr_b200: the stream state of row {b} belongs to another search configuration ({s.search} != {search})')
+	_need_cuda(log_probs)
+	lp = log_probs if log_probs.dtype == torch.float32 else log_probs.float()
+	dev = lp.device
+	if B == 0:
+		z = torch.empty(0, K, 0, dtype = torch.int32, device = dev)
+		return z, z.clone(), torch.empty(0, K, dtype = torch.int32, device = dev), torch.empty(0, K, device = dev)
+	lib = _lib.load()
+	state_bytes = beam_stream_state_bytes(W, 0 if lm is None else lm.order)
+	for s, n in zip(states, frames):
+		s._reserve(n, W, state_bytes, dev)
+	rows = (_lib.BeamStreamRow * B)()
+	for r, s, n, e in zip(rows, states, frames, eos):
+		r.state, r.nodes, r.state_bytes, r.capacity = s.state.data_ptr(), s.nodes.data_ptr(), s.state.numel(), s.capacity
+		r.t0, r.frames, r.is_eos, r.finished = s.t0, n, int(e), int(s.finished)
+	L_cap = max(1, max(s.t0 + n for s, n in zip(states, frames)))
+	nbytes = ctypes.c_int64()
+	_lib.check(lib.cab_ctc_beam_search_stream_workspace(B, T, N, W, K, ctypes.byref(nbytes)), 'cab_ctc_beam_search_stream_workspace')
+	ws = torch.empty(nbytes.value, dtype = torch.uint8, device = dev)
+	tokens = torch.empty(B, K, L_cap, dtype = torch.int32, device = dev)
+	frames_out = torch.empty_like(tokens)
+	lengths = torch.empty(B, K, dtype = torch.int32, device = dev)
+	scores = torch.empty(B, K, dtype = torch.float32, device = dev)
+	lm_arg = None if lm is None else ctypes.byref(lm.device_struct(dev))
+	space = 0 if lm is None else lm.space
+	rc = lib.cab_ctc_beam_search_stream(
+		_p(lp) if T > 0 else None, lp.stride(0), lp.stride(1), lp.stride(2), rows, B, T, C, N, float(cutoff_prob), blank, W, K, _p(ws), nbytes.value,
+		_p(tokens), _p(frames_out), L_cap, _p(lengths), _p(scores), lm_arg, float(alpha), float(beta), space, _stream()
+	)
+	_lib.check(rc, 'cab_ctc_beam_search_stream')
+	for s, n, e in zip(states, frames, eos):
+		s.search = search
+		s.t0 += n
+		s.finished = e
+	return tokens, frames_out, lengths, scores
+
+
 def entropy(log_probs, lengths = None, eps_id = -1):
 	_need_cuda(log_probs, lengths)
 	log_probs = log_probs.to(torch.float32).contiguous()

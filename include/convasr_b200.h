@@ -565,6 +565,51 @@ int cab_ctc_beam_search_lm(const float* log_probs, int64_t stride_b, int64_t str
                            float* out_scores, const cab_ngram_lm_t* lm, float alpha, float beta, int space,
                            cab_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Streaming (resumable) CTC prefix beam search, acoustic only (lm null) or with the word n-gram
+ *   LM above.  A stream's log-probs arrive in chunks; each call advances every row's stream by
+ *   that row's `frames` (0 allowed) and returns its current K best hypotheses.  After the call
+ *   that consumed frames 0..t of a stream, tokens, frames, lengths and scores equal bit for bit
+ *   what cab_ctc_beam_search (cab_ctc_beam_search_lm) returns for frames 0..t of that stream
+ *   with the same arguments: with an LM they include the last word's term and the re-rank,
+ *   computed for the outputs only; the stored state stays the search's beam set.
+ *   State block (device, cab_ctc_beam_search_stream_state_bytes(W, lm_order) bytes, zeroed
+ *   before the stream's first call): int32 {t0, beam count, finished, 0}, then per beam the
+ *   prefix hash and parent hash (uint64), p_blank, p_nonblank (fp32), last class, node id and
+ *   parent rank (int32), and with an LM the trie node, the bonus and the order - 1 context
+ *   word ids.  Node table (device): `capacity` frames of W entries {int32 parent, int32 class},
+ *   indexed by the stream's absolute frame (node id = frame * W + rank); out_frames count from
+ *   the stream's start.  The caller keeps t0 and finished in the descriptor in step with the
+ *   state (t0 += frames, finished = is_eos after each call) and grows a node table by copying
+ *   its first t0 frames into a larger one.
+ *   log_probs [B, C, T] through element strides (null allowed when T = 0); workspace of
+ *   cab_ctc_beam_search_stream_workspace bytes; outputs as cab_ctc_beam_search.
+ *   Refused before any launch: W, N, K, blank, cutoff_prob and the LM as above; a null row
+ *   array, state or node table; a state block smaller than the state bytes; frames outside
+ *   [0, T]; a finished stream; t0 + frames above capacity; capacity * W above INT32_MAX; two
+ *   rows with one state block.  Three launches (prune, search, back-trace).
+ * ------------------------------------------------------------------------------------- */
+typedef struct {
+    void* state;          /* device state block */
+    void* nodes;          /* device node table, capacity * W entries of 8 bytes */
+    int64_t state_bytes;  /* bytes of the state block */
+    int64_t capacity;     /* frames the node table holds */
+    int64_t t0;           /* frames the stream consumed before this call */
+    int32_t frames;       /* frames of this call, [0, T] */
+    int32_t is_eos;       /* nonzero: this call ends the stream */
+    int32_t finished;     /* nonzero: an earlier call ended the stream (refused) */
+    int32_t reserved;
+} cab_beam_stream_t;
+
+int cab_ctc_beam_search_stream_state_bytes(int W, int lm_order, int64_t* bytes);
+int cab_ctc_beam_search_stream_workspace(int B, int T, int N, int W, int K, int64_t* bytes);
+int cab_ctc_beam_search_stream(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                               const cab_beam_stream_t* rows, int B, int T, int C, int N, float cutoff_prob,
+                               int blank, int W, int K, void* workspace, int64_t workspace_bytes,
+                               int32_t* out_tokens, int32_t* out_frames, int L_cap, int32_t* out_lengths,
+                               float* out_scores, const cab_ngram_lm_t* lm, float alpha, float beta, int space,
+                               cab_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
