@@ -62,6 +62,11 @@ class BeamStreamRow(ctypes.Structure):  # cab_beam_stream_t
 				('is_eos', c_i32), ('finished', c_i32), ('reserved', c_i32)]
 
 
+class BeamStreamIncrementalRow(ctypes.Structure):  # cab_beam_stream_incremental_t
+	_fields_ = [('state', c_void_p), ('nodes', c_void_p), ('state_bytes', c_i64), ('capacity', c_i64), ('base', c_i64), ('t0', c_i64),
+				('commit', c_i32), ('shift', c_i32), ('frames', c_i32), ('is_eos', c_i32), ('finished', c_i32), ('reserved', c_i32)]
+
+
 ACT_NONE, ACT_RELU, ACT_HARDTANH, ACT_LEAKY_RELU = 0, 1, 2, 3
 EPI_ACT_BF16, EPI_LOGSOFTMAX, EPI_LOGITS_F32, EPI_LOGITS_ROWS = 0, 1, 2, 3
 MAX_CONV_SOURCES = 18
@@ -147,9 +152,14 @@ SIGNATURES = {
 	'cab_ctc_beam_search_stream': [c_void_p, c_i64, c_i64, c_i64, ctypes.POINTER(BeamStreamRow), c_int, c_int, c_int, c_int, c_float, c_int, c_int,
 									c_int, c_void_p, c_i64, c_void_p, c_void_p, c_int, c_void_p, c_void_p, ctypes.POINTER(NgramLM), c_float, c_float,
 									c_int, c_void_p],
+	'cab_ctc_beam_search_stream_incremental_workspace': [c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(c_i64)],
+	'cab_ctc_beam_search_stream_incremental': [c_void_p, c_i64, c_i64, c_i64, ctypes.POINTER(BeamStreamIncrementalRow), c_int, c_int, c_int, c_int,
+												c_float, c_int, c_int, c_int, c_void_p, c_i64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+												c_int, c_void_p, c_void_p, ctypes.POINTER(NgramLM), c_float, c_float, c_int, c_void_p],
 }
 HOST_ONLY = {'cab_bn_bwd_apply_covers', 'cab_ctc_alignment_long_workspace', 'cab_ctc_loss_one_cta_covers', 'cab_ctc_loss_long_workspace',
-			'cab_ctc_beam_search_workspace', 'cab_ctc_beam_search_stream_state_bytes', 'cab_ctc_beam_search_stream_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
+			'cab_ctc_beam_search_workspace', 'cab_ctc_beam_search_stream_state_bytes', 'cab_ctc_beam_search_stream_workspace',
+			'cab_ctc_beam_search_stream_incremental_workspace'}  # queries that launch nothing (left out of the per-entry-point device timing)
 INTROSPECTION = {'cab_abi_version': c_int, 'cab_last_error': ctypes.c_char_p, 'cab_launch_count': c_i64}
 
 

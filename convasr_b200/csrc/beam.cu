@@ -17,6 +17,7 @@
 #include "../../include/convasr_b200.h"
 #include <atomic>
 #include <cmath>
+#include <vector>
 
 namespace cab {
 extern std::atomic<int64_t> g_launch_count;
@@ -373,17 +374,20 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
     const int64_t len64 = lengths ? lengths[b] : T;
     int len = len64 < 0 ? 0 : (len64 > T ? T : (int)len64);
     int t0 = 0;
+    bool fresh = true;
     BeamStreamState ss;
     if constexpr (STREAM) {
         const cab_beam_stream_t row = rows[b];
         beam_state_layout(static_cast<unsigned char*>(row.state), W, LM ? lm.order : 0, &ss);
         t0 = ss.hdr[0];
-        nb = t0 > 0 ? ss.hdr[1] : 1;
+        // hdr[3] != 0: the block holds a live beam set whatever t0 is (an incremental stream's t0 counts from its window)
+        fresh = t0 == 0 && ss.hdr[3] == 0;
+        nb = fresh ? 1 : ss.hdr[1];
         // the caller checked t0 + frames against the capacity; the clamp only keeps a state out of step in bounds
         const int64_t room = row.capacity - t0;
         len = row.frames < 0 ? 0 : (row.frames > T ? T : row.frames);
         if (len > room) len = room < 0 ? 0 : (int)room;
-        if (t0 > 0 && tid < nb) {
+        if (!fresh && tid < nb) {
             s_hash[tid] = ss.hash[tid]; s_phash[tid] = ss.phash[tid]; s_pb[tid] = ss.pb[tid]; s_pnb[tid] = ss.pnb[tid];
             s_last[tid] = ss.last[tid]; s_node[tid] = ss.node[tid]; s_prank[tid] = ss.prank[tid];
             if constexpr (LM) {
@@ -393,7 +397,7 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
             }
         }
     }
-    if (tid == 0 && t0 == 0) {
+    if (tid == 0 && fresh) {
         s_hash[0] = 0; s_phash[0] = 0; s_pb[0] = 0.f; s_pnb[0] = -INFINITY; s_last[0] = -1; s_node[0] = -1; s_prank[0] = -1;
         if constexpr (LM) {
             s_tnode[0] = 0;
@@ -654,8 +658,7 @@ beam_search_kernel(const int* __restrict__ p_cls, const float* __restrict__ p_lp
         if (tid == 0) {
             ss.hdr[0] = t0 + len;
             ss.hdr[1] = nb;
-            ss.hdr[2] = rows[b].is_eos != 0;
-            ss.hdr[3] = 0;
+            ss.hdr[2] = rows[b].is_eos != 0;  // hdr[3] is left as it is: 0 for full-history streams
         }
     }
     if constexpr (LM) {
@@ -725,6 +728,117 @@ beam_backtrace_kernel(const BeamNode* __restrict__ nodes, const int* __restrict_
     out_lengths[o] = L;
 }
 
+// ------------------------------------------------------------------------------------------
+// Incremental streams (cab_ctc_beam_search_stream_incremental).  Node records are written once; a kept prefix keeps its
+// node; a new prefix's parent is the node of a beam live in the current frame.  So every later hypothesis descends from
+// one of the beams live after a call, and the deepest common ancestor of those beams, the commit node, and its chain
+// are final.  A call emits the chain between the previous and the new commit node as final tokens, and each hypothesis
+// only down to the commit node.  The node table holds a window of the stream: node ids and the state block's t0 count
+// from the window's first frame, whose absolute frame (`base`) the row carries.  Nothing below the commit node is read
+// again, so the caller may drop the frames before the commit node's frame from the window (`shift`).
+//   beam_rebase_kernel           before the search: moves frames [shift, t0) of the window to the front, parents
+//                                below the new window become -2 (never followed), node ids and t0 in the state block
+//                                are rebased
+//   beam_search_kernel<LM, true> unchanged; the block's hdr[3] != 0 marks a live beam set even at t0 == 0
+//   beam_commit_kernel           the new commit node and the final segment
+//   beam_tail_kernel             each hypothesis from its node down to the commit node
+// ------------------------------------------------------------------------------------------
+struct BeamIncrRow {      // device descriptor of an incremental row; window-relative ids and frames after the shift
+    BeamNode* nodes;
+    unsigned char* state;
+    int64_t base;         // absolute frame of the window's first frame
+    int t0;               // frames in the window before this call, before the shift
+    int shift;            // frames dropped from the window's front before the search
+    int commit;           // previous commit node, -1 = the root
+    int pad;
+};
+
+__global__ void __launch_bounds__(256)
+beam_rebase_kernel(const BeamIncrRow* __restrict__ rows, int W, int lm_order) {
+    const BeamIncrRow row = rows[blockIdx.x];
+    if (row.shift == 0) return;
+    const int lo = row.shift * W, n = (row.t0 - row.shift) * W;  // the caller checked t0 - shift <= shift: no overlap
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        BeamNode e = row.nodes[lo + i];
+        e.parent = e.parent >= lo ? e.parent - lo : -2;
+        row.nodes[i] = e;
+    }
+    BeamStreamState ss;
+    beam_state_layout(row.state, W, lm_order, &ss);
+    for (int i = threadIdx.x; i < ss.hdr[1]; i += blockDim.x) ss.node[i] = ss.node[i] >= lo ? ss.node[i] - lo : -2;
+    __syncthreads();
+    if (threadIdx.x == 0) ss.hdr[0] -= row.shift;
+}
+
+// one CTA per row, thread j < nb: LCA(beam 0, beam j) by walking the larger of two ids to its parent (ids decrease
+// strictly along a chain, so the larger one is not a common ancestor); the commit node is the smallest of these.  Only
+// nodes above the previous commit node are read.
+__global__ void __launch_bounds__(kBeamMaxW)
+beam_commit_kernel(const BeamIncrRow* __restrict__ rows, int W, int lm_order, int L_cap, int* __restrict__ out_tokens,
+                   int64_t* __restrict__ out_frames, int* __restrict__ out_lengths, int* __restrict__ out_commit) {
+    __shared__ int s_commit, s_len;
+    const int b = blockIdx.x, j = threadIdx.x;
+    const BeamIncrRow row = rows[b];
+    const BeamNode* bn = row.nodes;
+    BeamStreamState ss;
+    beam_state_layout(row.state, W, lm_order, &ss);
+    const int nb = ss.hdr[1], P = row.commit;
+    if (j == 0) s_commit = INT32_MAX;
+    __syncthreads();
+    if (j < nb) {
+        int x = ss.node[0], y = ss.node[j];
+        while (x != y && max(x, y) > P) {
+            if (x > y) x = bn[x].parent;
+            else y = bn[y].parent;
+        }
+        atomicMin(&s_commit, x == y ? max(x, P) : P);
+    }
+    __syncthreads();
+    const int cn = nb > 0 ? s_commit : P;
+    if (j == 0) {
+        int L = 0;
+        for (int id = cn; id > P; id = bn[id].parent) ++L;
+        int* tok = out_tokens + (size_t)b * L_cap;
+        int64_t* frm = out_frames + (size_t)b * L_cap;
+        int pos = L - 1;
+        for (int id = cn; id > P; id = bn[id].parent, --pos) {
+            if (pos < L_cap) { tok[pos] = bn[id].cls; frm[pos] = row.base + id / W; }
+        }
+        s_len = L;
+        out_lengths[b] = L;
+        out_commit[b] = cn;
+        if (ss.hdr[0] > 0) ss.hdr[3] = 1;
+    }
+    __syncthreads();
+    for (int i = s_len + j; i < L_cap; i += kBeamMaxW) {
+        out_tokens[(size_t)b * L_cap + i] = -1;
+        out_frames[(size_t)b * L_cap + i] = -1;
+    }
+}
+
+// beam_backtrace_kernel<true> stopping at the commit node: one thread per hypothesis, absolute frames
+__global__ void __launch_bounds__(kBeamMaxW)
+beam_tail_kernel(const BeamIncrRow* __restrict__ rows, const int* __restrict__ commit, const int* __restrict__ final_node, int W,
+                 int K, int L_cap, int* __restrict__ out_tokens, int64_t* __restrict__ out_frames, int* __restrict__ out_lengths) {
+    const int b = blockIdx.x, r = threadIdx.x;
+    if (r >= K) return;
+    const BeamNode* bn = rows[b].nodes;
+    const int64_t base = rows[b].base;
+    const int cn = commit[b];
+    const size_t o = (size_t)b * K + r;
+    const int start = final_node[o];
+    int L = 0;
+    for (int id = start; id > cn; id = bn[id].parent) ++L;
+    int* tok = out_tokens + o * L_cap;
+    int64_t* frm = out_frames + o * L_cap;
+    int pos = L - 1;
+    for (int id = start; id > cn; id = bn[id].parent, --pos) {
+        if (pos < L_cap) { tok[pos] = bn[id].cls; frm[pos] = base + id / W; }
+    }
+    for (int i = L; i < L_cap; ++i) { tok[i] = -1; frm[i] = -1; }
+    out_lengths[o] = L;
+}
+
 static size_t beam_align(size_t x) { return (x + 255) & ~(size_t)255; }
 
 // workspace: pruned classes int32 [B, T, N], their log-probs fp32 [B, T, N], counts int32 [B, T], node table
@@ -767,12 +881,12 @@ static size_t beam_search_smem(int W, int N, bool lm) {
 }
 
 // prune -> search -> back-trace; the arguments are checked by the caller.  STREAM: `rows` are the host descriptors,
-// copied into the workspace before the launches
+// copied into the workspace before the launches.  backtrace = false (incremental streams): prune and search only
 template <bool LM, bool STREAM = false>
 static int beam_search_launch(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t, const int64_t* output_lengths,
                               int B, int T, int C, int N, float cutoff_prob, int blank, int W, int K, void* workspace, int32_t* out_tokens,
                               int32_t* out_frames, int L_cap, int32_t* out_lengths, float* out_scores, const BeamLm& lm,
-                              cudaStream_t stream, const cab_beam_stream_t* rows = nullptr) {
+                              cudaStream_t stream, const cab_beam_stream_t* rows = nullptr, bool backtrace = true) {
     size_t off[5];
     unsigned char* ws = static_cast<unsigned char*>(workspace);
     BeamNode* nodes = nullptr;
@@ -810,6 +924,7 @@ static int beam_search_launch(const float* log_probs, int64_t stride_b, int64_t 
                                                                       final_node, out_scores, lm, d_rows);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    if (!backtrace) return 0;
     beam_backtrace_kernel<STREAM><<<B, kBeamMaxW, 0, stream>>>(nodes, final_node, T, W, K, L_cap, out_tokens, out_frames, out_lengths,
                                                                 d_rows);
     CAB_CHECK_LAUNCH();
@@ -957,4 +1072,107 @@ extern "C" int cab_ctc_beam_search_stream(const float* log_probs, int64_t stride
     return beam_search_launch<false, true>(log_probs, stride_b, stride_c, stride_t, nullptr, B, T, C, N, cutoff_prob, blank, W, K,
                                            workspace, out_tokens, out_frames, L_cap, out_lengths, out_scores, v,
                                            static_cast<cudaStream_t>(stream_), rows);
+}
+
+// incremental workspace: the streaming workspace, then the rows' BeamIncrRow descriptors
+static size_t beam_incr_workspace_bytes(int B, int T, int N, int K) {
+    return beam_stream_workspace_bytes(B, T, N, K) + beam_align((size_t)B * sizeof(BeamIncrRow));
+}
+
+extern "C" int cab_ctc_beam_search_stream_incremental_workspace(int B, int T, int N, int W, int K, int64_t* bytes) {
+    CAB_CHECK_ARG(bytes != nullptr, "null output");
+    CAB_CHECK_ARG(B > 0 && T >= 0, "bad shape B=%d T=%d", B, T);
+    CAB_CHECK_ARG(W >= 1 && W <= kBeamMaxW, "beam_width=%d out of [1, %d]", W, kBeamMaxW);
+    CAB_CHECK_ARG(N >= 1 && N <= kBeamMaxN, "N=%d out of [1, %d]", N, kBeamMaxN);
+    CAB_CHECK_ARG(K >= 1 && K <= W, "K=%d out of [1, beam_width=%d]", K, W);
+    *bytes = (int64_t)beam_incr_workspace_bytes(B, T, N, K);
+    return 0;
+}
+
+extern "C" int cab_ctc_beam_search_stream_incremental(const float* log_probs, int64_t stride_b, int64_t stride_c, int64_t stride_t,
+                                                      const cab_beam_stream_incremental_t* rows, int B, int T, int C, int N,
+                                                      float cutoff_prob, int blank, int W, int K, void* workspace, int64_t workspace_bytes,
+                                                      int32_t* out_final_tokens, int64_t* out_final_frames, int32_t* out_final_lengths,
+                                                      int32_t* out_commit, int32_t* out_tokens, int64_t* out_frames, int L_cap,
+                                                      int32_t* out_lengths, float* out_scores, const cab_ngram_lm_t* lm, float alpha,
+                                                      float beta, int space, cab_stream_t stream_) {
+    CAB_CHECK_ARG(rows && workspace && out_final_tokens && out_final_frames && out_final_lengths && out_commit && out_tokens && out_frames &&
+                  out_lengths && out_scores, "null pointer argument");
+    CAB_CHECK_ARG(B > 0 && T >= 0 && C > 0, "bad shape B=%d T=%d C=%d", B, T, C);
+    CAB_CHECK_ARG(T == 0 || log_probs, "null log_probs");
+    CAB_CHECK_ARG(W >= 1 && W <= kBeamMaxW, "beam_width=%d out of [1, %d]", W, kBeamMaxW);
+    CAB_CHECK_ARG(N >= 1 && N <= kBeamMaxN && N <= C, "N=%d out of [1, %d] (C=%d)", N, kBeamMaxN, C);
+    CAB_CHECK_ARG(K >= 1 && K <= W, "K=%d out of [1, beam_width=%d]", K, W);
+    CAB_CHECK_ARG(blank >= 0 && blank < C, "blank=%d out of range (C=%d)", blank, C);
+    CAB_CHECK_ARG(cutoff_prob > 0.f && cutoff_prob <= 1.f, "cutoff_prob=%g out of (0, 1]", (double)cutoff_prob);
+    CAB_CHECK_ARG(L_cap >= 1, "L_cap=%d must be positive", L_cap);
+    CAB_CHECK_ARG(workspace_bytes >= (int64_t)beam_incr_workspace_bytes(B, T, N, K), "workspace of %lld bytes is too small (%lld needed)",
+                  (long long)workspace_bytes, (long long)beam_incr_workspace_bytes(B, T, N, K));
+    BeamLm v{};
+    if (lm) {
+        const int rc = beam_lm_view(lm, C, blank, alpha, beta, space, &v);
+        if (rc != 0) return rc;
+    }
+    const int lm_order = lm ? lm->order : 0;
+    const int64_t need_state = (int64_t)beam_state_layout(nullptr, W, lm_order, nullptr);
+    bool any_shift = false;
+    for (int b = 0; b < B; ++b) {
+        const cab_beam_stream_incremental_t& r = rows[b];
+        CAB_CHECK_ARG(r.state && r.nodes, "row %d: null state or node table", b);
+        CAB_CHECK_ARG(r.state_bytes >= need_state, "row %d: state block of %lld bytes, %lld needed", b, (long long)r.state_bytes,
+                      (long long)need_state);
+        CAB_CHECK_ARG(!r.finished, "row %d: the stream has ended (an earlier call had is_eos)", b);
+        CAB_CHECK_ARG(r.frames >= 0 && r.frames <= T, "row %d: frames=%d out of [0, T=%d]", b, r.frames, T);
+        CAB_CHECK_ARG(r.capacity >= 0 && r.capacity <= INT32_MAX / W, "row %d: node table capacity %lld frames out of [0, %d]", b,
+                      (long long)r.capacity, INT32_MAX / W);
+        CAB_CHECK_ARG(r.base >= 0, "row %d: window base frame %lld negative", b, (long long)r.base);
+        CAB_CHECK_ARG(r.t0 >= 0 && r.t0 <= r.capacity, "row %d: t0=%lld overruns the node table (%lld frames)", b, (long long)r.t0,
+                      (long long)r.capacity);
+        CAB_CHECK_ARG(r.commit >= -1 && (int64_t)r.commit < r.t0 * W, "row %d: commit node %d out of [-1, t0 * W = %lld)", b, r.commit,
+                      (long long)(r.t0 * W));
+        const int64_t cf = r.commit >= 0 ? r.commit / W : 0;  // frames the window may drop: those before the commit node's
+        CAB_CHECK_ARG(r.shift >= 0 && r.shift <= cf && (r.shift == 0 || r.t0 - r.shift <= r.shift),
+                      "row %d: shift=%d out of [0, %lld] (the commit node's frame) or below t0 - shift = %lld (the moved frames overlap)", b,
+                      r.shift, (long long)cf, (long long)(r.t0 - r.shift));
+        const int64_t t0 = r.t0 - r.shift;
+        CAB_CHECK_ARG(t0 + r.frames <= r.capacity, "row %d: t0=%lld (after the shift) + frames=%d overruns the node table (%lld frames)", b,
+                      (long long)t0, r.frames, (long long)r.capacity);
+        const int64_t open = t0 + r.frames - (r.commit >= 0 ? cf - r.shift + 1 : 0);  // frames after the commit node's
+        CAB_CHECK_ARG(L_cap >= open, "row %d: L_cap=%d below the %lld frames after the commit node", b, L_cap, (long long)open);
+        for (int c = 0; c < b; ++c) CAB_CHECK_ARG(rows[c].state != r.state, "rows %d and %d share a state block", c, b);
+        any_shift |= r.shift > 0;
+    }
+    std::vector<cab_beam_stream_t> srows(B);
+    std::vector<BeamIncrRow> irows(B);
+    for (int b = 0; b < B; ++b) {
+        const cab_beam_stream_incremental_t& r = rows[b];
+        srows[b] = cab_beam_stream_t{r.state, r.nodes, r.state_bytes, r.capacity, r.t0 - r.shift, r.frames, r.is_eos, 0, 0};
+        irows[b] = BeamIncrRow{static_cast<BeamNode*>(r.nodes), static_cast<unsigned char*>(r.state), r.base + r.shift, (int)r.t0, r.shift,
+                               r.commit >= 0 ? r.commit - r.shift * W : -1, 0};
+    }
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    unsigned char* ws = static_cast<unsigned char*>(workspace);
+    BeamIncrRow* d_irows = reinterpret_cast<BeamIncrRow*>(ws + beam_stream_workspace_bytes(B, T, N, K));
+    CAB_CHECK_CUDA(cudaMemcpyAsync(d_irows, irows.data(), (size_t)B * sizeof(BeamIncrRow), cudaMemcpyHostToDevice, stream));
+    if (any_shift) {
+        beam_rebase_kernel<<<B, 256, 0, stream>>>(d_irows, W, lm_order);
+        CAB_CHECK_LAUNCH();
+        g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    }
+    const int rc = lm ? beam_search_launch<true, true>(log_probs, stride_b, stride_c, stride_t, nullptr, B, T, C, N, cutoff_prob, blank, W, K,
+                                                       workspace, nullptr, nullptr, L_cap, nullptr, out_scores, v, stream, srows.data(), false)
+                      : beam_search_launch<false, true>(log_probs, stride_b, stride_c, stride_t, nullptr, B, T, C, N, cutoff_prob, blank, W, K,
+                                                        workspace, nullptr, nullptr, L_cap, nullptr, out_scores, v, stream, srows.data(), false);
+    if (rc != 0) return rc;
+    size_t off[5];
+    beam_stream_workspace_layout(B, T, N, K, off);
+    const int* final_node = reinterpret_cast<const int*>(ws + off[3]);
+    beam_commit_kernel<<<B, kBeamMaxW, 0, stream>>>(d_irows, W, lm_order, L_cap, out_final_tokens, out_final_frames, out_final_lengths,
+                                                    out_commit);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    beam_tail_kernel<<<B, kBeamMaxW, 0, stream>>>(d_irows, out_commit, final_node, W, K, L_cap, out_tokens, out_frames, out_lengths);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
 }

@@ -5,7 +5,8 @@ collapse (that lives in transcript_generators.GreedyCTCGenerator).  K=1 is the f
 (ties -> lowest id, as torch.argmax); K>1 is the native top-K kernel (K <= 8).
 BeamSearchDecoder: CTC prefix beam search on the GPU (csrc/beam.cu), acoustic only or fused with a word n-gram LM read
 from an ARPA file (convasr_b200/lm.py); KenLM's binary format is not read.
-OnlineBeamSearchDecoder: the same search resumed chunk by chunk, one state per stream.
+OnlineBeamSearchDecoder: the same search resumed chunk by chunk, one state per stream; decode_incremental returns the
+tokens that became final and the tails after them, at a cost per call that does not grow with the stream.
 """
 import math
 
@@ -105,7 +106,8 @@ class OnlineBeamSearchDecoder(BeamSearchDecoder):
 	After the chunk containing frame t the result is bit for bit BeamSearchDecoder's on frames 0..t of the stream
 	(with an LM, the last word's term and the re-rank included).  Each call may batch any streams in any rows; a row's
 	`output_lengths` entry is its frame count in this call (0 allowed).  A state belongs to the decoder that made it;
-	after an is_eos call it is finished and feeding it again raises."""
+	after an is_eos call it is finished and feeding it again raises.  decode_incremental splits each result into the
+	tokens that became final and the tails after them, and its cost per call does not grow with the stream."""
 
 	def new_state(self, capacity = 1024):
 		"""a new stream; `capacity` is the node table's first size in frames (it grows by doubling)"""
@@ -118,14 +120,7 @@ class OnlineBeamSearchDecoder(BeamSearchDecoder):
 	def decode_nbest(self, log_probs, states, is_eos, output_lengths = None):
 		"""device tensors as BeamSearchDecoder.decode_nbest, [B, topk, L] tokens and frames with L the longest stream's
 		frames so far; frames count from the stream's start"""
-		if any(s.finished for s in states if isinstance(s, ops.BeamStreamState)):
-			raise RuntimeError('convasr_b200: a stream of this call has ended (is_eos was set on an earlier call); start a new state')
-		if log_probs.shape[1] != len(self.labels):
-			raise ValueError(f'convasr_b200: log_probs have {log_probs.shape[1]} classes, the decoder {len(self.labels)} labels')
-		config = self._config()
-		for b, s in enumerate(states):
-			if not isinstance(s, ops.BeamStreamState) or s.config != config:
-				raise ValueError(f'convasr_b200: the stream state of row {b} was not made by this decoder configuration (new_state())')
+		self._check_states(log_probs, states)
 		tokens, frames, lengths, scores = ops.ctc_beam_search_stream(
 			log_probs, states, is_eos, output_lengths, beam_width = self.beam_width, cutoff_top_n = self.cutoff_top_n,
 			cutoff_prob = self.cutoff_prob, topk = self.topk, blank = self.blank_id, lm = self.lm, alpha = self.beam_alpha, beta = self.beam_beta
@@ -136,3 +131,30 @@ class OnlineBeamSearchDecoder(BeamSearchDecoder):
 		"""token lists as BeamSearchDecoder.decode, for each row's stream so far"""
 		r = self.decode_nbest(log_probs, states, is_eos, output_lengths)
 		return self._token_lists(r)
+
+	def decode_incremental(self, log_probs, states, is_eos, output_lengths = None):
+		"""The same search at a cost per call that does not grow with the stream (ops.ctc_beam_search_stream_incremental):
+		per row, (the tokens that became final in this call, [the tail after everything final so far, per hypothesis the
+		search kept, best first]).  All final lists of a stream concatenated, followed by tail k, are hypothesis k of
+		decode() on the same frames; final tokens are never retracted.  A state's first incremental call binds it to
+		decode_incremental for life; decode / decode_nbest refuse it afterwards."""
+		self._check_states(log_probs, states)
+		ft, _, fl, tokens, _, lengths, scores = ops.ctc_beam_search_stream_incremental(
+			log_probs, states, is_eos, output_lengths, beam_width = self.beam_width, cutoff_top_n = self.cutoff_top_n,
+			cutoff_prob = self.cutoff_prob, topk = self.topk, blank = self.blank_id, lm = self.lm, alpha = self.beam_alpha, beta = self.beam_beta
+		)
+		fl, lengths, scores = fl.cpu().tolist(), lengths.cpu().tolist(), scores.cpu().tolist()
+		n_max = max([max(l) for l in lengths], default = 0)
+		ft, tokens = ft[:, :max(fl, default = 0)].cpu().tolist(), tokens[:, :, :n_max].cpu().tolist()
+		return [(f[:n], [tok[:l] for tok, l, s in zip(tb, lb, sb) if s > -math.inf])
+				for f, n, tb, lb, sb in zip(ft, fl, tokens, lengths, scores)]
+
+	def _check_states(self, log_probs, states):
+		if any(s.finished for s in states if isinstance(s, ops.BeamStreamState)):
+			raise RuntimeError('convasr_b200: a stream of this call has ended (is_eos was set on an earlier call); start a new state')
+		if log_probs.shape[1] != len(self.labels):
+			raise ValueError(f'convasr_b200: log_probs have {log_probs.shape[1]} classes, the decoder {len(self.labels)} labels')
+		config = self._config()
+		for b, s in enumerate(states):
+			if not isinstance(s, ops.BeamStreamState) or s.config != config:
+				raise ValueError(f'convasr_b200: the stream state of row {b} was not made by this decoder configuration (new_state())')

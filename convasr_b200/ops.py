@@ -488,6 +488,11 @@ class BeamStreamState:
 		self.initial_capacity = max(1, int(capacity))
 		self.state = None  # uint8 device tensor, zeroed: a fresh stream
 		self.nodes = None  # int32 device tensor [capacity, W, 2]
+		# ctc_beam_search_stream_incremental: the node table is a window of the stream starting at absolute frame `base`;
+		# t0 and `commit` (the commit node's id, -1 = the root) count from it
+		self.incremental = False
+		self.base = 0
+		self.commit = -1
 
 	@property
 	def capacity(self):
@@ -504,6 +509,23 @@ class BeamStreamState:
 				nodes[:self.t0].copy_(self.nodes[:self.t0])
 			self.nodes = nodes
 
+	def _window(self, frames, W, state_bytes, dev):
+		"""incremental calls: the frames to drop from the window's front before this call (those before the commit node's
+		frame, once that frame is at least half the capacity: the moved frames then do not overlap their destination), and
+		a node table that holds the rest plus this call's frames, grown by doubling only when that outgrows it"""
+		cf = self.commit // W if self.commit >= 0 else 0
+		shift = cf if cf > 0 and 2 * cf >= self.capacity else 0
+		if self.state is None:
+			self.state = torch.zeros(state_bytes, dtype = torch.uint8, device = dev)
+		need = self.t0 - shift + frames
+		if self.nodes is None or need > self.capacity:
+			cap = max(need, 2 * self.capacity, self.initial_capacity)
+			nodes = torch.empty(cap, W, 2, dtype = torch.int32, device = dev)
+			if self.t0 > 0:
+				nodes[:self.t0].copy_(self.nodes[:self.t0])  # unshifted: the call moves them
+			self.nodes = nodes
+		return shift
+
 
 def beam_stream_state_bytes(beam_width, lm_order = 0):
 	"""bytes of one stream's state block (host-only query)"""
@@ -512,19 +534,19 @@ def beam_stream_state_bytes(beam_width, lm_order = 0):
 	return n.value
 
 
-def ctc_beam_search_stream(log_probs, states, is_eos, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0, topk = 1,
-							blank = None, lm = None, alpha = 0.0, beta = 0.0):
-	"""Streaming CTC prefix beam search: row b of fp32 [B, C, T] log_probs (any strides) holds the next output_lengths[b]
-	frames (None: T; 0 is allowed) of the stream states[b] (BeamStreamState, one per row, each at most once).  is_eos:
-	a bool, or one per row: that row's stream ends with this call.  Returns ctc_beam_search's tensors with [B, topk, L]
-	tokens and frames, L the longest stream's frames so far: the stream's current n-best list, frames counted from its
-	start, bit for bit what ctc_beam_search returns for the stream's frames so far with the same arguments (with an LM,
-	the last word's term and the re-rank included).  A finished stream, or a state bound to another configuration, is
-	refused."""
+def _stream_args(log_probs, states, is_eos, output_lengths, beam_width, cutoff_top_n, cutoff_prob, topk, blank, lm, alpha, beta, incremental):
+	"""the checks and per-row arguments both streaming calls share"""
 	states = list(states)
 	for b, s in enumerate(states):
 		if s.finished:
 			raise RuntimeError(f'convasr_b200: the stream of row {b} has ended (is_eos was set on an earlier call); start a new state')
+		if s.incremental and not incremental:
+			raise RuntimeError(f'convasr_b200: the stream state of row {b} is fed by incremental calls (ctc_beam_search_stream_incremental): its node '
+								'table holds only the frames after the commit node, not the history a full-history call back-traces; keep using '
+								'incremental calls, or start a new state')
+		if incremental and not s.incremental and s.search is not None:
+			raise RuntimeError(f'convasr_b200: the stream state of row {b} is fed by full-history calls (ctc_beam_search_stream); an incremental '
+								'call needs a state that only incremental calls have fed; start a new state')
 	B, C, T = log_probs.shape
 	if len(states) != B:
 		raise ValueError(f'convasr_b200: {len(states)} stream states for a batch of {B}')
@@ -547,6 +569,20 @@ def ctc_beam_search_stream(log_probs, states, is_eos, output_lengths = None, bea
 			raise ValueError(f'convasr_b200: the stream state of row {b} belongs to another search configuration ({s.search} != {search})')
 	_need_cuda(log_probs)
 	lp = log_probs if log_probs.dtype == torch.float32 else log_probs.float()
+	return states, lp, B, C, T, eos, frames, blank, N, W, K, search
+
+
+def ctc_beam_search_stream(log_probs, states, is_eos, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0, topk = 1,
+							blank = None, lm = None, alpha = 0.0, beta = 0.0):
+	"""Streaming CTC prefix beam search: row b of fp32 [B, C, T] log_probs (any strides) holds the next output_lengths[b]
+	frames (None: T; 0 is allowed) of the stream states[b] (BeamStreamState, one per row, each at most once).  is_eos:
+	a bool, or one per row: that row's stream ends with this call.  Returns ctc_beam_search's tensors with [B, topk, L]
+	tokens and frames, L the longest stream's frames so far: the stream's current n-best list, frames counted from its
+	start, bit for bit what ctc_beam_search returns for the stream's frames so far with the same arguments (with an LM,
+	the last word's term and the re-rank included).  A finished stream, a state bound to another configuration, or one
+	fed by ctc_beam_search_stream_incremental is refused."""
+	states, lp, B, C, T, eos, frames, blank, N, W, K, search = _stream_args(log_probs, states, is_eos, output_lengths, beam_width, cutoff_top_n,
+																			cutoff_prob, topk, blank, lm, alpha, beta, incremental = False)
 	dev = lp.device
 	if B == 0:
 		z = torch.empty(0, K, 0, dtype = torch.int32, device = dev)
@@ -579,6 +615,72 @@ def ctc_beam_search_stream(log_probs, states, is_eos, output_lengths = None, bea
 		s.t0 += n
 		s.finished = e
 	return tokens, frames_out, lengths, scores
+
+
+def ctc_beam_search_stream_incremental(log_probs, states, is_eos, output_lengths = None, beam_width = 100, cutoff_top_n = 40, cutoff_prob = 1.0,
+										topk = 1, blank = None, lm = None, alpha = 0.0, beta = 0.0):
+	"""ctc_beam_search_stream (same arguments and search) at a cost per call that does not grow with the stream.
+
+	Every later hypothesis of a stream descends from one of the beams live after a call, so their deepest common
+	ancestor (the commit node) and its labels are final.  Returns device tensors
+	  final_tokens int32 / final_frames int64 [B, F], final_lengths int32 [B]: the labels that became final in this call
+	    and their absolute emission frames (counted from the stream's start), -1 past each length;
+	  tokens int32 / frames int64 [B, topk, L], lengths int32 [B, topk], scores fp32 [B, topk]: the n-best continuations
+	    after everything final so far (the tails), scores as ctc_beam_search_stream's.
+	For each hypothesis k the search kept (score > -inf), the final segments of all calls so far concatenated, followed
+	by tail k, are bit for bit hypothesis k of ctc_beam_search on the stream's frames so far, in tokens, frames, length
+	and score, with and without an LM.  Final tokens are never retracted; a hypothesis the search did not keep has score
+	-inf and a tail of length 0.  F and L are bounded by the frames since the commit node, not by the stream.
+
+	Each state's node table is a window that starts at most at the commit node's frame: it is rebased on the device when
+	the commit node's frame passes half its capacity and grows by doubling only when the frames since the commit node
+	outgrow it.  Where the beams do not converge the window grows as the full-history table does.  The call copies the
+	B new commit nodes to the host (one synchronisation).  A state's first incremental call binds it to incremental
+	calls for life; a state fed by ctc_beam_search_stream, a finished one, or one bound to another configuration is
+	refused."""
+	states, lp, B, C, T, eos, frames, blank, N, W, K, search = _stream_args(log_probs, states, is_eos, output_lengths, beam_width, cutoff_top_n,
+																			cutoff_prob, topk, blank, lm, alpha, beta, incremental = True)
+	dev = lp.device
+	if B == 0:
+		z = torch.empty(0, 0, dtype = torch.int32, device = dev)
+		t = torch.empty(0, K, 0, dtype = torch.int32, device = dev)
+		return (z, z.long(), torch.empty(0, dtype = torch.int32, device = dev), t, t.long(), torch.empty(0, K, dtype = torch.int32, device = dev),
+				torch.empty(0, K, device = dev))
+	lib = _lib.load()
+	state_bytes = beam_stream_state_bytes(W, 0 if lm is None else lm.order)
+	shifts = [s._window(n, W, state_bytes, dev) for s, n in zip(states, frames)]
+	rows = (_lib.BeamStreamIncrementalRow * B)()
+	L_cap = 1
+	for r, s, n, e, sh in zip(rows, states, frames, eos, shifts):
+		r.state, r.nodes, r.state_bytes, r.capacity = s.state.data_ptr(), s.nodes.data_ptr(), s.state.numel(), s.capacity
+		r.base, r.t0, r.commit, r.shift, r.frames, r.is_eos, r.finished = s.base, s.t0, s.commit, sh, n, int(e), int(s.finished)
+		L_cap = max(L_cap, s.t0 - sh + n - (s.commit // W - sh + 1 if s.commit >= 0 else 0))
+	nbytes = ctypes.c_int64()
+	_lib.check(lib.cab_ctc_beam_search_stream_incremental_workspace(B, T, N, W, K, ctypes.byref(nbytes)), 'cab_ctc_beam_search_stream_incremental_workspace')
+	ws = torch.empty(nbytes.value, dtype = torch.uint8, device = dev)
+	final_tokens = torch.empty(B, L_cap, dtype = torch.int32, device = dev)
+	final_frames = torch.empty(B, L_cap, dtype = torch.int64, device = dev)
+	final_lengths = torch.empty(B, dtype = torch.int32, device = dev)
+	commit = torch.empty(B, dtype = torch.int32, device = dev)
+	tokens = torch.empty(B, K, L_cap, dtype = torch.int32, device = dev)
+	frames_out = torch.empty(B, K, L_cap, dtype = torch.int64, device = dev)
+	lengths = torch.empty(B, K, dtype = torch.int32, device = dev)
+	scores = torch.empty(B, K, dtype = torch.float32, device = dev)
+	lm_arg = None if lm is None else ctypes.byref(lm.device_struct(dev))
+	space = 0 if lm is None else lm.space
+	rc = lib.cab_ctc_beam_search_stream_incremental(
+		_p(lp) if T > 0 else None, lp.stride(0), lp.stride(1), lp.stride(2), rows, B, T, C, N, float(cutoff_prob), blank, W, K, _p(ws), nbytes.value,
+		_p(final_tokens), _p(final_frames), _p(final_lengths), _p(commit), _p(tokens), _p(frames_out), L_cap, _p(lengths), _p(scores), lm_arg,
+		float(alpha), float(beta), space, _stream()
+	)
+	_lib.check(rc, 'cab_ctc_beam_search_stream_incremental')
+	for s, n, e, sh, c in zip(states, frames, eos, shifts, commit.tolist()):
+		s.search, s.incremental = search, True
+		s.base += sh
+		s.t0 += n - sh
+		s.commit = c
+		s.finished = e
+	return final_tokens, final_frames, final_lengths, tokens, frames_out, lengths, scores
 
 
 def entropy(log_probs, lengths = None, eps_id = -1):

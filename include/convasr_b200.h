@@ -610,6 +610,61 @@ int cab_ctc_beam_search_stream(const float* log_probs, int64_t stride_b, int64_t
                                float* out_scores, const cab_ngram_lm_t* lm, float alpha, float beta, int space,
                                cab_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Incremental streaming search: the same search and state block as cab_ctc_beam_search_stream,
+ *   with a per-call cost that does not grow with the stream.  Every later hypothesis of a stream
+ *   descends from one of the beams live after a call, so the deepest common ancestor of those
+ *   beams (the commit node) and the labels on its chain are final.  Each call writes the part
+ *   of that chain between the previous and the new commit node (out_final_*: int32 tokens and
+ *   int64 absolute emission frames [B, L_cap], -1 past out_final_lengths [B]) and each
+ *   hypothesis only from the commit node on (out_tokens int32 / out_frames int64
+ *   [B, K, L_cap], out_lengths, out_scores as cab_ctc_beam_search_stream).  The final
+ *   segments of a stream concatenated, followed by tail k, are bit for bit hypothesis k of
+ *   cab_ctc_beam_search (_lm) on the stream's frames so far, where that hypothesis has
+ *   nonzero probability; final tokens are never retracted.  out_commit [B] (device): the new
+ *   commit node, window-relative after the shift, -1 the root.
+ *   Node table: a window of the stream.  Node ids and the block's t0 count from the window's
+ *   first frame, at absolute frame `base`.  `shift` > 0 drops the window's first `shift`
+ *   frames before the search (one more launch): frames [shift, t0) move to the front, parents
+ *   before the window become -2 (below the commit node, never followed), node ids and t0 in
+ *   the state block are rebased.  The caller then keeps, for the next call, base += shift,
+ *   t0 += frames - shift, commit = out_commit, finished = is_eos; it grows a node table by
+ *   copying its first t0 frames into a larger one.  The state block's int32 hdr[3] becomes 1
+ *   once the stream has consumed a frame (a live beam set whatever t0 is); a block used here
+ *   is not passed to cab_ctc_beam_search_stream, whose node ids are absolute.
+ *   Refused before any launch, besides cab_ctc_beam_search_stream's checks (t0 counted in
+ *   the window): a negative base; commit outside [-1, t0 * W); shift outside [0, the commit
+ *   node's frame] or, when positive, below t0 - shift (the moved frames must not overlap
+ *   their destination); t0 - shift + frames above capacity; L_cap below the frames after
+ *   the commit node (t0 - shift + frames - (commit >= 0 ? commit / W - shift + 1 : 0)).
+ *   Four launches (prune, search, commit, tail back-trace), five with a shift.
+ * ------------------------------------------------------------------------------------- */
+typedef struct {
+    void* state;          /* device state block (cab_ctc_beam_search_stream_state_bytes) */
+    void* nodes;          /* device node table of the window, capacity * W entries of 8 bytes */
+    int64_t state_bytes;  /* bytes of the state block */
+    int64_t capacity;     /* frames the node table holds */
+    int64_t base;         /* absolute frame of the window's first frame, before the shift */
+    int64_t t0;           /* frames of the window consumed before this call, before the shift */
+    int32_t commit;       /* commit node after the previous call, before the shift; -1 = the root */
+    int32_t shift;        /* frames dropped from the window's front before this call, 0 = none */
+    int32_t frames;       /* frames of this call, [0, T] */
+    int32_t is_eos;       /* nonzero: this call ends the stream */
+    int32_t finished;     /* nonzero: an earlier call ended the stream (refused) */
+    int32_t reserved;
+} cab_beam_stream_incremental_t;
+
+int cab_ctc_beam_search_stream_incremental_workspace(int B, int T, int N, int W, int K, int64_t* bytes);
+int cab_ctc_beam_search_stream_incremental(const float* log_probs, int64_t stride_b, int64_t stride_c,
+                                           int64_t stride_t, const cab_beam_stream_incremental_t* rows,
+                                           int B, int T, int C, int N, float cutoff_prob, int blank, int W,
+                                           int K, void* workspace, int64_t workspace_bytes,
+                                           int32_t* out_final_tokens, int64_t* out_final_frames,
+                                           int32_t* out_final_lengths, int32_t* out_commit,
+                                           int32_t* out_tokens, int64_t* out_frames, int L_cap,
+                                           int32_t* out_lengths, float* out_scores, const cab_ngram_lm_t* lm,
+                                           float alpha, float beta, int space, cab_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
