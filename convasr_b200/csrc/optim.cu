@@ -4,7 +4,7 @@
 // Replaces (reference file:line): torch.nn.utils.clip_grad_norm_ at train.py:776-779,
 // optimizers.NovoGrad.step optimizers.py:72-90 (a Python loop with ~8 launches per tensor), and
 // torch.optim.SGD as configured at train.py:657-662.  HBM bound: every element of p, g, m is read
-// and p, m written exactly once (5 x 4 B per parameter per step); 128-bit accesses.
+// and p, m written exactly once (5 x 4 B per parameter per step); 128-bit accesses where the tensors are 16-byte aligned.
 //
 // Tensors are described by device tables (pointers, sizes) and a flat chunk list for load balance.
 #include "common.cuh"
@@ -27,7 +27,9 @@ mt_sumsq_kernel(const long long* __restrict__ grad_ptrs, const long long* __rest
     const float* g = reinterpret_cast<const float*>(grad_ptrs[ti]) + off;
     const long long n = min((long long)chunk_elems, numels[ti] - off);
     float acc = 0.f;
-    const long long n4 = n >> 2;
+    // 128-bit loads only from a 16-byte aligned base (chunk offsets are multiples of 4): a gradient may be a view at any
+    // float offset of a larger buffer
+    const long long n4 = (reinterpret_cast<uintptr_t>(g) & 15) == 0 ? n >> 2 : 0;
     const float4* g4 = reinterpret_cast<const float4*>(g);
     for (long long i = threadIdx.x; i < n4; i += kOptThreads) {
         const float4 v = g4[i];
@@ -133,7 +135,9 @@ mt_update_kernel(const long long* __restrict__ param_ptrs, const long long* __re
         }
         m_out = buf;
     };
-    const long long n4 = n >> 2;
+    // the float4 path needs all three bases 16-byte aligned; a tensor with any other offset takes the scalar loop
+    const bool vec = ((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(m)) & 15) == 0;
+    const long long n4 = vec ? n >> 2 : 0;
     float4* p4 = reinterpret_cast<float4*>(p);
     const float4* g4 = reinterpret_cast<const float4*>(g);
     float4* m4 = reinterpret_cast<float4*>(m);

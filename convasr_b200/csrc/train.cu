@@ -934,8 +934,13 @@ bn_multi_fwd_kernel(const MultiArgs m, int B, int T, int C, int ld, int act, flo
     }
 }
 
-// dz = g * act'(z) * mask * dropout with the gate read off the stored output: relu / leaky z > 0 <=> out > 0;
-// hardtanh a < z < b <=> a < out * (1 - p) < b (a kept element is act(z) / (1 - p)); dropped or masked elements get 0
+// dz = g * act'(z) * mask * dropout with the gate read off the stored output v = out * (1 - p) (a kept element is
+// act(z) / (1 - p), rounded to bf16 -- or to hi + lo in the split tier -- and scaled back in fp32); dropped or masked
+// elements get 0.  relu / leaky: z > 0 <=> v > 0 holds exactly (rounding and scaling keep the sign and zero).  hardtanh:
+// the gate is a < v < b, which is NOT the same as a < z < b next to a clamp bound -- a z within one rounding of the stored
+// value from a or b (bf16: z in [19.9375, 20) stores 20.0 for b = 20; split tier: ~2^-16 relative; wider with dropout,
+// whose 1 / (1 - p) and (1 - p) round) reads as clamped and gets gate 0 where autograd's z-gate gives 1, or the reverse.
+// Recomputing z would mean re-reading every branch; the tests pin this contract exactly.
 template <bool SPLIT>
 __global__ void __launch_bounds__(256)
 act_bwd_dz_kernel(const __nv_bfloat16* __restrict__ out, const __nv_bfloat16* __restrict__ out_lo,

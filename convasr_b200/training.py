@@ -373,13 +373,16 @@ class NativeStack(torch.autograd.Function):
 		sync = getattr(model, '_grad_sync', None)
 		# all the small gradients (decoder bias, BN gamma / beta, grouped conv bias) live in one flat buffer: one all-reduce
 		bn_list = [(rep, None) for rep in reps] + [(rep, k) for rep in reps for k, (_, c, _) in enumerate(rep.res) if c is not None]
-		small_n = c_ld + sum(2 * (rep.conv.C_out if k is None else rep.res[k][1].C_out) for rep, k in bn_list) + sum(rep.grouped.out_channels for rep in reps if rep.grouped is not None)
+		# every slice starts on a 16-byte boundary, so the optimizer reads these gradients with 128-bit accesses (dgamma, the
+		# second row of a [2, C] slice, is C floats in and stays aligned only when C is a multiple of 4)
+		r4 = lambda n: (n + 3) // 4 * 4
+		small_n = c_ld + sum(r4(2 * (rep.conv.C_out if k is None else rep.res[k][1].C_out)) for rep, k in bn_list) + sum(r4(rep.grouped.out_channels) for rep in reps if rep.grouped is not None)
 		small = torch.zeros(small_n, dtype = torch.float32, device = dev)
 		cursor = [c_ld]
 
 		def take(n):
 			v = small[cursor[0]:cursor[0] + n]
-			cursor[0] += n
+			cursor[0] += r4(n)
 			return v
 
 		max_c = max(rep.conv.C_out for rep in reps)
@@ -628,6 +631,14 @@ def forward_training(model, x, xlen):
 	reps = getattr(model, '_train_graph', None)
 	if reps is None:
 		reps = model._train_graph = _graph(model)
+	if split:
+		# the split-bf16 BatchNorm kernels exist only for the row pitches the streamed kernel covers (the bf16 tier has a row
+		# walker for the others): refuse before the step launches anything.  The pitch alone decides, any row count > 0 will do.
+		lib = _lib.load()
+		for rep in reps:
+			if lib.cab_bn_bwd_apply_covers(1, rep.conv.co_alloc, 1) != 1:
+				raise NotImplementedError(f'convasr_b200: training of this module tree is not built (BatchNorm width {rep.conv.C_out}: row pitch '
+										f'{rep.conv.co_alloc} has no split-bf16 BatchNorm kernel, the fp32 tier; set_precision(\'bf16\') trains it); there is no ATen / cuDNN fallback')
 	hi, lo, Fr, C = model._packed_features(x, xlen, split)
 	params = []
 	for rep in reps:
