@@ -82,6 +82,11 @@ SIGNATURES = {
 							c_void_p, c_void_p, c_float, c_float, c_int, c_float, c_void_p, c_void_p, c_void_p],
 	'cab_frontend_features': [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_float, c_int, c_float,
 								c_int, c_int, c_float, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+	'cab_frontend_features_fixed': [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_float,
+									c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p],
+	'cab_frontend_stream': [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_float,
+							c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p],
+	'cab_stream_copy': [c_void_p, c_int, c_i64, c_void_p],
 	'cab_instnorm_pack': [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_int, c_int, c_int, c_void_p, c_void_p,
 						c_void_p, c_void_p, c_void_p],
 	'cab_conv1d_fused': [ctypes.POINTER(ConvSource), c_int, ctypes.POINTER(ConvEpilogue), c_void_p],

@@ -10,7 +10,7 @@ import sys
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, 'csrc')
 LIB_PATH = os.path.join(PKG_DIR, 'libconvasr_b200.so')
-SOURCES = ['api.cu', 'frontend.cu', 'conv_gemm.cu', 'wgrad_gemm.cu', 'ctc.cu', 'train.cu', 'optim.cu', 'grouped_conv.cu', 'beam.cu']
+SOURCES = ['api.cu', 'frontend.cu', 'conv_gemm.cu', 'wgrad_gemm.cu', 'ctc.cu', 'train.cu', 'optim.cu', 'grouped_conv.cu', 'beam.cu', 'streaming.cu']
 HEADERS = ['common.cuh', os.path.join('..', '..', 'include', 'convasr_b200.h')]
 
 NVCC_FLAGS = [

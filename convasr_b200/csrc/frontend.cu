@@ -134,6 +134,12 @@ struct FrontendParams {
     int normalize;
 };
 
+// logmel16_kernel modes.  kComputedStats is the one-shot path with per-utterance abs-max and instance-norm statistics;
+// kFixedStats multiplies the signal by the caller's scale and emits no statistics; kStream is kFixedStats over per-stream
+// staged samples: row b holds samples [base, base + n_staged) of its stream and the CTA tiles start at frame f_first.
+enum { kComputedStats = 0, kFixedStats = 1, kStream = 2 };
+enum { kRowFirstFrame = 0, kRowFrames, kRowBase, kRowStaged, kRowReflect, kStreamRowInts };
+
 template <int LOG2N>
 __global__ void __launch_bounds__(kFrontendWarps * 32)
 logmel_kernel(const FrontendParams p) {
@@ -285,9 +291,12 @@ __device__ __forceinline__ void fft16(float2 (&v)[16]) {
 }
 __host__ __device__ constexpr int brev4(int p) { return ((p & 1) << 3) | ((p & 2) << 1) | ((p & 4) >> 1) | ((p & 8) >> 3); }
 
+template <int MODE>
 __global__ void __launch_bounds__(kF16Warps * 32)
 logmel16_kernel(const FrontendParams p, float* __restrict__ partials /* [B][tiles][n_mels][2] mean, M2, or null */, int stats_masked,
-                float* __restrict__ stats /* [B][n_mels][2] mean, sd */, unsigned int* __restrict__ done /* [B] zeroed */, float norm_eps) {
+                float* __restrict__ stats /* [B][n_mels][2] mean, sd */, unsigned int* __restrict__ done /* [B] zeroed */, float norm_eps,
+                const float* __restrict__ scale /* kFixedStats / kStream: the caller's signal scale [B] */,
+                const int32_t* __restrict__ stream_rows /* kStream: [B][kStreamRowInts] (cab_frontend_stream) */) {
     constexpr int N = 256;
     extern __shared__ __align__(16) unsigned char smem16[];
     const int n_samples = (kF16Frames - 1) * p.hop + p.win;      // pre-emphasised samples this CTA needs
@@ -302,12 +311,15 @@ logmel16_kernel(const FrontendParams p, float* __restrict__ partials /* [B][tile
     __shared__ uint64_t bar;
 
     const int b = blockIdx.y;
-    const int f0 = blockIdx.x * kF16Frames;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int esz = p.is_int16 ? 2 : 4;
-    const int start = f0 * p.hop + p.first_off;                  // sample index of s_e[0] (may be negative: reflect)
+    // kStream: sample indices below are relative to the row's first staged sample (base); frames with a negative start
+    // are only emitted while base == 0, so the reflected head is addressed exactly as in the one-shot row
+    const int32_t* srow = MODE == kStream ? stream_rows + b * kStreamRowInts : nullptr;
+    const int f0 = blockIdx.x * kF16Frames + (MODE == kStream ? srow[kRowFirstFrame] : 0);
+    const int start = f0 * p.hop + p.first_off - (MODE == kStream ? srow[kRowBase] : 0);  // sample index of s_e[0] (may be negative: reflect)
     // raw window [r0, r1): everything s_e needs, incl. the sample before (pre-emphasis) and the reflected head
-    const bool reflect = (p.nfft / 2) < p.T;
+    const bool reflect = MODE == kStream ? srow[kRowReflect] != 0 : (p.nfft / 2) < p.T;
     int r0 = start - 1, r1 = start + n_samples;
     if (start < 0) { r0 = 0; r1 = max(r1, -start + 1); }
     r0 = max(r0, 0); r1 = min(r1, p.T);
@@ -354,9 +366,10 @@ logmel16_kernel(const FrontendParams p, float* __restrict__ partials /* [B][tile
         tw[q] = w;
     }
     int n_valid = p.T;
-    if (p.xlen != nullptr) n_valid = min(p.T, frac_len(p.xlen[b], p.T));
+    if (MODE == kStream) n_valid = srow[kRowStaged];
+    else if (p.xlen != nullptr) n_valid = min(p.T, frac_len(p.xlen[b], p.T));
     float denom = 1.f;
-    if (p.normalize) denom = __fmul_rn(__fadd_rn(p.absmax[b], 1e-5f), p.denom_mult);
+    if (MODE == kComputedStats && p.normalize) denom = __fmul_rn(__fadd_rn(p.absmax[b], 1e-5f), p.denom_mult);
     if (bulk) mbar_wait(&bar, 0);
     auto raw = [&](int n) -> float {  // sample n of this row, n in [0, T)
         if (bulk) return p.is_int16 ? (float)reinterpret_cast<const short*>(s_raw)[n - c0] : reinterpret_cast<const float*>(s_raw)[n - c0];
@@ -365,7 +378,7 @@ logmel16_kernel(const FrontendParams p, float* __restrict__ partials /* [B][tile
     // pre-emphasised, masked, reflect-padded signal: e[n] = s[n] - preemph * s[n-1], s = x / denom (models.py:570-575).  The
     // division is a multiplication by the reciprocal here (<= 1 ulp from the reference's quotient, far inside the 2e-4
     // log-mel bar; two IEEE divisions per sample were a quarter of this kernel's instructions)
-    const float inv_denom = p.normalize ? __frcp_rn(denom) : 1.f;
+    const float inv_denom = MODE != kComputedStats ? scale[b] : p.normalize ? __frcp_rn(denom) : 1.f;
     // fast path (int16, bulk-staged, interior tile): 8 consecutive samples per thread from one 16-byte shared-memory load
     // plus the sample before; the group is aligned because start - c0 is a multiple of 8 there
     const bool fast = bulk && p.is_int16 && start >= 8 && ((start - c0) & 7) == 0 && p.preemph > 0.f;
@@ -463,18 +476,20 @@ logmel16_kernel(const FrontendParams p, float* __restrict__ partials /* [B][tile
     int F_valid = p.F;
     if (p.xlen != nullptr && stats_masked) F_valid = min(p.F, frac_len(p.xlen[b], p.F));
     const int n_here = max(0, min(kF16Frames, F_valid - f0));
-    // stores: a half-warp writes the 64 frames of one mel row (256 contiguous bytes)
+    // stores: a half-warp writes the 64 frames of one mel row (256 contiguous bytes); kStream rows start at their first new frame
     {
-        float* outb = p.out + size_t(b) * p.n_mels * p.F + f0;
+        const int fo = MODE == kStream ? blockIdx.x * kF16Frames : f0;
+        float* outb = p.out + size_t(b) * p.n_mels * p.F + fo;
         const int c4 = (tid & 15) * 4, r0_ = tid >> 4;
         for (int m = r0_; m < p.n_mels; m += (kF16Warps * 32) >> 4) {
             const float* rowv = s_out + m * (kF16Frames + 1) + c4;
             float* dst = outb + size_t(m) * p.F + c4;
 #pragma unroll
             for (int j = 0; j < 4; ++j)
-                if (f0 + c4 + j < p.F) dst[j] = rowv[j];
+                if (fo + c4 + j < p.F) dst[j] = rowv[j];
         }
     }
+    if constexpr (MODE != kComputedStats) return;
     // statistics: one thread per mel channel walks its row twice (exact two-pass mean / centred second moment)
     for (int mch = tid; partials != nullptr && mch < p.n_mels; mch += blockDim.x) {
         const float* rowv = s_out + mch * (kF16Frames + 1);
@@ -550,6 +565,9 @@ __global__ void instnorm_stats_kernel(const float* __restrict__ feat, const floa
     }
 }
 
+// FIXED: stats holds the caller's (mean, invstd) per (b, c) and the kernel multiplies by invstd; otherwise (mean, sd) as
+// computed by the statistics kernels, divided by
+template <bool FIXED>
 __global__ void __launch_bounds__(256)
 instnorm_pack_kernel(const float* __restrict__ feat, const float* __restrict__ xlen,
                      const float* __restrict__ stats, int B, int C, int F, int F_pad, int C_pad,
@@ -569,7 +587,8 @@ instnorm_pack_kernel(const float* __restrict__ feat, const float* __restrict__ x
             v = feat[(size_t(b) * C + c) * F + f];
             if (normalize) {
                 const float mean = stats[2 * (b * C + c)], sd = stats[2 * (b * C + c) + 1];
-                v = __fdiv_rn(v - mean, sd);
+                if constexpr (FIXED) v = __fmul_rn(v - mean, sd);
+                else v = __fdiv_rn(v - mean, sd);
             }
         }
         if (out_f32 != nullptr && c < C && f < F) out_f32[(size_t(b) * C + c) * F + f] = v;
@@ -626,16 +645,18 @@ static size_t fft16_smem_bytes(int win, int hop, int n_mels) {
            sizeof(float) * (size_t)n_mels * (kF16Frames + 1) + 16 + sizeof(float) * (size_t)(n_samples + 32);
 }
 
-static int launch_logmel16(const FrontendParams& p, float* partials, int stats_masked, float* stats, unsigned int* done, float norm_eps, cudaStream_t stream) {
+template <int MODE = kComputedStats>
+static int launch_logmel16(const FrontendParams& p, float* partials, int stats_masked, float* stats, unsigned int* done, float norm_eps, cudaStream_t stream,
+                           const float* scale = nullptr, const int32_t* stream_rows = nullptr) {
     const size_t smem = fft16_smem_bytes(p.win, p.hop, p.n_mels);
     CAB_CHECK_ARG(smem <= 200 * 1024, "frontend tile does not fit shared memory (win=%d hop=%d)", p.win, p.hop);
-    static size_t smem_set = 0;
+    static size_t smem_set = 0;  // one per mode
     if (smem > smem_set) {
-        CAB_CHECK_CUDA(cudaFuncSetAttribute(logmel16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CAB_CHECK_CUDA(cudaFuncSetAttribute(logmel16_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         smem_set = smem;
     }
     dim3 grid((p.F + kF16Frames - 1) / kF16Frames, p.B);
-    logmel16_kernel<<<grid, kF16Warps * 32, smem, stream>>>(p, partials, stats_masked, stats, done, norm_eps);
+    logmel16_kernel<MODE><<<grid, kF16Warps * 32, smem, stream>>>(p, partials, stats_masked, stats, done, norm_eps, scale, stream_rows);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     return 0;
@@ -751,11 +772,73 @@ extern "C" int cab_frontend_features(const void* signal, int signal_is_int16, co
     dim3 grid((F_pad + kPackFrames - 1) / kPackFrames, B);
     const size_t smem = sizeof(float) * kPackFrames * (C_pad + 1);
     CAB_CHECK_ARG(smem <= 48 * 1024, "C_pad=%d too large for the pack tile", C_pad);
-    instnorm_pack_kernel<<<grid, 256, smem, stream>>>(ws_logmel, (normalize_features && norm_masked) ? xlen_frac : nullptr, stats, B, n_mels, F, F_pad, C_pad, static_cast<__nv_bfloat16*>(out_hi),
+    instnorm_pack_kernel<false><<<grid, 256, smem, stream>>>(ws_logmel, (normalize_features && norm_masked) ? xlen_frac : nullptr, stats, B, n_mels, F, F_pad, C_pad, static_cast<__nv_bfloat16*>(out_hi),
                                                       static_cast<__nv_bfloat16*>(out_lo), out_f32, normalize_features);
     CAB_CHECK_LAUNCH();
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     return 0;
+}
+
+// frontend + instance norm under fixed normalisation (cab_frontend_features_fixed): the same STFT / mel / log kernel with
+// the caller's signal scale, then the pack with the caller's (mean, invstd).  Two launches, no statistics.
+static int frontend_fixed_params(FrontendParams& p, int B, int T, int F, int win_length, int hop, int nfft, int n_mels, const float* window,
+                                 const float* mel_fb, const int32_t* mel_band, const float* twiddle, float preemphasis, float log_eps,
+                                 float* ws_logmel) {
+    CAB_CHECK_ARG(window && mel_fb && mel_band && twiddle && ws_logmel, "null pointer argument");
+    CAB_CHECK_ARG(use_fft16(nfft, win_length, hop), "fixed normalisation and streaming cover the nfft = 256 frontend only (nfft=%d win=%d hop=%d)", nfft, win_length, hop);
+    p = FrontendParams{};
+    p.window = window; p.mel_fb = mel_fb; p.mel_band = mel_band; p.twiddle = reinterpret_cast<const float2*>(twiddle);
+    p.out = ws_logmel; p.B = B; p.T = T; p.F = F;
+    p.win = win_length; p.hop = hop; p.nfft = nfft; p.n_mels = n_mels; p.n_freq = nfft / 2 + 1;
+    p.first_off = -(nfft / 2) + (nfft - win_length) / 2;
+    p.preemph = preemphasis; p.log_eps = log_eps; p.denom_mult = 1.f;
+    return 0;
+}
+
+static int launch_pack_fixed(const float* logmel, const float* xlen_frac, const float* norm_stats, int B, int C, int F, int F_pad, int C_pad,
+                             void* out_hi, void* out_lo, cudaStream_t stream) {
+    dim3 grid((F_pad + kPackFrames - 1) / kPackFrames, B);
+    const size_t smem = sizeof(float) * kPackFrames * (C_pad + 1);
+    CAB_CHECK_ARG(smem <= 48 * 1024, "C_pad=%d too large for the pack tile", C_pad);
+    instnorm_pack_kernel<true><<<grid, 256, smem, stream>>>(logmel, xlen_frac, norm_stats, B, C, F, F_pad, C_pad, static_cast<__nv_bfloat16*>(out_hi),
+                                                            static_cast<__nv_bfloat16*>(out_lo), nullptr, 1);
+    CAB_CHECK_LAUNCH();
+    g_launch_count.fetch_add(1, std::memory_order_relaxed);
+    return 0;
+}
+
+extern "C" int cab_frontend_features_fixed(const void* signal, int signal_is_int16, const float* xlen_frac, int B, int T, int win_length, int hop,
+                                           int nfft, int n_mels, const float* window, const float* mel_fb, const int32_t* mel_band,
+                                           const float* twiddle, float preemphasis, float log_eps, const float* signal_scale,
+                                           const float* norm_stats, int norm_masked, float* ws_logmel, int F_pad, int C_pad, void* out_hi,
+                                           void* out_lo, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CAB_CHECK_ARG(signal && signal_scale && norm_stats && out_hi, "null pointer argument");
+    CAB_CHECK_ARG(B > 0 && T > 0, "bad shape B=%d T=%d", B, T);
+    CAB_CHECK_ARG(hop > 0, "bad hop %d", hop);
+    const int F = T / hop + 1;
+    CAB_CHECK_ARG(F_pad >= F && C_pad >= n_mels && C_pad % 8 == 0, "bad output layout F_pad=%d C_pad=%d", F_pad, C_pad);
+    FrontendParams p;
+    if (int rc = frontend_fixed_params(p, B, T, F, win_length, hop, nfft, n_mels, window, mel_fb, mel_band, twiddle, preemphasis, log_eps, ws_logmel)) return rc;
+    p.signal = signal; p.xlen = xlen_frac; p.is_int16 = signal_is_int16;
+    if (int rc = launch_logmel16<kFixedStats>(p, nullptr, 0, nullptr, nullptr, 0.f, stream, signal_scale)) return rc;
+    return launch_pack_fixed(ws_logmel, norm_masked ? xlen_frac : nullptr, norm_stats, B, n_mels, F, F_pad, C_pad, out_hi, out_lo, stream);
+}
+
+extern "C" int cab_frontend_stream(const float* staged, int pitch, const int32_t* rows, int B, int F, int win_length, int hop, int nfft,
+                                   int n_mels, const float* window, const float* mel_fb, const int32_t* mel_band, const float* twiddle,
+                                   float preemphasis, float log_eps, const float* signal_scale, const float* norm_stats, float* ws_logmel,
+                                   int C_pad, void* out_hi, void* out_lo, cab_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CAB_CHECK_ARG(staged && rows && signal_scale && norm_stats && out_hi, "null pointer argument");
+    CAB_CHECK_ARG(B > 0 && F > 0 && pitch > 0 && pitch % 4 == 0, "bad shape B=%d F=%d pitch=%d (a multiple of 4 samples)", B, F, pitch);
+    CAB_CHECK_ARG((reinterpret_cast<uintptr_t>(staged) & 15) == 0, "staged samples must be 16-byte aligned");
+    CAB_CHECK_ARG(C_pad >= n_mels && C_pad % 8 == 0, "bad output layout C_pad=%d", C_pad);
+    FrontendParams p;
+    if (int rc = frontend_fixed_params(p, B, pitch, F, win_length, hop, nfft, n_mels, window, mel_fb, mel_band, twiddle, preemphasis, log_eps, ws_logmel)) return rc;
+    p.signal = staged; p.is_int16 = 0;
+    if (int rc = launch_logmel16<kStream>(p, nullptr, 0, nullptr, nullptr, 0.f, stream, signal_scale, rows)) return rc;
+    return launch_pack_fixed(ws_logmel, nullptr, norm_stats, B, n_mels, F, F, C_pad, out_hi, out_lo, stream);
 }
 
 extern "C" int cab_instnorm_pack(const float* feat, const float* xlen_frac, int B, int C, int F,
@@ -776,7 +859,7 @@ extern "C" int cab_instnorm_pack(const float* feat, const float* xlen_frac, int 
         dim3 grid((F_pad + kPackFrames - 1) / kPackFrames, B);
         size_t smem = sizeof(float) * kPackFrames * (C_pad + 1);
         CAB_CHECK_ARG(smem <= 48 * 1024, "C_pad=%d too large for the pack tile", C_pad);
-        instnorm_pack_kernel<<<grid, 256, smem, stream>>>(feat, xlen_frac, ws_stats, B, C, F, F_pad, C_pad,
+        instnorm_pack_kernel<false><<<grid, 256, smem, stream>>>(feat, xlen_frac, ws_stats, B, C, F, F_pad, C_pad,
                                                           static_cast<__nv_bfloat16*>(out_hi),
                                                           static_cast<__nv_bfloat16*>(out_lo), out_f32, normalize);
         CAB_CHECK_LAUNCH();

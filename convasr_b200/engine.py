@@ -367,7 +367,11 @@ class StackPlan:
 			T_out = (x.T + 2 * pad - (k - 1) - 1) // 2 + 1
 		else:
 			T_out = x.T + L.dT
-		srcs = self._sources(L, x, tmp, residuals)
+		return self.run_gemm(L, self._sources(L, x, tmp, residuals), xlen if L.mask else None, B, T_out, dev)
+
+	def run_gemm(self, L, srcs, xlen, B, T_out, dev):
+		"""the fused GEMM of launch L over its operand pairs `srcs` and its epilogue: an _Act, or per head (logits, log_probs,
+		argmax); xlen: the temporal mask (None: none)"""
 		code, a, b = L.act
 		if self.fp8:
 			return self._run_epilogue_fp8(L, srcs, xlen, B, T_out, dev)
@@ -375,7 +379,7 @@ class StackPlan:
 			srcs = self._fold_excess_sources(srcs, B, T_out, L.C_alloc, dev)
 			out_hi = torch.empty(B, T_out, L.C_alloc, dtype = BF16, device = dev)
 			out_lo = torch.empty_like(out_hi) if self.fp32_tier else None
-			ops.conv1d_fused(srcs, B, T_out, L.C_alloc, bias = L.bias, act = code, act_a = a, act_b = b, xlen = xlen if L.mask else None, out_hi = out_hi, out_lo = out_lo)
+			ops.conv1d_fused(srcs, B, T_out, L.C_alloc, bias = L.bias, act = code, act_a = a, act_b = b, xlen = xlen, out_hi = out_hi, out_lo = out_lo)
 			return _Act(out_hi, out_lo, T_out, L.C_out)
 		if L.epilogue == _lib.EPI_LOGSOFTMAX or code != _lib.ACT_NONE:
 			logits = torch.empty(B, L.C_out, T_out, dtype = torch.float32, device = dev)
@@ -396,7 +400,7 @@ class StackPlan:
 		code, a, b = L.act
 		if L.epilogue == _lib.EPI_ACT_BF16:
 			out = torch.empty(B, T_out, L.C_alloc, dtype = FP8, device = dev)
-			ops.conv1d_fused_fp8(srcs, B, T_out, L.C_alloc, L.alpha, 1.0 / L.out_scale, bias = L.bias, act = code, act_a = a, act_b = b, xlen = xlen if L.mask else None, out = out)
+			ops.conv1d_fused_fp8(srcs, B, T_out, L.C_alloc, L.alpha, 1.0 / L.out_scale, bias = L.bias, act = code, act_a = a, act_b = b, xlen = xlen, out = out)
 			return _Act(out, None, T_out, L.C_out)
 		if L.epilogue == _lib.EPI_LOGSOFTMAX:
 			logits = torch.empty(B, L.C_out, T_out, dtype = torch.float32, device = dev)

@@ -123,12 +123,19 @@ class LogFilterBankFrontend(nn.Module):
 			denom_multiplier = self.debug_short_long_records_normalize_signal_multiplier
 		)
 
-	def features(self, signal, xlen, norm, F_pad_even, C_pad, want_lo):
+	def features(self, signal, xlen, norm, F_pad_even, C_pad, want_lo, normalisation = None):
 		"""signal -> instance-normalised bf16 channels-last features in one native call (what JasperNet.forward does at
-		models.py:286-301); norm: the model's MaskedInstanceNorm1d or None"""
+		models.py:286-301); norm: the model's MaskedInstanceNorm1d or None; normalisation: a FixedNormalisation to apply
+		instead of the per-utterance statistics"""
 		mel, band, twiddle, window, log_eps = self._device_tables(signal.device)
 		Fr = signal.shape[1] // self.hop_length + 1
 		F_pad = Fr + (Fr % 2) if F_pad_even else Fr
+		if normalisation is not None:
+			hi, lo = ops.frontend_features_fixed(
+				signal, xlen, window, mel, band, twiddle, self.hop_length, self.nfft, self.preemphasis, log_eps, normalisation.signal_scale,
+				normalisation.stats(), norm is not None and norm.temporal_mask, F_pad, C_pad, want_lo = want_lo
+			)
+			return hi, lo, Fr
 		hi, lo, _ = ops.frontend_features(
 			signal, xlen, window, mel, band, twiddle, self.hop_length, self.nfft, self.preemphasis, log_eps, self.normalize_signal,
 			self.debug_short_long_records_normalize_signal_multiplier, norm is not None, norm is not None and norm.temporal_mask, norm.eps if norm is not None else 0.0,
@@ -157,6 +164,34 @@ def normalize_signal(signal, dim = -1, eps = 1e-5, denom_multiplier = 1.0):
 	"""models.py:684-686 (host-side helper; the model path fuses this into the frontend kernel)"""
 	signal_max = signal.abs().max(dim = dim, keepdim = True).values + eps
 	return signal / (signal_max * denom_multiplier) if signal.numel() > 0 else signal
+
+
+class FixedNormalisation:
+	"""Normalisation fixed ahead of time instead of measured on each utterance: `signal_scale` [B] multiplies the signal in
+	place of 1 / (max|x| + 1e-5) (models.py:684-686) and the instance norm applies `mean` / `invstd` [B, n_mels] in place of
+	the per-utterance statistics (models.py:694-719).  fp32 CUDA tensors.  A stream cannot know its own statistics before
+	it ends, so this is what streaming inference (convasr_b200.streaming) runs on; `JasperNet.forward(..., normalisation=)`
+	computes the same features in one shot.  convasr_b200.streaming.estimate_normalisation computes one from a prefix."""
+
+	def __init__(self, signal_scale, mean, invstd):
+		for name, t in (('signal_scale', signal_scale), ('mean', mean), ('invstd', invstd)):
+			if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != torch.float32:
+				raise TypeError(f'convasr_b200: FixedNormalisation.{name} must be an fp32 CUDA tensor')
+		if signal_scale.ndim != 1 or mean.ndim != 2 or mean.shape != invstd.shape or mean.shape[0] != signal_scale.shape[0]:
+			raise ValueError(f'convasr_b200: FixedNormalisation shapes signal_scale {tuple(signal_scale.shape)}, mean {tuple(mean.shape)}, invstd {tuple(invstd.shape)}; want [B], [B, n_mels], [B, n_mels]')
+		self.signal_scale, self.mean, self.invstd = signal_scale.contiguous(), mean.contiguous(), invstd.contiguous()
+
+	def __len__(self):
+		return self.signal_scale.shape[0]
+
+	def __getitem__(self, i):
+		"""rows i (an int or a slice) as a FixedNormalisation of their own"""
+		i = slice(i, i + 1) if isinstance(i, int) else i
+		return FixedNormalisation(self.signal_scale[i], self.mean[i], self.invstd[i])
+
+	def stats(self):
+		"""fp32 [B, n_mels, 2] (mean, invstd), the layout of the native pack"""
+		return torch.stack([self.mean, self.invstd], dim = -1).contiguous()
 
 
 class MaskedInstanceNorm1d(nn.InstanceNorm1d):
@@ -436,9 +471,13 @@ class JasperNet(nn.Module):
 		return self
 
 	# -- forward --------------------------------------------------------------------------
-	def forward(self, x, xlen = None, y = None, ylen = None):
+	def forward(self, x, xlen = None, y = None, ylen = None, normalisation = None):
+		"""normalisation: None normalises every utterance by its own statistics (the reference); a FixedNormalisation
+		(eval mode, nfft = 256 frontend) applies the given signal scale and instance-norm statistics instead"""
 		if not x.is_cuda:
 			raise RuntimeError('convasr_b200: model inputs must be CUDA tensors (there is no CPU fallback)')
+		if normalisation is not None:
+			self._check_fixed_normalisation(normalisation, x.shape[0])
 		if xlen is not None:
 			xlen = xlen.to(device = x.device, dtype = torch.float32).contiguous()
 		if self.frontend is not None:
@@ -459,7 +498,7 @@ class JasperNet(nn.Module):
 				raise NotImplementedError(f'convasr_b200: training of this module tree is not built ({why}); there is no ATen / cuDNN fallback')
 			logits, log_probs = training.forward_training(self, x, xlen)  # frontend, conv/BN forward + backward on this repo's kernels
 		else:
-			logits, log_probs = self._forward_native(x, xlen)
+			logits, log_probs = self._forward_native(x, xlen, normalisation)
 		olen = [compute_output_lengths(l, xlen) for l in logits]
 		aux = {}
 		if y is not None and ylen is not None:
@@ -508,7 +547,19 @@ class JasperNet(nn.Module):
 		graph.replay()
 		return [(lg.clone(), lp.clone(), am.clone()) for lg, lp, am in outs]
 
-	def _packed_features(self, x, xlen, want_lo, c_align = 64):
+	def _check_fixed_normalisation(self, normalisation, B):
+		if self.training:
+			raise RuntimeError('convasr_b200: fixed normalisation is an inference feature; call model.eval()')
+		if not isinstance(normalisation, FixedNormalisation):
+			raise TypeError('convasr_b200: normalisation must be a models.FixedNormalisation')
+		fe = self.frontend
+		if not isinstance(fe, LogFilterBankFrontend) or fe.nfft != 256:
+			raise NotImplementedError('convasr_b200: fixed normalisation needs the model\'s LogFilterBankFrontend with nfft = 256 (other FFT sizes are not built)')
+		n_mels = fe.mel.weight.shape[0]
+		if len(normalisation) != B or normalisation.mean.shape[1] != n_mels:
+			raise ValueError(f'convasr_b200: normalisation has {len(normalisation)} rows of {normalisation.mean.shape[1]} channels; the input has {B} rows of {n_mels} mel channels')
+
+	def _packed_features(self, x, xlen, want_lo, c_align = 64, normalisation = None):
 		"""raw input (signal when the frontend is in the model, else fp32 features [B, C, F]) -> (bf16 hi, lo or None, frames, channels):
 		log-mel frontend + masked instance norm + channels-last packing (models.py:286-301)"""
 		nf = self.normalize_features
@@ -517,7 +568,7 @@ class JasperNet(nn.Module):
 		stride = self.backbone[0].conv[0][0].stride[0]
 		if self.frontend is not None and isinstance(self.frontend, LogFilterBankFrontend) and self.frontend.nfft == 256:
 			C = self.frontend.mel.weight.shape[0]
-			hi, lo, Fr = self.frontend.features(x, xlen, nf, stride == 2, engine._ceil_to(C, c_align), want_lo)
+			hi, lo, Fr = self.frontend.features(x, xlen, nf, stride == 2, engine._ceil_to(C, c_align), want_lo, normalisation)
 			return hi, lo, Fr, C
 		feats = self.frontend(x, xlen = xlen) if self.frontend is not None else x
 		B, C, Fr = feats.shape
@@ -526,19 +577,19 @@ class JasperNet(nn.Module):
 		hi, lo, _ = ops.instnorm_pack(feats, norm_xlen, nf.eps if nf is not None else -1.0, F_pad = F_pad, C_pad = engine._ceil_to(C, c_align), want_lo = want_lo, normalize = nf is not None)
 		return hi, lo, Fr, C
 
-	def _raw_to_outputs(self, x, xlen):
+	def _raw_to_outputs(self, x, xlen, normalisation = None):
 		"""raw input (signal or features) -> per head (logits, log_probs, argmax); kernels only"""
 		plan = self._get_plan()
-		hi, lo, Fr, C = self._packed_features(x, xlen, plan.fp32_tier, plan.feat_align)
+		hi, lo, Fr, C = self._packed_features(x, xlen, plan.fp32_tier, plan.feat_align, normalisation)
 		if plan.fp8:
 			hi = ops.quantize_e4m3(hi, plan.blocks[0][0].in_scale)
 		return plan.run(engine._Act(hi, lo, Fr, C), xlen)
 
-	def _forward_native(self, x, xlen):
-		if getattr(self, '_graphs_enabled', False) and not torch.cuda.is_current_stream_capturing():
+	def _forward_native(self, x, xlen, normalisation = None):
+		if normalisation is None and getattr(self, '_graphs_enabled', False) and not torch.cuda.is_current_stream_capturing():
 			outs = self._graphed_raw(x, xlen)
 		else:
-			outs = self._raw_to_outputs(x, xlen)
+			outs = self._raw_to_outputs(x, xlen, normalisation)
 		logits, log_probs = [], []
 		for lg, lp, am in outs:
 			lp._convasr_argmax = am  # lets GreedyCTCGenerator skip its own argmax pass

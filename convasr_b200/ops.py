@@ -57,8 +57,9 @@ def make_mel_band(mel_fb):
 
 def frontend_logmel(
 	signal, xlen, window, mel_fb, mel_band, twiddle, hop, nfft, preemphasis = 0.97, log_eps = 2.0**-14,
-	normalize_signal = True, denom_multiplier = 1.0
+	normalize_signal = True, denom_multiplier = 1.0, absmax = None
 ):
+	"""absmax: fp32 [B] that receives max |x| of each row when normalize_signal"""
 	_need_cuda(signal, xlen, window, mel_fb, mel_band, twiddle)
 	assert signal.ndim == 2
 	if signal.dtype == torch.int16:
@@ -71,7 +72,7 @@ def frontend_logmel(
 	n_mels = mel_fb.shape[0]
 	F = T // hop + 1
 	out = torch.empty(B, n_mels, F, dtype = torch.float32, device = signal.device)
-	ws = torch.empty(B, dtype = torch.float32, device = signal.device)
+	ws = torch.empty(B, dtype = torch.float32, device = signal.device) if absmax is None else absmax
 	xl = None if xlen is None else xlen.to(torch.float32).contiguous()
 	if B == 0 or T == 0:
 		return out
@@ -114,7 +115,59 @@ def frontend_features(signal, xlen, window, mel_fb, mel_band, twiddle, hop, nfft
 	return hi, lo, logmel
 
 
-def instnorm_pack(feat, xlen, eps, F_pad = None, C_pad = None, want_lo = False, want_f32 = False, want_hi = None, normalize = True):
+def frontend_features_fixed(signal, xlen, window, mel_fb, mel_band, twiddle, hop, nfft, preemphasis, log_eps, signal_scale, norm_stats, norm_masked,
+							F_pad, C_pad, want_lo = False):
+	"""frontend_features under fixed normalisation (cab_frontend_features_fixed): signal_scale fp32 [B], norm_stats fp32
+	[B, n_mels, 2] (mean, invstd) -> (bf16 hi [B, F_pad, C_pad], bf16 lo or None)"""
+	_need_cuda(signal, xlen, window, mel_fb, mel_band, twiddle, signal_scale, norm_stats)
+	assert signal.ndim == 2
+	is_i16 = int(signal.dtype == torch.int16)
+	if not is_i16:
+		signal = signal.to(torch.float32)
+	signal = signal.contiguous()
+	B, T = signal.shape
+	n_mels = mel_fb.shape[0]
+	assert signal_scale.shape == (B, ) and norm_stats.shape == (B, n_mels, 2)
+	dev = signal.device
+	logmel = torch.empty(B, n_mels, T // hop + 1, dtype = torch.float32, device = dev)
+	hi = torch.empty(B, F_pad, C_pad, dtype = BF16, device = dev)
+	lo = torch.empty_like(hi) if want_lo else None
+	xl = None if xlen is None else xlen.to(torch.float32).contiguous()
+	rc = _lib.load().cab_frontend_features_fixed(
+		_p(signal), is_i16, _p(xl), B, T, window.numel(), hop, nfft, n_mels, _p(window), _p(mel_fb), _p(mel_band), _p(twiddle), float(preemphasis),
+		float(log_eps), _p(signal_scale), _p(norm_stats), int(bool(norm_masked)), _p(logmel), F_pad, C_pad, _p(hi), _p(lo), _stream()
+	)
+	_lib.check(rc, 'cab_frontend_features_fixed')
+	return hi, lo
+
+
+def frontend_stream(staged, rows, F, window, mel_fb, mel_band, twiddle, hop, nfft, preemphasis, log_eps, signal_scale, norm_stats, C_pad, want_lo = False):
+	"""streaming frontend (cab_frontend_stream): staged fp32 [B, pitch] samples, rows int32 [B, 5] on the device ->
+	(bf16 hi [B, F, C_pad], bf16 lo or None)"""
+	_need_cuda(staged, rows, window, mel_fb, mel_band, twiddle, signal_scale, norm_stats)
+	assert staged.dtype == torch.float32 and staged.is_contiguous() and rows.dtype == torch.int32 and rows.is_contiguous()
+	B, pitch = staged.shape
+	n_mels = mel_fb.shape[0]
+	dev = staged.device
+	logmel = torch.empty(B, n_mels, F, dtype = torch.float32, device = dev)
+	hi = torch.empty(B, F, C_pad, dtype = BF16, device = dev)
+	lo = torch.empty_like(hi) if want_lo else None
+	rc = _lib.load().cab_frontend_stream(
+		_p(staged), pitch, _p(rows), B, F, window.numel(), hop, nfft, n_mels, _p(window), _p(mel_fb), _p(mel_band), _p(twiddle), float(preemphasis),
+		float(log_eps), _p(signal_scale), _p(norm_stats), _p(logmel), C_pad, _p(hi), _p(lo), _stream()
+	)
+	_lib.check(rc, 'cab_frontend_stream')
+	return hi, lo
+
+
+def stream_copy(jobs, max_bytes):
+	"""batched device copies (cab_stream_copy): jobs int64 [n, 3] (dst, src or 0 for zeros, bytes) on the device"""
+	_need_cuda(jobs)
+	assert jobs.dtype == torch.int64 and jobs.is_contiguous() and jobs.ndim == 2 and jobs.shape[1] == 3
+	_lib.check(_lib.load().cab_stream_copy(_p(jobs), jobs.shape[0], int(max_bytes), _stream()), 'cab_stream_copy')
+
+
+def instnorm_pack(feat, xlen, eps, F_pad = None, C_pad = None, want_lo = False, want_f32 = False, want_hi = None, normalize = True, stats = None):
 	"""fp32 [B,C,F] -> (bf16 hi [B,F_pad,C_pad], bf16 lo or None, fp32 [B,C,F] or None)"""
 	_need_cuda(feat, xlen)
 	feat = feat.to(torch.float32).contiguous()
@@ -125,7 +178,7 @@ def instnorm_pack(feat, xlen, eps, F_pad = None, C_pad = None, want_lo = False, 
 	hi = torch.empty(B, F_pad, C_pad, dtype = BF16, device = feat.device) if want_hi or want_lo else None
 	lo = torch.empty_like(hi) if want_lo else None
 	f32 = torch.empty_like(feat) if want_f32 else None
-	stats = torch.empty(B, C, 2, dtype = torch.float32, device = feat.device)
+	stats = torch.empty(B, C, 2, dtype = torch.float32, device = feat.device) if stats is None else stats  # given: receives (mean, sd)
 	xl = None if xlen is None else xlen.to(torch.float32).contiguous()
 	rc = _lib.load().cab_instnorm_pack(
 		_p(feat), _p(xl), B, C, F, float(eps), int(bool(normalize)), F_pad, C_pad, _p(hi), _p(lo), _p(f32), _p(stats), _stream()

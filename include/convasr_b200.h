@@ -83,6 +83,34 @@ int cab_frontend_features(const void* signal, int signal_is_int16, const float* 
                           void* out_lo, float* out_f32, float* ws_absmax, float* ws_partials,
                           cab_stream_t stream);
 
+/* cab_frontend_features under FIXED normalisation (nfft = 256 frontend only): every sample is multiplied by
+ * signal_scale[b] instead of being divided by the utterance's abs-max, and the instance norm applies the caller's
+ * statistics: out = (logmel - mean) * invstd with norm_stats fp32 [B, n_mels, 2] = (mean, invstd).  Two launches, no
+ * statistics are computed.  norm_masked: frames >= ceil(xlen_frac * F) are written as 0 (as cab_frontend_features).
+ * ws_logmel: fp32 [B, n_mels, T / hop + 1]. */
+int cab_frontend_features_fixed(const void* signal, int signal_is_int16, const float* xlen_frac, int B, int T, int win_length,
+                                int hop, int nfft, int n_mels, const float* window, const float* mel_fb,
+                                const int32_t* mel_band, const float* twiddle, float preemphasis, float log_eps,
+                                const float* signal_scale, const float* norm_stats, int norm_masked, float* ws_logmel,
+                                int F_pad, int C_pad, void* out_hi, void* out_lo, cab_stream_t stream);
+
+/* Streaming frontend (convasr_b200/streaming.py): the frames of cab_frontend_features_fixed, computed from per-stream
+ * staged samples.  staged: fp32 [B, pitch] (16-byte aligned, pitch a multiple of 4); rows: device int32 [B, 5] =
+ * (first frame, frames, base, staged, reflect): row b holds samples [base, base + staged) of its stream, emits frames
+ * [first, first + frames) to out rows [0, frames) (rows up to F - 1 are written and are don't-care), samples at or past
+ * base + staged read as 0 (the right zero pad at the end of the stream) and reflect selects the reflect (1) or constant
+ * (0) left pad.  Frames whose window starts before sample 0 need base = 0.  out_hi / out_lo: bf16 [B, F, C_pad];
+ * ws_logmel: fp32 [B, n_mels, F]. */
+int cab_frontend_stream(const float* staged, int pitch, const int32_t* rows, int B, int F, int win_length, int hop, int nfft,
+                        int n_mels, const float* window, const float* mel_fb, const int32_t* mel_band, const float* twiddle,
+                        float preemphasis, float log_eps, const float* signal_scale, const float* norm_stats,
+                        float* ws_logmel, int C_pad, void* out_hi, void* out_lo, cab_stream_t stream);
+
+/* Batched device copies of the streaming model: jobs is a device int64 [n_jobs, 3] of (dst, src, bytes); src 0 writes
+ * zeros.  Pointers and sizes are multiples of 16 bytes, max_bytes bounds every size, and no two ranges of one call
+ * overlap.  One launch for all jobs (gather of launch inputs, append of new rows, rebase of stream buffers). */
+int cab_stream_copy(const int64_t* jobs, int n_jobs, int64_t max_bytes, cab_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------
  * A5-A9: Conv1d (+folded BatchNorm) + residual 1x1 convs + activation + temporal mask as ONE
  *   tcgen05/TMEM implicit GEMM.  Replaces ConvBn1d.forward (models.py:127-139) in its
